@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port)
+    python bench.py --steps K --dump-outputs DIR             # also save a sample of the last timed step's result
 
 Workload (config C5 of BASELINE.json, weak-scaled): 1000-qubit product of a 12 500*N-term operator A
 (each rank holds one 12 500-row block, seeds 100+rank) with a 10 000-term operator B (seed 7),
@@ -41,6 +42,8 @@ CPU_CHUNK_B = 1000
 CPU_CHUNKS = 3
 SPAN_GENERATORS = 28
 C1_TERMS = 500
+DUMP_TERMS = 4096                                     # --dump-outputs: 4096 sampled rows x 2000 bits as float32 = 33 MB
+DUMP_SEED = 20240
 
 
 def make_operator(n_terms, seed):
@@ -169,6 +172,32 @@ def pinned_pair(symp, coeff):
     return ts.numpy(), tc.numpy(), int(ts.numel() * ts.element_size() + tc.numel() * tc.element_size())
 
 
+def dump_outputs(out_dir, xz, c, prefix=""):
+    """Save the result operator of a timed step as its caller sees it (PauliwordOp.symp_matrix and .coeff_vec) so
+    that two builds can be compared output for output. The result has 1.25e8 terms per GPU (34 GB), so the rows
+    are a fixed, seeded sample of DUMP_TERMS term positions; n_terms and the coefficient sums cover all of it.
+    Files: <prefix><name>.npy, float32 (0/1 Pauli bits) or float64, 33 MB in all."""
+    import torch
+
+    from symmer_b200 import ops
+    n_terms = int(xz.shape[0])
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_terms, size=min(n_terms, DUMP_TERMS), replace=False))
+    sel = torch.from_numpy(idx).to(xz.device)
+    symp = ops.to_host(ops.unpack(xz[sel].contiguous(), N_QUBITS))
+    coeff = c[sel].cpu().numpy()
+    total = complex(c.sum().item())
+    arrays = {
+        "n_terms": np.array([n_terms], dtype=np.float64),
+        "coeff_vec_sum": np.array([total.real, total.imag, c.abs().sum().item()], dtype=np.float64),
+        "term_index": idx.astype(np.float64),
+        "symp_matrix": symp.astype(np.float32),
+        "coeff_vec_real": coeff.real.astype(np.float64),
+        "coeff_vec_imag": coeff.imag.astype(np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -219,10 +248,11 @@ def run_ours(args):
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)   # > 126 MB L2
 
-    def timed(fn, n):
-        """n steps, each bracketed by CUDA events on the launching stream; L2 flushed between steps."""
-        ms = []
-        for _ in range(n):
+    def timed(fn, n, keep_last=False):
+        """n steps, each bracketed by CUDA events on the launching stream; L2 flushed between steps.
+        With keep_last, returns (times, output of the last step)."""
+        ms, last = [], None
+        for i in range(n):
             flush.fill_(1)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -230,8 +260,10 @@ def run_ours(args):
             e1.record()
             torch.cuda.synchronize()
             ms.append(e0.elapsed_time(e1))
+            if keep_last and i == n - 1:
+                last = out
             del out
-        return ms
+        return (ms, last) if keep_last else ms
 
     # ---------------------------------------------------------------- device-resident arm (`value`)
     A_op, B_op = PauliwordOp(a_np, ac_np), PauliwordOp(b_np, bc_np)
@@ -252,7 +284,7 @@ def run_ours(args):
     ops.emit_kernel_events = []
     launches0 = ops.launch_count()
     t_wall0 = time.perf_counter()
-    ms_steps = timed(step_resident, args.steps)
+    ms_steps, last_out = timed(step_resident, args.steps, keep_last=True)
     barrier()
     wall = time.perf_counter() - t_wall0
     launches = ops.launch_count() - launches0
@@ -261,6 +293,9 @@ def run_ours(args):
     ops.emit_events = None
     ops.emit_kernel_events = None
     step_ms = float(np.mean(ms_steps))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_out, prefix=f"rank{rank}_" if world > 1 else "")
+    del last_out
 
     # ---------------------------------------------------------------- end-to-end arm (`e2e`): host buffers in, result summary out
     def step_e2e():
@@ -565,7 +600,15 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--check", action="store_true", help="(always on) verify the timed product's output; the run fails if it does not hold")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of the last timed step's result to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the result of this engine's timed product; the reference arm has none")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)      # fail before any GPU work if DIR cannot be created
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -26,11 +26,17 @@ def test_api_case_on_host_double(case, api_golden, host_ops):
 
 
 def test_double_is_gone_after_the_block():
+    import torch
     from symmer_b200 import ops
+    real_device = ops.device
     with host_double():
         assert ops.device().type == "cpu"
-    with pytest.raises(RuntimeError):
-        ops.device()                      # no CUDA device here: the product path refuses to run
+    assert ops.device is real_device
+    if torch.cuda.is_available():
+        assert ops.device().type == "cuda"
+    else:
+        with pytest.raises(RuntimeError):
+            ops.device()                  # no CUDA device: the product path refuses to run
 
 
 def test_double_matches_the_oracle_on_core_paths(golden, host_ops):
