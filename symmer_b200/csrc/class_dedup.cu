@@ -16,6 +16,7 @@
 // which takes the ordinary global sort. No tensor cores: integer/bit work on L2-resident tables,
 // shared-memory bound.
 #include <algorithm>
+#include <type_traits>
 
 #include "rows.cuh"
 #include "sort.cuh"
@@ -529,11 +530,33 @@ __global__ void __launch_bounds__(THREADS, MINB) class_dedup_kernel(ClassJob J, 
 // into the global candidate array by the counting sort (small groups ordered by their owner thread afterwards); a
 // class with a large hash group, or with records that never found a slot, sends its candidates to the overflow array.
 // ------------------------------------------------------------------------------------------------
-// PRE_LOG > 0: a presence filter in front of the table rounds. Two bitmaps of 2^PRE_LOG bits, indexed by a function of
-// the hash alone: every record sets its bit in the first map and, if it was already set, in the second. After a
-// barrier a record whose bit is clear in the SECOND map shares its hash with nobody in the class: it is unique, and
-// it never enters the rounds (one shared-memory atomic and one load instead of a store, a load and a compare per
-// round). On a product without duplicates ~95 % of the records stop here, and the table can be half the size.
+// PRE_LOG > 0: a presence filter in front of the table rounds. Two bitmaps of 2^PRE_LOG bits, indexed by a cheap function
+// of the masked sketch key (cd_filter_index): every record sets its bit in the first map and, if it was already set, in the
+// second. After a barrier a record whose bit is clear in the SECOND map shares its key with nobody in the class: it is a
+// unique row (equal rows have equal keys) and is done without ever being hashed. On a product without duplicates ~95 % of
+// the records stop here. The others ("survivors") are compacted into a dense list of record ids; the hash (mix64), the
+// table rounds, the mate bits and the counting sort of the candidates walk that list, so a thread handles one entry per
+// round instead of RPT predicated slots. PRE_LOG = 0 (tuning knob 11 = 3): no filter, every record is a survivor and the
+// list is the identity (not stored).
+//
+// Dynamic shared memory, in 4-byte words, with AREA = SLOTS + 2 * PRE_WORDS:
+//   [0, AREA)           enumeration + filter:  table [0, SLOTS) | map1 | map2
+//                       table rounds:          table [0, SLOTS) | ... | survivor list (CAP 16-bit ids) [AREA - CAP/2, AREA)
+//                       candidates:            group counters [0, CAP) | ... | survivor list
+//   [AREA, +CAP)        pairs
+//   [.., +CAP/32)       mate bits, by list index
+//   [.., +CD32_BM_WORDS) copy of the non-empty bitmap
+// The list is written after every thread has read map2 (the barriers of its block prefix) and read until the candidates
+// have left, so neither the table nor the group counters may reach it.
+
+// presence-filter bit of a record: a function of the masked key alone, so equal rows share it and a debug key mask that
+// zeroes the key forces every record through the table; the 64 -> 32 fold keeps the bits that vary inside a class (the
+// class and owner-class functionals fix only a few linear combinations of the key)
+template <int PRE_LOG>
+__device__ __forceinline__ uint32_t cd_filter_index(uint64_t key) {
+    return (((uint32_t)key ^ (uint32_t)(key >> 32)) * 0x85EBCA6Bu) >> (32 - PRE_LOG);
+}
+
 template <int THREADS, int CAP, int LOG_SLOTS, int PRE_LOG>
 __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, ProductRows rows, TileMap tm, double thr,
                                                                     uint64_t *__restrict__ cand, uint64_t *__restrict__ over,
@@ -541,16 +564,19 @@ __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, P
     constexpr int SLOTS = 1 << LOG_SLOTS;
     constexpr int RPT = CAP / THREADS;
     constexpr int PRE_WORDS = PRE_LOG > 0 ? (1 << PRE_LOG) / 32 : 0;
-    static_assert(CAP % THREADS == 0 && CAP <= 65536 && RPT <= 32, "record ids are 16 bits, one state bit per record");
-    static_assert(CAP <= SLOTS + 2 * PRE_WORDS, "the group counters live in the table (and the maps behind it) after the rounds");
+    constexpr int AREA = SLOTS + 2 * PRE_WORDS;
+    constexpr int LIST_AT = PRE_LOG > 0 ? AREA - CAP / 2 : AREA;
+    static_assert(CAP % THREADS == 0 && CAP <= 65536 && RPT <= 32, "record ids and list indices are 16 bits, one state bit per record");
+    static_assert(SLOTS <= LIST_AT && CAP <= LIST_AT, "the table and the group counters stay below the survivor list");
     extern __shared__ __align__(16) unsigned char cd_smem[];
     uint32_t *table = reinterpret_cast<uint32_t *>(cd_smem);
-    uint32_t *map1 = table + SLOTS;                     // contiguous with the table: the group counters may run into them
+    uint32_t *map1 = table + SLOTS;
     uint32_t *map2 = map1 + PRE_WORDS;
-    uint32_t *pairs = map2 + PRE_WORDS;
-    uint32_t *mate = pairs + CAP;                       // one bit per record: a same-hash record saw it holding a slot
+    uint16_t *list = reinterpret_cast<uint16_t *>(table + LIST_AT);
+    uint32_t *pairs = table + AREA;
+    uint32_t *mate = pairs + CAP;                       // one bit per list entry: a same-hash record saw it holding a slot
     uint32_t *s_bits = mate + CAP / 32;
-    __shared__ uint32_t s_count, s_ncand, s_base;
+    __shared__ uint32_t s_count, s_nsurv, s_ncand, s_base;
     __shared__ uint32_t s_warp[33];
     const int tid = threadIdx.x;
     const uint32_t K = 1u << J.k;
@@ -560,10 +586,21 @@ __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, P
     const bool bm_shared = bm_words <= (uint32_t)CD32_BM_WORDS;
     if (bm_shared)
         for (uint32_t i = tid; i < bm_words; i += THREADS) s_bits[i] = J.bits[i];
+    auto record_of = [&](uint32_t e) -> uint32_t {   // pair-list position of survivor e
+        if constexpr (PRE_LOG > 0) return list[e];
+        else return e;
+    };
+    auto drop_if_small = [&](uint32_t pr) {          // a unique row survives unless its own coefficient fails the threshold
+        const uint32_t t = J.vq[pr & vmask] * J.M_total + J.lookp[pr >> vbits];
+        double re, im;
+        rows.coeff_unphased(t, re, im);
+        if (!keep_test(re, im, thr)) tm.mark_dropped(t);
+    };
 
     for (uint32_t c = blockIdx.x; c < K; c += gridDim.x) {
         if (tid == 0) {
             s_count = 0;
+            s_nsurv = 0;
             s_ncand = 0;
         }
         for (int i = tid; i < CAP / 32; i += THREADS) mate[i] = 0u;
@@ -584,169 +621,197 @@ __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, P
             __syncthreads();
             continue;
         }
-        // ---- records of this thread: the top 32 bits of the mixed sketch are THE hash of this kernel
-        uint32_t h32[RPT];
-        uint32_t rr[RPT];      // representative (local id) of the record's hash group; later | rank << 16
-        uint32_t unres = 0, candm = 0, winm = 0;
-#pragma unroll
-        for (int j = 0; j < RPT; ++j) {
-            const uint32_t i = tid + j * THREADS;
-            h32[j] = 0;
-            rr[j] = i;
-            if (i < total) {
-                const uint32_t pr = pairs[i];
-                h32[j] = (uint32_t)((mix64(__ldg(J.look8 + (pr >> vbits)) ^ __ldg(J.vsk + (pr & vmask))) & J.key_mask) >> 32);
-                unres |= 1u << j;
-            }
-        }
+        // ---- presence filter over the records of this thread (pair-list positions tid + j * THREADS)
+        uint32_t n_surv = total;
         if constexpr (PRE_LOG > 0) {
-#pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-                if ((unres >> j) & 1u) {
-                    const uint32_t b = (h32[j] * 0x85EBCA6Bu) >> (32 - PRE_LOG);
-                    const uint32_t bit = 1u << (b & 31u);
-                    if (atomicOr(map1 + (b >> 5), bit) & bit) atomicOr(map2 + (b >> 5), bit);
-                }
-            }
-            __syncthreads();
-#pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-                if ((unres >> j) & 1u) {
-                    const uint32_t b = (h32[j] * 0x85EBCA6Bu) >> (32 - PRE_LOG);
-                    if (!((map2[b >> 5] >> (b & 31u)) & 1u)) unres &= ~(1u << j);   // nobody shares this hash: unique
-                }
-            }
-        }
-        for (int round = 0; round < CD_MAX_ROUNDS; ++round) {
-            const uint32_t mult = 0x9E3779B1u + 2u * (uint32_t)round * 0x632BE5ABu;   // odd for every round
-            const uint32_t add = (uint32_t)round * 0x7F4A7C15u;
-            if (unres) {
-#pragma unroll
-                for (int j = 0; j < RPT; ++j)
-                    if ((unres >> j) & 1u) table[(h32[j] * mult + add) >> (32 - LOG_SLOTS)] = (h32[j] & 0xffff0000u) | (tid + j * THREADS);
-            }
-            if (!__syncthreads_or(unres != 0u)) break;
-            if (unres) {
-#pragma unroll
-                for (int j = 0; j < RPT; ++j) {
-                    if ((unres >> j) & 1u) {
-                        const uint32_t mine = (h32[j] & 0xffff0000u) | (tid + j * THREADS);
-                        const uint32_t v = table[(h32[j] * mult + add) >> (32 - LOG_SLOTS)];
-                        if (v == mine) {
-                            winm |= 1u << j;
-                            unres &= ~(1u << j);
-                        } else if (((v ^ mine) >> 16) == 0u) {
-                            rr[j] = v & 0xffffu;
-                            atomicOr(mate + (rr[j] >> 5), 1u << (rr[j] & 31u));
-                            candm |= 1u << j;
-                            unres &= ~(1u << j);
-                        }
-                    }
-                }
-            }
-            __syncthreads();
-        }
-        candm |= unres;
-#pragma unroll
-        for (int j = 0; j < RPT; ++j)
-            if (((winm >> j) & 1u) && ((mate[(tid + j * THREADS) >> 5] >> (tid & 31)) & 1u)) candm |= 1u << j;
-        if (check_thr) {   // unique rows survive unless their own coefficient fails the threshold
+            uint32_t fi[RPT];
+            uint32_t live = 0, surv = 0;
 #pragma unroll
             for (int j = 0; j < RPT; ++j) {
                 const uint32_t i = tid + j * THREADS;
-                if (i < total && !((candm >> j) & 1u)) {
+                fi[j] = 0;
+                if (i < total) {
                     const uint32_t pr = pairs[i];
-                    const uint32_t t = J.vq[pr & vmask] * J.M_total + J.lookp[pr >> vbits];
-                    double re, im;
-                    rows.coeff_unphased(t, re, im);
-                    if (!keep_test(re, im, thr)) tm.mark_dropped(t);
+                    fi[j] = cd_filter_index<PRE_LOG>((__ldg(J.look8 + (pr >> vbits)) ^ __ldg(J.vsk + (pr & vmask))) & J.key_mask);
+                    const uint32_t bit = 1u << (fi[j] & 31u);
+                    if (atomicOr(map1 + (fi[j] >> 5), bit) & bit) atomicOr(map2 + (fi[j] >> 5), bit);
+                    live |= 1u << j;
                 }
             }
-        }
-        if (__syncthreads_or(candm != 0u)) {
-            uint32_t *cnt = table;   // CAP group counters, then their offsets
-            for (int i = tid; i < CAP; i += THREADS) cnt[i] = 0u;
             __syncthreads();
-            bool slow = (candm & unres) != 0u;
 #pragma unroll
             for (int j = 0; j < RPT; ++j)
-                if (((candm & ~unres) >> j) & 1u) rr[j] |= atomicAdd(cnt + rr[j], 1u) << 16;
-            __syncthreads();
-            uint32_t sum = 0;
+                if (((live >> j) & 1u) && ((map2[fi[j] >> 5] >> (fi[j] & 31u)) & 1u)) surv |= 1u << j;
+            if (check_thr) {
 #pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-                const uint32_t cj = cnt[tid + j * THREADS];
-                slow |= cj > (uint32_t)CD_SMALL_GROUP;
-                sum += cj;
+                for (int j = 0; j < RPT; ++j)
+                    if (((live & ~surv) >> j) & 1u) drop_if_small(pairs[tid + j * THREADS]);
             }
-            if (!__syncthreads_or(slow)) {
-                uint32_t nc;
-                const uint32_t first = cd_block_prefix<THREADS>(sum, s_warp, &s_ncand, nc);
-                if (tid == 0) s_base = atomicAdd(counters, nc);
-                uint32_t base = first;
+            uint32_t pos = cd_block_prefix<THREADS>((uint32_t)__popc(surv), s_warp, &s_nsurv, n_surv);
 #pragma unroll
-                for (int j = 0; j < RPT; ++j) {
-                    const uint32_t cj = cnt[tid + j * THREADS];
-                    cnt[tid + j * THREADS] = base;
-                    base += cj;
+            for (int j = 0; j < RPT; ++j)
+                if ((surv >> j) & 1u) list[pos++] = (uint16_t)(tid + j * THREADS);
+            __syncthreads();
+        }
+        // ---- the survivors, NS list entries per thread (e = tid + s * THREADS; entries past n_surv are empty). NS is the
+        // smallest instance that holds the class's list, so a thread only issues the slots a list of this length can fill.
+        auto survivors = [&](auto ns_tag) {
+            constexpr int NS = decltype(ns_tag)::value;
+            // the top 32 bits of the mixed sketch are THE hash of this kernel; table entries are [hash : 16 | list index : 16]
+            uint32_t h32[NS];
+            uint32_t rr[NS];      // list index of the representative of the entry's hash group; later | rank << 16
+            uint32_t unres = 0, candm = 0, winm = 0;   // one bit per list entry: no slot yet / saw a same-hash entry / holds a slot
+#pragma unroll
+            for (int s = 0; s < NS; ++s) {
+                const uint32_t e = tid + s * THREADS;
+                h32[s] = 0;
+                rr[s] = e;
+                if (e < n_surv) {
+                    const uint32_t pr = pairs[record_of(e)];
+                    h32[s] = (uint32_t)((mix64(__ldg(J.look8 + (pr >> vbits)) ^ __ldg(J.vsk + (pr & vmask))) & J.key_mask) >> 32);
+                    unres |= 1u << s;
                 }
-                __syncthreads();
-                uint64_t *dst = cand + s_base;
+            }
+            for (int round = 0; round < CD_MAX_ROUNDS; ++round) {
+                const uint32_t mult = 0x9E3779B1u + 2u * (uint32_t)round * 0x632BE5ABu;   // odd for every round
+                const uint32_t add = (uint32_t)round * 0x7F4A7C15u;
+                if (unres) {
 #pragma unroll
-                for (int j = 0; j < RPT; ++j) {
-                    if ((candm >> j) & 1u) {
-                        const uint32_t pr = pairs[tid + j * THREADS];
-                        const uint32_t v = pr & vmask, lo = pr >> vbits;
-                        const int b = J.nblk == 1 ? 0 : (int)(J.vkey[v] >> (J.k + 1));
-                        dst[cnt[rr[j] & 0xffffu] + (rr[j] >> 16)] =
-                            ((uint64_t)(h32[j] >> (32 - J.hbits)) << 32) | cd_ord_of(J, b, J.lookp[lo], J.vq[v]);
+                    for (int s = 0; s < NS; ++s) {
+                        if ((unres >> s) & 1u) table[(h32[s] * mult + add) >> (32 - LOG_SLOTS)] = (h32[s] & 0xffff0000u) | (tid + s * THREADS);
                     }
                 }
-                __syncthreads();
-                // the thread that owns a representative orders its group (2-3 records) by enumeration position
+                if (!__syncthreads_or(unres != 0u)) break;
+                if (unres) {
 #pragma unroll
-                for (int j = 0; j < RPT; ++j) {
-                    const uint32_t off_j = cnt[tid + j * THREADS];
-                    const uint32_t end_j = j + 1 < RPT ? cnt[tid + (j + 1) * THREADS] : first + sum;
-                    const uint32_t cj = end_j - off_j;
-                    if (cj >= 2u) {
-                        uint64_t *seg = dst + off_j;
-                        for (uint32_t a = 1; a < cj; ++a) {
-                            const uint64_t key = seg[a];
-                            uint32_t bpos = a;
-                            while (bpos > 0 && seg[bpos - 1] > key) {
-                                seg[bpos] = seg[bpos - 1];
-                                --bpos;
+                    for (int s = 0; s < NS; ++s) {
+                        if ((unres >> s) & 1u) {
+                            const uint32_t mine = (h32[s] & 0xffff0000u) | (tid + s * THREADS);
+                            const uint32_t v = table[(h32[s] * mult + add) >> (32 - LOG_SLOTS)];
+                            if (v == mine) {
+                                winm |= 1u << s;
+                                unres &= ~(1u << s);
+                            } else if (((v ^ mine) >> 16) == 0u) {
+                                rr[s] = v & 0xffffu;
+                                atomicOr(mate + (rr[s] >> 5), 1u << (rr[s] & 31u));
+                                candm |= 1u << s;
+                                unres &= ~(1u << s);
                             }
-                            seg[bpos] = key;
                         }
                     }
                 }
                 __syncthreads();
-                for (uint32_t i = tid; i < nc; i += THREADS) {   // [hash | ord] -> candidate record [hash | t | 0]
-                    const uint64_t key = dst[i];
-                    dst[i] = ((key >> 32) << (64 - J.hbits)) | ((uint64_t)cd_t_of_ord(J, (uint32_t)key) << 2);
-                }
-            } else {
-                // a large hash group (a square's identity terms, a molecular H*H) or records without a slot: this class's
-                // candidates take the global sort with the overflowed classes
-                uint32_t nc;
-                uint32_t pos = cd_block_prefix<THREADS>((uint32_t)__popc(candm), s_warp, &s_ncand, nc);
-                if (tid == 0) s_base = atomicAdd(counters + 1, nc);
-                __syncthreads();
-                const uint32_t ob = s_base;
+            }
+            // ---- candidates: saw a mate, was seen by one, or never found a free slot (then its mates did not either)
+            candm |= unres;
 #pragma unroll
-                for (int j = 0; j < RPT; ++j) {
-                    if ((candm >> j) & 1u) {
-                        const uint32_t pr = pairs[tid + j * THREADS];
-                        const uint32_t v = pr & vmask, lo = pr >> vbits;
-                        const int b = J.nblk == 1 ? 0 : (int)(J.vkey[v] >> (J.k + 1));
-                        const uint64_t ord = cd_ord_of(J, b, J.lookp[lo], J.vq[v]);
-                        over[(size_t)ob + pos++] = ((((uint64_t)h32[j] << 32) >> (J.tb + 2)) << (J.tb + 2)) | (ord << 2);
+            for (int s = 0; s < NS; ++s) {
+                if (((winm >> s) & 1u) && ((mate[(tid + s * THREADS) >> 5] >> (tid & 31)) & 1u)) candm |= 1u << s;
+            }
+            if (check_thr) {
+#pragma unroll
+                for (int s = 0; s < NS; ++s) {
+                    const uint32_t e = tid + s * THREADS;
+                    if (e < n_surv && !((candm >> s) & 1u)) drop_if_small(pairs[record_of(e)]);
+                }
+            }
+            if (__syncthreads_or(candm != 0u)) {
+                uint32_t *cnt = table;   // group counters by list index, then their offsets
+#pragma unroll
+                for (int s = 0; s < NS; ++s) {
+                    cnt[tid + s * THREADS] = 0u;
+                }
+                __syncthreads();
+                bool slow = (candm & unres) != 0u;
+#pragma unroll
+                for (int s = 0; s < NS; ++s) {
+                    if (((candm & ~unres) >> s) & 1u) rr[s] |= atomicAdd(cnt + rr[s], 1u) << 16;
+                }
+                __syncthreads();
+                uint32_t sum = 0;
+#pragma unroll
+                for (int s = 0; s < NS; ++s) {
+                    const uint32_t cj = cnt[tid + s * THREADS];
+                    slow |= cj > (uint32_t)CD_SMALL_GROUP;
+                    sum += cj;
+                }
+                if (!__syncthreads_or(slow)) {
+                    uint32_t nc;
+                    const uint32_t first = cd_block_prefix<THREADS>(sum, s_warp, &s_ncand, nc);
+                    if (tid == 0) s_base = atomicAdd(counters, nc);
+                    uint32_t base = first;
+#pragma unroll
+                    for (int s = 0; s < NS; ++s) {
+                        const uint32_t cj = cnt[tid + s * THREADS];
+                        cnt[tid + s * THREADS] = base;
+                        base += cj;
+                    }
+                    __syncthreads();
+                    uint64_t *dst = cand + s_base;
+#pragma unroll
+                    for (int s = 0; s < NS; ++s) {
+                        if ((candm >> s) & 1u) {
+                            const uint32_t pr = pairs[record_of(tid + s * THREADS)];
+                            const uint32_t v = pr & vmask, lo = pr >> vbits;
+                            const int b = J.nblk == 1 ? 0 : (int)(J.vkey[v] >> (J.k + 1));
+                            dst[cnt[rr[s] & 0xffffu] + (rr[s] >> 16)] =
+                                ((uint64_t)(h32[s] >> (32 - J.hbits)) << 32) | cd_ord_of(J, b, J.lookp[lo], J.vq[v]);
+                        }
+                    }
+                    __syncthreads();
+                    // the thread that owns a representative orders its group (2-3 records) by enumeration position
+#pragma unroll
+                    for (int s = 0; s < NS; ++s) {
+                        const uint32_t off_s = cnt[tid + s * THREADS];
+                        const uint32_t end_s = s + 1 < NS ? cnt[tid + (s + 1) * THREADS] : first + sum;
+                        const uint32_t cj = end_s - off_s;
+                        if (cj >= 2u) {
+                            uint64_t *seg = dst + off_s;
+                            for (uint32_t a = 1; a < cj; ++a) {
+                                const uint64_t key = seg[a];
+                                uint32_t bpos = a;
+                                while (bpos > 0 && seg[bpos - 1] > key) {
+                                    seg[bpos] = seg[bpos - 1];
+                                    --bpos;
+                                }
+                                seg[bpos] = key;
+                            }
+                        }
+                    }
+                    __syncthreads();
+                    for (uint32_t i = tid; i < nc; i += THREADS) {   // [hash | ord] -> candidate record [hash | t | 0]
+                        const uint64_t key = dst[i];
+                        dst[i] = ((key >> 32) << (64 - J.hbits)) | ((uint64_t)cd_t_of_ord(J, (uint32_t)key) << 2);
+                    }
+                } else {
+                    // a large hash group (a square's identity terms, a molecular H*H) or records without a slot: this class's
+                    // candidates take the global sort with the overflowed classes
+                    uint32_t nc;
+                    uint32_t pos = cd_block_prefix<THREADS>((uint32_t)__popc(candm), s_warp, &s_ncand, nc);
+                    if (tid == 0) s_base = atomicAdd(counters + 1, nc);
+                    __syncthreads();
+                    const uint32_t ob = s_base;
+#pragma unroll
+                    for (int s = 0; s < NS; ++s) {
+                        if ((candm >> s) & 1u) {
+                            const uint32_t pr = pairs[record_of(tid + s * THREADS)];
+                            const uint32_t v = pr & vmask, lo = pr >> vbits;
+                            const int b = J.nblk == 1 ? 0 : (int)(J.vkey[v] >> (J.k + 1));
+                            const uint64_t ord = cd_ord_of(J, b, J.lookp[lo], J.vq[v]);
+                            over[(size_t)ob + pos++] = ((((uint64_t)h32[s] << 32) >> (J.tb + 2)) << (J.tb + 2)) | (ord << 2);
+                        }
                     }
                 }
             }
-        }
+        };
+        // block-uniform. The 2 / 4 / 8 instances pay on duplicate-heavy products: the span-28 product of bench.py fills
+        // ~6 entries per thread, and its class kernel takes 2.53 ms with them, 2.77 ms with the 18-entry one (B200)
+        const uint32_t ns = (n_surv + THREADS - 1) / THREADS;
+        if (ns <= 1) survivors(std::integral_constant<int, 1>());
+        else if (ns <= 2) survivors(std::integral_constant<int, 2>());
+        else if (ns <= 4) survivors(std::integral_constant<int, 4>());
+        else if (ns <= 8) survivors(std::integral_constant<int, 8>());
+        else survivors(std::integral_constant<int, RPT>());
         __syncthreads();
     }
 }
