@@ -355,17 +355,14 @@ size_t sym_sort_pairs_ws_bytes(int64_t T);
 int sym_sort_pairs(uint64_t *keys, uint32_t *vals, int64_t T, int32_t begin_bit, void *ws,
                    size_t ws_bytes, void *stream);
 /* Tuning knobs (A/B switches kept for measurement). which = 0: cross-term count up to which
- * sym_mul_cleanup scatters by t (above it: knob 6; default 2^22); 1: row emission (0 two kernels, 1 CTA-fused, 2 warp-fused); 2: radix scatter shape;
- * 3: extra sort bits; 4: apply/expval kernel (1 binned, 0 four-row); 5: GF(2) large path (1 blocked
- * panels, 0 one pivot per sweep); 6: large products in ordered-tile mode (1, default) or sorted-hash
- * order (0); 7: B rows per CTA of the tiled row emission (default 16); 8: record sort as one-sweep
- * passes with decoupled look-back (1, default) or histogram + scan + scatter per pass (0); 9: in
- * ordered-tile mode the first radix pass generates the records itself (1) or pair_keys_kernel writes them
- * first (0, default: measured faster); 10: duplicate detection of ordered-tile products by class-local
+ * sym_mul_cleanup scatters by t (above it: knob 6; default 2^22); 4: apply/expval kernel (1 binned,
+ * 0 four-row); 5: GF(2) large path (1 blocked panels, 0 one pivot per sweep); 6: large products in
+ * ordered-tile mode (1, default) or sorted-hash order (0); 7: B rows per CTA of the tiled row emission
+ * (default 16); 8: record sort as one-sweep passes with decoupled look-back (1, default) or histogram +
+ * scan + scatter per pass (0); 10: duplicate detection of ordered-tile products by class-local
  * enumeration (1, default) or by the global record sort (0); 11: class kernel shape (2, default: compact
  * 4-byte entries with the presence filter; 3: the same without the filter, 128 KB table; 1: 8-byte entries,
- * 9216 records per class; 0: 512-thread CTAs, 4096 records); 12: tensor-core commute kernel (2, default:
- * warp-specialised, 2 stages, 2 CTAs/SM; 1, 3, 4: other stage / expander-warp counts; 0: the round-1 kernel). */
+ * 9216 records per class; 0: 512-thread CTAs, 4096 records). Any other number is SYM_E_INVALID. */
 int sym_set_tuning(int32_t which, int64_t value);
 /* Measurement hook: two cudaEvent_t (as void*, NULL to disable) recorded on the stream immediately
  * before and after the row-emission kernel (emit_kernel) of the next *_emit calls, so that a

@@ -4,11 +4,19 @@
 // (`matmul_GF2`: integer GEMM then mod 2, utils.py:63-78) with exact int32 accumulation in TMEM.
 //
 // One CTA computes a 128 (A rows) x 256 (B rows) tile of the output. The packed operands (16 B of
-// bits per row and stage) are read from L2 and expanded on the fly to 0/1 bytes in shared memory in
-// the canonical K-major no-swizzle UMMA layout (8-row x 16-byte core matrices), double-buffered:
-// while the tensor core consumes stage s (4 x tcgen05.mma kind::i8, M=128 N=256 K=32), all warps
-// expand stage s+1. Completion is tracked with tcgen05.commit -> mbarrier. Epilogue: tcgen05.ld of
-// the int32 accumulators, parity, byte stores. Never pre-unpacks the operands in HBM (8x the bytes).
+// bits per row and stage) are read from L2 and expanded on the fly to operand bytes in shared memory in
+// the canonical K-major no-swizzle UMMA layout (8-row x 16-byte core matrices). The kernel is
+// warp-specialised: EXPANDER warps turn packed bits into operand bytes, one ISSUER warp feeds the tensor
+// core (4 x tcgen05.mma kind::i8, M=128 N=256 K=32 per stage); they meet only through mbarriers
+// (full[s]: every expander has written stage s; empty[s]: the MMAs that read stage s have completed,
+// signalled by tcgen05.commit), so there is no block-wide barrier in the main loop and the tensor core
+// works on stage s while the next stage is being expanded. Epilogue: tcgen05.ld of the int32
+// accumulators, parity, byte stores. Never pre-unpacks the operands in HBM (8x the bytes).
+//
+// Shape: 2 stages of 48 KB, 8 expander warps, two CTAs per SM (256 TMEM columns each). Measured on B200
+// at 1000 qubits: 5.7e11 pairs/s, against 4.4e11 for a form where all warps expand and meet the MMAs at
+// a block barrier, and 4.0e11 for one CTA per SM with 3-4 stages and 8 or 16 expander warps: the
+// expansion (ALU) needs the second CTA's warps to hide its latency.
 #include "common.cuh"
 
 namespace symb {
@@ -20,7 +28,7 @@ constexpr int STAGE_WORDS = 2;                      // 64-bit words of packed bi
 constexpr int STAGE_KBYTES = STAGE_WORDS * 64;      // 128 unpacked bytes of K per stage
 constexpr int A_STAGE_BYTES = MMA_M * STAGE_KBYTES; // 16 KB
 constexpr int B_STAGE_BYTES = MMA_N * STAGE_KBYTES; // 32 KB
-constexpr int NUM_STAGES = 2;
+constexpr int MMA_STAGES = 2;
 constexpr int TMEM_COLS = 256;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -87,18 +95,6 @@ __device__ __forceinline__ uint4 expand16(uint32_t bits) {
     return v;
 }
 
-// Expand one row's 128 bits (two packed words) into the stage buffer. `rows` = rows of this operand
-// tile (128 or 256); chunk c of row r lives at c*rows*16 + (r/8)*128 + (r%8)*16.
-__device__ __forceinline__ void expand_row(unsigned char *stage, int rows, int r, uint64_t w0, uint64_t w1) {
-    unsigned char *base = stage + (r >> 3) * 128 + (r & 7) * 16;
-    const uint32_t lbo = (uint32_t)rows * 16u;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-        *reinterpret_cast<uint4 *>(base + c * lbo) = expand16((uint32_t)(w0 >> (16 * c)) & 0xFFFFu);
-        *reinterpret_cast<uint4 *>(base + (4 + c) * lbo) = expand16((uint32_t)(w1 >> (16 * c)) & 0xFFFFu);
-    }
-}
-
 // Word-major copies of the operands: t[k][row] = word k of row `row` (for B with the X and Z halves
 // swapped, so that A'.B'^T is the symplectic form). With this layout the per-stage reads of a tile
 // are coalesced (consecutive rows -> consecutive 8-byte words).
@@ -122,139 +118,6 @@ __global__ void __launch_bounds__(256) transpose_words_kernel(const uint64_t *__
     }
 }
 
-__global__ void __launch_bounds__(MMA_THREADS, 2) commute_mma_kernel(const uint64_t *__restrict__ a_t, uint32_t M,
-                                                                      const uint64_t *__restrict__ b_t, uint32_t N, int W,
-                                                                      uint8_t *__restrict__ out, size_t pitch) {
-    extern __shared__ __align__(1024) unsigned char smem[];
-    unsigned char *sA[NUM_STAGES], *sB[NUM_STAGES];
-#pragma unroll
-    for (int s = 0; s < NUM_STAGES; ++s) {
-        sA[s] = smem + s * (A_STAGE_BYTES + B_STAGE_BYTES);
-        sB[s] = sA[s] + A_STAGE_BYTES;
-    }
-    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + NUM_STAGES * (A_STAGE_BYTES + B_STAGE_BYTES));  // [0..1] stage free, [2] done
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 4);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t i0 = blockIdx.y * MMA_M, j0 = blockIdx.x * MMA_N;
-
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        mbar_init(&bars[2], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
-
-    const uint32_t idesc = make_idesc_i8(MMA_M, MMA_N);
-    const int words = 2 * W;               // K in packed words; A' = [x | z], B' = [z | x]
-    const int iters = words / STAGE_WORDS;  // 2W is even
-
-    // this thread's rows: one B row, and (threads 0..127) one A row
-    const uint32_t jb = j0 + tid;
-    const bool b_ok = jb < N;
-    const uint32_t ia = i0 + tid;
-    const bool a_ok = tid < MMA_M && ia < M;
-
-    // software pipeline: the packed words of iteration it+1 are fetched (coalesced reads of the
-    // word-major operands) while iteration it is expanded
-    auto fetch = [&](int it, uint64_t &bw0, uint64_t &bw1, uint64_t &aw0, uint64_t &aw1) {
-        const size_t k0 = (size_t)it * STAGE_WORDS;
-        bw0 = b_ok ? b_t[k0 * N + jb] : 0ull;
-        bw1 = b_ok ? b_t[(k0 + 1) * N + jb] : 0ull;
-        aw0 = a_ok ? a_t[k0 * M + ia] : 0ull;
-        aw1 = a_ok ? a_t[(k0 + 1) * M + ia] : 0ull;
-    };
-    uint64_t bw0, bw1, aw0, aw1;
-    fetch(0, bw0, bw1, aw0, aw1);
-    for (int it = 0; it < iters; ++it) {
-        const int s = it & 1;
-        uint64_t nb0 = 0, nb1 = 0, na0 = 0, na1 = 0;
-        if (it + 1 < iters) fetch(it + 1, nb0, nb1, na0, na1);
-        if (it >= NUM_STAGES) mbar_wait(&bars[s], ((it >> 1) - 1) & 1);   // MMAs that read this buffer are done
-        expand_row(sB[s], MMA_N, tid, bw0, bw1);
-        if (tid < MMA_M) expand_row(sA[s], MMA_M, tid, aw0, aw1);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the tensor core
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint32_t a_addr = smem_u32(sA[s]), b_addr = smem_u32(sB[s]);
-#pragma unroll
-            for (int kk = 0; kk < STAGE_KBYTES / 32; ++kk) {
-                const uint64_t da = make_smem_desc(a_addr + kk * 2 * (MMA_M * 16), MMA_M * 16, 128);
-                const uint64_t db = make_smem_desc(b_addr + kk * 2 * (MMA_N * 16), MMA_N * 16, 128);
-                umma_i8(tmem_base, da, db, idesc, (it > 0 || kk > 0) ? 1u : 0u);
-            }
-            umma_commit(&bars[s]);
-            if (it == iters - 1) umma_commit(&bars[2]);
-        }
-        bw0 = nb0; bw1 = nb1; aw0 = na0; aw1 = na1;
-    }
-    mbar_wait(&bars[2], 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-
-    // epilogue: warp w reads TMEM lanes 32*(w%4).., columns 128*(w/4)..; thread = one output row
-    const uint32_t row = i0 + (warp & 3) * 32 + lane;
-    const uint32_t col_half = (warp >> 2) * 128;
-#pragma unroll 1
-    for (int cb = 0; cb < 128; cb += 32) {
-        uint32_t v[32];
-        const uint32_t taddr = tmem_base + (((uint32_t)(warp & 3) * 32u) << 16) + col_half + cb;
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-            "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-              "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-              "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-              "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-            : "r"(taddr));
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        if (row < M) {
-            const uint32_t jbase = j0 + col_half + cb;
-            // pitch = bytes between output rows (>= N). With a pitch that is a multiple of 32 every 32-byte chunk
-            // is aligned and may spill into the row's padding, so the vector stores cover ragged N too.
-            uint8_t *dst = out + (size_t)row * pitch + jbase;
-            if (jbase + 32 <= pitch && ((reinterpret_cast<uintptr_t>(dst) & 15) == 0)) {
-                uint32_t p[8];
-#pragma unroll
-                for (int q = 0; q < 8; ++q)
-                    p[q] = ((v[4 * q] & 1u) ^ 1u) | (((v[4 * q + 1] & 1u) ^ 1u) << 8) | (((v[4 * q + 2] & 1u) ^ 1u) << 16) |
-                           (((v[4 * q + 3] & 1u) ^ 1u) << 24);
-                reinterpret_cast<uint4 *>(dst)[0] = make_uint4(p[0], p[1], p[2], p[3]);
-                reinterpret_cast<uint4 *>(dst)[1] = make_uint4(p[4], p[5], p[6], p[7]);
-            } else {
-#pragma unroll
-                for (int q = 0; q < 32; ++q)
-                    if (jbase + q < N) dst[q] = (uint8_t)((v[q] & 1u) ^ 1u);
-            }
-        }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// Warp-specialised form (tuning knob 12 >= 1, the default): EXPANDER warps turn packed bits into operand
-// bytes, one ISSUER warp feeds the tensor core; they meet only through mbarriers (full[s]: every
-// expander has written stage s; empty[s]: the MMAs that read stage s have completed, signalled by
-// tcgen05.commit), so there is no block-wide barrier in the main loop and the tensor core works on
-// stage s while the next stage is being expanded. Default shape: 2 stages of 48 KB, 8 expander warps,
-// two CTAs per SM (256 TMEM columns each) — deeper pipelines with one CTA per SM measured slower,
-// the expansion (ALU) needs the second CTA's warps to hide its latency.
-// ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -267,24 +130,22 @@ __device__ __forceinline__ void expand_word(unsigned char *stage, int rows, int 
     for (int c = 0; c < 4; ++c) *reinterpret_cast<uint4 *>(base + (c0 + c) * lbo) = expand16((uint32_t)(w >> (16 * c)) & 0xFFFFu);
 }
 
-// STAGES x 48 KB of operand bytes; HALVES = 1: 8 expander warps, a thread expands both words of its rows;
-// HALVES = 2: 16 expander warps, a thread expands one word (more warps per scheduler to hide the ALU latency)
-template <int STAGES, int HALVES, int MINB>
-__global__ void __launch_bounds__(MMA_THREADS * HALVES + 32, MINB) commute_mma_ws_kernel(const uint64_t *__restrict__ a_t, uint32_t M,
-                                                                                          const uint64_t *__restrict__ b_t, uint32_t N,
-                                                                                          int W, uint8_t *__restrict__ out, size_t pitch) {
-    constexpr int EXPANDERS = MMA_THREADS * HALVES;
+// MMA_STAGES x 48 KB of operand bytes; 8 expander warps, a thread expands both words of its rows
+__global__ void __launch_bounds__(MMA_THREADS + 32, 2) commute_mma_ws_kernel(const uint64_t *__restrict__ a_t, uint32_t M,
+                                                                             const uint64_t *__restrict__ b_t, uint32_t N, int W,
+                                                                             uint8_t *__restrict__ out, size_t pitch) {
+    constexpr int EXPANDERS = MMA_THREADS;
     extern __shared__ __align__(1024) unsigned char smem[];
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem + STAGES * (A_STAGE_BYTES + B_STAGE_BYTES));
-    uint64_t *empty = full + STAGES;
-    uint64_t *done = empty + STAGES;
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem + MMA_STAGES * (A_STAGE_BYTES + B_STAGE_BYTES));
+    uint64_t *empty = full + MMA_STAGES;
+    uint64_t *done = empty + MMA_STAGES;
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(done + 1);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const uint32_t i0 = blockIdx.y * MMA_M, j0 = blockIdx.x * MMA_N;
     if (tid == 0) {
 #pragma unroll
-        for (int s = 0; s < STAGES; ++s) {
+        for (int s = 0; s < MMA_STAGES; ++s) {
             mbar_init(&full[s], EXPANDERS);
             mbar_init(&empty[s], 1);
         }
@@ -320,23 +181,23 @@ __global__ void __launch_bounds__(MMA_THREADS * HALVES + 32, MINB) commute_mma_w
                 }
                 umma_commit(&empty[s]);
                 if (it == iters - 1) umma_commit(done);
-                if (++s == STAGES) {
+                if (++s == MMA_STAGES) {
                     s = 0;
                     ph ^= 1u;
                 }
             }
         }
     } else {
-        // ---- expander warps: thread = (B row, word half) and, for rows < 128, the same of an A row
-        const int r = tid % MMA_THREADS, half = tid / MMA_THREADS;   // half = 0 when HALVES == 1
+        // ---- expander warps: thread = B row and, for rows < 128, an A row
+        const int r = tid;
         const uint32_t jb = j0 + r;
         const bool b_ok = jb < N;
         const uint32_t ia = i0 + r;
         const bool a_ok = r < MMA_M && ia < M;
         uint64_t bw[2], aw[2];
 #pragma unroll
-        for (int h = 0; h < 2 / HALVES; ++h) {
-            const size_t k = (size_t)(HALVES == 2 ? half : h);
+        for (int h = 0; h < 2; ++h) {
+            const size_t k = (size_t)h;
             bw[h] = b_ok ? b_t[k * N + jb] : 0ull;
             aw[h] = a_ok ? a_t[k * M + ia] : 0ull;
         }
@@ -346,28 +207,28 @@ __global__ void __launch_bounds__(MMA_THREADS * HALVES + 32, MINB) commute_mma_w
             uint64_t nb[2] = {0ull, 0ull}, na[2] = {0ull, 0ull};
             if (it + 1 < iters) {
 #pragma unroll
-                for (int h = 0; h < 2 / HALVES; ++h) {
-                    const size_t k = (size_t)(it + 1) * STAGE_WORDS + (HALVES == 2 ? half : h);
+                for (int h = 0; h < 2; ++h) {
+                    const size_t k = (size_t)(it + 1) * STAGE_WORDS + h;
                     nb[h] = b_ok ? b_t[k * N + jb] : 0ull;
                     na[h] = a_ok ? a_t[k * M + ia] : 0ull;
                 }
             }
-            if (it >= STAGES) mbar_wait(&empty[s], ph ^ 1u);
+            if (it >= MMA_STAGES) mbar_wait(&empty[s], ph ^ 1u);
             unsigned char *stA = smem + s * (A_STAGE_BYTES + B_STAGE_BYTES), *stB = stA + A_STAGE_BYTES;
 #pragma unroll
-            for (int h = 0; h < 2 / HALVES; ++h) {
-                const int c0 = 4 * (HALVES == 2 ? half : h);
+            for (int h = 0; h < 2; ++h) {
+                const int c0 = 4 * h;
                 expand_word(stB, MMA_N, r, c0, bw[h]);
                 if (r < MMA_M) expand_word(stA, MMA_M, r, c0, aw[h]);
             }
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the tensor core
             mbar_arrive(&full[s]);
 #pragma unroll
-            for (int h = 0; h < 2 / HALVES; ++h) {
+            for (int h = 0; h < 2; ++h) {
                 bw[h] = nb[h];
                 aw[h] = na[h];
             }
-            if (++s == STAGES) {
+            if (++s == MMA_STAGES) {
                 s = 0;
                 ph ^= 1u;
             }
@@ -419,9 +280,6 @@ __global__ void __launch_bounds__(MMA_THREADS * HALVES + 32, MINB) commute_mma_w
     }
 }
 
-int g_commute_variant = 2;   // tuning knob 12 (default 2, measured fastest on B200: 5.3e11 pairs/s at 1000 q against 4.4e11 for 0): 0 = all warps expand + block barrier (2 CTAs/SM); warp-specialised: 1 = 3 stages x 8 expander
-                             // warps, 2 = 2 stages x 8 warps x 2 CTAs/SM, 3 = 3 stages x 16 expander warps, 4 = 4 stages x 16 warps
-
 }  // namespace symb
 
 using namespace symb;
@@ -456,30 +314,18 @@ extern "C" int sym_commute_mma_pitched(const uint64_t *a_xz, int64_t M, const ui
     transpose_words_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((words + 31) / 32)), 256, 0, st>>>(b_xz, (uint32_t)N,
                                                                                                         words, 1, b_t);
     SYM_LAUNCH_OK();
-    constexpr size_t smem = NUM_STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 64;
-    constexpr size_t stage_bytes = A_STAGE_BYTES + B_STAGE_BYTES;
+    constexpr size_t smem = MMA_STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 128;
     static bool attr_done[64] = {};   // per device
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel<3, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(3 * stage_bytes + 128)));
-        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel<2, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * stage_bytes + 128)));
-        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel<3, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(3 * stage_bytes + 128)));
-        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel<4, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(4 * stage_bytes + 128)));
+        SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
     const int64_t tiles_m = (M + MMA_M - 1) / MMA_M;
     SYM_REQUIRE(tiles_m <= 65535, "too many A rows for one launch (slice A)");
     dim3 grid((unsigned)((N + MMA_N - 1) / MMA_N), (unsigned)tiles_m);
-#define WS_LAUNCH(ST, HV, MB) \
-    commute_mma_ws_kernel<ST, HV, MB><<<grid, MMA_THREADS * HV + 32, ST * stage_bytes + 128, st>>>(a_t, (uint32_t)M, b_t, (uint32_t)N, W, out, (size_t)out_pitch)
-    if (g_commute_variant == 1) WS_LAUNCH(3, 1, 1);
-    else if (g_commute_variant == 2) WS_LAUNCH(2, 1, 2);
-    else if (g_commute_variant == 3) WS_LAUNCH(3, 2, 1);
-    else if (g_commute_variant == 4) WS_LAUNCH(4, 2, 1);
-    else
-        commute_mma_kernel<<<grid, MMA_THREADS, smem, st>>>(a_t, (uint32_t)M, b_t, (uint32_t)N, W, out, (size_t)out_pitch);
+    commute_mma_ws_kernel<<<grid, MMA_THREADS + 32, smem, st>>>(a_t, (uint32_t)M, b_t, (uint32_t)N, W, out, (size_t)out_pitch);
     SYM_LAUNCH_OK();
     return SYM_OK;
 }

@@ -622,10 +622,8 @@ __global__ void total_to_i64_kernel(const uint32_t *__restrict__ total, int64_t 
 // 2*EMIT_UN independent 16-byte loads are in flight per thread (the kernel is latency-bound
 // otherwise). Stores are streaming (st.global.cs): the output is never re-read, and A/B must stay
 // L2-resident. LW: chunks per row = 1 << LW.
-// tuning knob 1: 0 = compaction kernel + emission kernel (default; measured fastest on B200: 7.1 ms for 1.25e8
-// rows of 272 B against 8.8 ms for the CTA-fused form, whose barrier between the two phases stalls the block),
-// 1 = CTA-fused, 2 = warp-fused
-int g_emit_variant = 0;
+// Compaction and emission are two kernels: measured on B200, 7.1 ms for 1.25e8 rows of 272 B against 8.8 ms
+// for a CTA-fused form, whose barrier between the two phases stalls the block.
 
 // optional CUDA events recorded around the row-emission kernel (sym_set_emit_events)
 static cudaEvent_t g_emit_ev0 = nullptr, g_emit_ev1 = nullptr;
@@ -673,131 +671,6 @@ __global__ void __launch_bounds__(256) emit_generic_kernel(Rows rows, const uint
     out_xz[g] = rows.chunk(kept_t[rec], (int)c);
 }
 
-// Fused compaction + row emission (the dominant kernel of a large product: HBM-write bound).
-// A CTA owns D = ROWS_PP*UN consecutive dedup positions; because slot[] is an exclusive scan of the
-// keep flags, its survivors occupy the contiguous output range [slot[d0], slot[d0] + count).
-// Phase 1 (first D threads): survivor -> term id into shared memory, final coefficient straight to
-// out_c (consecutive survivors write consecutive 16-byte slots). Phase 2 (all threads): thread =
-// (row, 16-byte chunk), UN rows in flight per thread, A[p]^B[q] gathered from the L2-resident
-// operands, 16-byte stores. No kept_t round trip through HBM and no separate compaction launch.
-template <class Rows, bool BY_T, int LW, int UN>
-__global__ void __launch_bounds__(256) emit_fused_kernel(Rows rows, RecFmt fmt, const uint64_t *__restrict__ sr,
-                                                          const uint8_t *__restrict__ keep, const uint8_t *__restrict__ multi,
-                                                          const uint32_t *__restrict__ slot, const double2 *__restrict__ acc,
-                                                          int64_t T, uint4 *__restrict__ out_xz, double2 *__restrict__ out_c) {
-    constexpr uint32_t ROWS_PP = 256u >> LW;
-    constexpr uint32_t D = ROWS_PP * UN;
-    static_assert(D <= 256, "one thread per position in phase 1");
-    __shared__ uint2 s_h[D];
-    __shared__ uint32_t s_count;
-    const int64_t d0 = (int64_t)blockIdx.x * D;
-    const uint32_t base = slot[d0];
-    if (threadIdx.x < D) {
-        const int64_t d = d0 + threadIdx.x;
-        uint8_t k = 0;
-        uint32_t s = 0;
-        if (d < T) {
-            k = keep[d];
-            s = slot[d];
-            if (k) {
-                uint32_t t;
-                int e = 0;
-                if (BY_T) {
-                    t = (uint32_t)d;
-                } else {
-                    const uint64_t rec = sr[d];
-                    t = fmt.t(rec);
-                    e = fmt.e(rec);
-                }
-                s_h[s - base] = rows.locate(t);
-                if (multi[d]) {
-                    out_c[s] = acc[d];
-                } else {   // singleton survivor: its coefficient was never materialised
-                    double re, im;
-                    rows.coeff(t, e, re, im);
-                    out_c[s] = make_double2(re, im);
-                }
-            }
-        }
-        if (d < T && (threadIdx.x == D - 1 || d == T - 1)) s_count = s + (uint32_t)k - base;
-    }
-    __syncthreads();
-    const uint32_t count = s_count;
-    const uint32_t r_in = threadIdx.x >> LW;
-    const uint32_t c = threadIdx.x & ((1u << LW) - 1u);
-    uint4 v[UN];
-#pragma unroll
-    for (int u = 0; u < UN; ++u) {
-        const uint32_t r = u * ROWS_PP + r_in;
-        if (r < count) v[u] = rows.chunk_at(s_h[r], (int)c);
-    }
-#pragma unroll
-    for (int u = 0; u < UN; ++u) {
-        const uint32_t r = u * ROWS_PP + r_in;
-        if (r < count) out_xz[(((size_t)base + r) << LW) + c] = v[u];
-    }
-}
-
-// Warp-level form of the fused compaction + emission: a warp owns 32 consecutive dedup positions, so
-// there is no CTA barrier and no idle half block. Phase 1: lane = position (survivor -> (p, q) handle
-// in the warp's shared-memory slice, coefficient straight to out_c); phase 2: lane = (row, 16-byte
-// chunk), 8 rows in flight per lane.
-template <class Rows, bool BY_T, int LW>
-__global__ void __launch_bounds__(256) emit_warp_kernel(Rows rows, RecFmt fmt, const uint64_t *__restrict__ sr,
-                                                         const uint8_t *__restrict__ keep, const uint8_t *__restrict__ multi,
-                                                         const uint32_t *__restrict__ slot, const double2 *__restrict__ acc,
-                                                         int64_t T, uint4 *__restrict__ out_xz, double2 *__restrict__ out_c) {
-    constexpr int RPP = 32 >> LW;            // rows per pass of one warp
-    constexpr int UN = (RPP * 8 <= 32) ? 8 : (32 / RPP);   // passes in flight
-    __shared__ uint2 s_h[8][32];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int64_t d0 = ((int64_t)blockIdx.x * 8 + wid) * 32;
-    if (d0 >= T) return;
-    const int64_t d = d0 + lane;
-    const uint8_t k = d < T ? keep[d] : 0;
-    const uint32_t bal = __ballot_sync(0xffffffffu, k != 0);
-    if (bal == 0u) return;
-    uint32_t base = lane == 0 ? slot[d0] : 0u;
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (k) {
-        const uint32_t local = __popc(bal & ((1u << lane) - 1u));
-        uint32_t t;
-        int e = 0;
-        if (BY_T) {
-            t = (uint32_t)d;
-        } else {
-            const uint64_t rec = sr[d];
-            t = fmt.t(rec);
-            e = fmt.e(rec);
-        }
-        s_h[wid][local] = rows.locate(t);
-        if (multi[d]) {
-            out_c[base + local] = acc[d];
-        } else {
-            double re, im;
-            rows.coeff(t, e, re, im);
-            out_c[base + local] = make_double2(re, im);
-        }
-    }
-    __syncwarp();
-    const int count = __popc(bal);
-    const int r_in = lane >> LW;
-    const int c = lane & ((1 << LW) - 1);
-    for (int r0 = 0; r0 < count; r0 += RPP * UN) {
-        uint4 v[UN];
-#pragma unroll
-        for (int u = 0; u < UN; ++u) {
-            const int r = r0 + u * RPP + r_in;
-            if (r < count) v[u] = rows.chunk_at(s_h[wid][r], c);
-        }
-#pragma unroll
-        for (int u = 0; u < UN; ++u) {
-            const int r = r0 + u * RPP + r_in;
-            if (r < count) out_xz[(((size_t)base + r) << LW) + c] = v[u];
-        }
-    }
-}
-
 size_t dedup_ws_bytes(int64_t T) {
     if (T < 1) T = 1;
     size_t n = (size_t)T;
@@ -814,13 +687,13 @@ size_t dedup_ws_bytes(int64_t T) {
            + arena_need(16, 4) + 4096;
 }
 
-// Sort on log2(T) + g_sort_extra_bits hash bits, rounded up to whole 8-bit passes. A sort bucket then
+// Sort on log2(T) + SORT_EXTRA_BITS hash bits, rounded up to whole 8-bit passes. A sort bucket then
 // holds T / 2^bits records on average, which link/sum resolve exactly with in-bucket scans: fewer
 // bits save radix passes (24 B of HBM traffic per record each) but lengthen those scans.
-int g_sort_extra_bits = 5;  // tuning knob 3
+constexpr int SORT_EXTRA_BITS = 5;
 static int sort_begin_bit(int64_t T, RecFmt fmt) {
     int lg = t_bits_for(T);
-    int want = ((lg + g_sort_extra_bits + 7) / 8) * 8;
+    int want = ((lg + SORT_EXTRA_BITS + 7) / 8) * 8;
     if (want < 8) want = 8;
     int begin = 64 - want;
     if (begin < fmt.tb + 2) begin = fmt.tb + 2;
@@ -933,40 +806,7 @@ static int dedup_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const Rows &r
     const uint32_t chunks = (uint32_t)(rows.words / 2);
     uint4 *o = reinterpret_cast<uint4 *>(out_xz);
     double2 *oc = reinterpret_cast<double2 *>(out_c);
-#define EMIT_FUSED(LW, UN)                                                                                      \
-    {                                                                                                           \
-        constexpr int64_t Dp = (int64_t)(256 >> LW) * UN;                                                       \
-        emit_fused_kernel<Rows, BY_T, LW, UN><<<(unsigned)((T + Dp - 1) / Dp), 256, 0, st>>>(                   \
-            rows, fmt, sr, L.keep, L.multi, L.slot, L.acc, T, o, oc);                                           \
-    }
-    if (g_emit_variant == 1 && (chunks == 1 || chunks == 2 || chunks == 4 || chunks == 8 || chunks == 16)) {
-        switch (chunks) {
-            case 1: EMIT_FUSED(0, 1); break;
-            case 2: EMIT_FUSED(1, 2); break;
-            case 4: EMIT_FUSED(2, 4); break;
-            case 8: EMIT_FUSED(3, 8); break;
-            default: EMIT_FUSED(4, 8); break;
-        }
-        SYM_LAUNCH_OK();
-        return SYM_OK;
-    }
-#undef EMIT_FUSED
-#define EMIT_WARP(LW)                                                                                           \
-    emit_warp_kernel<Rows, BY_T, LW><<<(unsigned)((T + 255) / 256), 256, 0, st>>>(rows, fmt, sr, L.keep, L.multi, L.slot,  \
-                                                                                 L.acc, T, o, oc)
-    if (g_emit_variant == 2 && (chunks == 1 || chunks == 2 || chunks == 4 || chunks == 8 || chunks == 16)) {
-        switch (chunks) {
-            case 1: EMIT_WARP(0); break;
-            case 2: EMIT_WARP(1); break;
-            case 4: EMIT_WARP(2); break;
-            case 8: EMIT_WARP(3); break;
-            default: EMIT_WARP(4); break;
-        }
-        SYM_LAUNCH_OK();
-        return SYM_OK;
-    }
-#undef EMIT_WARP
-    // two-kernel form (tuning knob 1 = 0, and the generic chunk counts): compaction, then row emission
+    // compaction, then row emission
     compact_kernel<Rows, BY_T><<<(unsigned)((T + 255) / 256), 256, 0, st>>>(rows, fmt, sr, L.keep, L.multi, L.slot, L.acc, T,
                                                                            L.kept, oc);
     SYM_LAUNCH_OK();
@@ -1136,9 +976,8 @@ static WorkList tile_worklist(const DedupLayout &L, int64_t T) {
 
 int g_tile_qgroup = 16;   // tuning knob 7: B rows per CTA of tile_emit_kernel
 
-int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
-                             const ProductKeySrc *ksrc, double thr, int64_t *n_out, int64_t *n_out_host, void *ws,
-                             size_t ws_bytes, cudaStream_t st) {
+int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, double thr,
+                             int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st) {
     if (ws_bytes < dedup_ws_bytes(T)) {
         set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
         return SYM_E_WORKSPACE;
@@ -1150,8 +989,7 @@ int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const Produc
     }
     const int begin = sort_begin_bit(T, fmt);
     uint64_t *sr = nullptr;
-    if (ksrc) SYM_TRY(radix_sort_product_keys(*ksrc, recs, L.alt, T, begin, L.hist, &sr, st));
-    else SYM_TRY(radix_sort_records(recs, L.alt, T, begin, L.hist, &sr, st));
+    SYM_TRY(radix_sort_records(recs, L.alt, T, begin, L.hist, &sr, st));
     const unsigned nb = (unsigned)((T + 255) / 256);
     ProductRows rows_sum = rows;
     if (thr >= 0.0 && rows.N > 0) {

@@ -388,28 +388,11 @@ static int64_t g_by_t_limit = (int64_t)1 << 22;
 // tuning knob 6: 1 (default) = products above the limit use the ordered-tile mode (first-occurrence
 // order at every size, streaming tiled row emission); 0 = the sorted-hash order path
 static int g_ordered_tiles = 1;
-// tuning knob 9: 1 = in ordered-tile mode the first radix pass generates the records from the sketch
-// tables; 0 (default, measured faster on B200: 9.65 vs 10.06 ms per 1.25e8 cross terms — generating a
-// key costs two 64-bit multiplies and runs twice, in the histogram and in pass 0, against 0.15 ms
-// for pair_keys_kernel writing 1 GB once) = a separate kernel writes them first
-static int g_fused_keys = 0;
-namespace symb { extern int g_emit_variant; extern int g_scatter_variant; extern int g_sort_extra_bits; extern int g_apply_variant; extern int g_rref_variant; extern int g_tile_qgroup; extern int g_onesweep; extern int g_class_dedup; extern int g_class_variant; extern int g_commute_variant; }
+namespace symb { extern int g_apply_variant; extern int g_rref_variant; extern int g_tile_qgroup; extern int g_onesweep; extern int g_class_dedup; extern int g_class_variant; }
 
 extern "C" int sym_set_tuning(int32_t which, int64_t value) {
     if (which == 0) {
         g_by_t_limit = value;
-        return SYM_OK;
-    }
-    if (which == 1) {
-        symb::g_emit_variant = (int)value;
-        return SYM_OK;
-    }
-    if (which == 2) {
-        symb::g_scatter_variant = (int)value;
-        return SYM_OK;
-    }
-    if (which == 3) {
-        symb::g_sort_extra_bits = (int)value;
         return SYM_OK;
     }
     if (which == 4) {
@@ -432,20 +415,12 @@ extern "C" int sym_set_tuning(int32_t which, int64_t value) {
         symb::g_onesweep = (int)value;
         return SYM_OK;
     }
-    if (which == 9) {
-        g_fused_keys = (int)value;
-        return SYM_OK;
-    }
     if (which == 10) {
         symb::g_class_dedup = (int)value;
         return SYM_OK;
     }
     if (which == 11) {
         symb::g_class_variant = (int)value;
-        return SYM_OK;
-    }
-    if (which == 12) {
-        symb::g_commute_variant = (int)value;
         return SYM_OK;
     }
     set_error("unknown tuning knob %d", which);
@@ -614,31 +589,13 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
             SYM_CUDA_OK(cudaMemcpyAsync(P.d_blocks, P.blocks, sizeof(TileBlock) * (size_t)P.nblk, cudaMemcpyHostToDevice, st));
         SYM_CUDA_OK(cudaMemsetAsync(P.drop, 0, sizeof(uint32_t) * 4 * (size_t)P.n_seg, st));
     }
-    // ordered-tile mode with few blocks: the first radix pass generates the records itself
-    ProductKeySrc ksrc;
-    const bool fused_keys = P.mode == MODE_TILES && !P.class_mode && P.nblk <= PKS_MAX_BLOCKS && g_fused_keys != 0;
-    if (fused_keys) {
-        ksrc.a_sk = P.a_sk;
-        ksrc.b_sk = P.b_sk;
-        ksrc.M_total = (uint32_t)M_total;
-        ksrc.key_mask = g_key_mask;
-        ksrc.tb = fmt.tb;
-        ksrc.nblk = P.nblk;
-        uint32_t ro = 0;
-        for (int b = 0; b < PKS_MAX_BLOCKS; ++b) {
-            const bool in = b < P.nblk;
-            ksrc.rec_off[b] = ro;
-            ksrc.p0[b] = in ? P.blocks[b].p0 : 0u;
-            ksrc.m_blk[b] = in ? P.blocks[b].m_blk : 0u;
-            ksrc.q0[b] = in ? P.blocks[b].q0 : 0u;
-            if (in) ro += P.blocks[b].m_blk * P.blocks[b].nq;
-            ksrc.rec_off[b + 1] = ro;
-        }
-    }
     size_t off = 0;
-    for (int b = 0; b < P.nblk && !fused_keys && !P.class_mode; ++b) {
+    for (int b = 0; b < P.nblk && !P.class_mode; ++b) {
         const TileBlock &tb = P.blocks[b];
         if (P.mode == MODE_TILES) {
+            // a separate kernel writes the records before the sort: generating them inside the first radix pass
+            // measured slower on B200 (10.06 vs 9.65 ms per 1.25e8 cross terms: a key costs two 64-bit multiplies
+            // and is generated twice, in the histogram and in pass 0, against 0.15 ms for writing 1 GB once)
             if (tb.m_blk > 0 && tb.nq > 0) {
                 dim3 grid((tb.m_blk + 255) / 256, (tb.nq + KEYS_QCH - 1) / KEYS_QCH);
                 if (grid.y > 65535) {
@@ -667,8 +624,8 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
                                           P.class_ws, P.class_ws_bytes, zero_threshold, n_out, n_out_host, P.rest, P.rest_bytes, st);
     }
     if (P.mode == MODE_TILES)
-        return dedup_product_plan_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), fused_keys ? &ksrc : nullptr,
-                                        zero_threshold, n_out, n_out_host, P.rest, P.rest_bytes, st);
+        return dedup_product_plan_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), zero_threshold, n_out, n_out_host,
+                                        P.rest, P.rest_bytes, st);
     return dedup_product_plan(P.recs, P.T, fmt, rows, P.mode == MODE_BY_T, zero_threshold, n_out, n_out_host, P.rest,
                               P.rest_bytes, st);
 }

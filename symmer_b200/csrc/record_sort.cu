@@ -13,6 +13,8 @@ constexpr int RS_THREADS = 256;
 constexpr int RS_ITEMS = 16;
 constexpr int RS_TILE = RS_THREADS * RS_ITEMS;  // 4096 records
 constexpr int RS_RADIX = 256;
+constexpr int RS_WARPS = RS_THREADS / 32;
+constexpr int RS_MIN_BLOCKS = 4;   // CTAs per SM of the scatter passes: 256 threads x 16 records, 4 CTAs/SM measured best
 
 __global__ void __launch_bounds__(RS_THREADS) rs_hist_kernel(const uint64_t *__restrict__ in, int64_t T, int shift,
                                                               uint32_t mask, uint32_t *__restrict__ hist, int64_t ntiles) {
@@ -29,34 +31,31 @@ __global__ void __launch_bounds__(RS_THREADS) rs_hist_kernel(const uint64_t *__r
     hist[(int64_t)threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
 }
 
-// THREADS x ITEMS = RS_TILE. Ranks are < 4096 and are kept as 16-bit halves to save registers.
-template <int THREADS, int ITEMS, int MINB>
-__global__ void __launch_bounds__(THREADS, MINB) rs_scatter_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
-                                                                    int64_t T, int shift, uint32_t mask,
-                                                                    const uint32_t *__restrict__ hist, int64_t ntiles) {
-    static_assert(THREADS * ITEMS == RS_TILE, "tile size is fixed");
-    constexpr int WARPS = THREADS / 32;
+// Ranks are < 4096 and are kept as 16-bit halves to save registers.
+__global__ void __launch_bounds__(RS_THREADS, RS_MIN_BLOCKS) rs_scatter_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
+                                                                               int64_t T, int shift, uint32_t mask,
+                                                                               const uint32_t *__restrict__ hist, int64_t ntiles) {
     extern __shared__ __align__(16) unsigned char rs_smem[];
     uint64_t *srec = reinterpret_cast<uint64_t *>(rs_smem);
     uint32_t(*wh)[RS_RADIX] = reinterpret_cast<uint32_t(*)[RS_RADIX]>(rs_smem + RS_TILE * 8);
-    uint32_t *dbase = reinterpret_cast<uint32_t *>(rs_smem + RS_TILE * 8 + WARPS * RS_RADIX * 4);
+    uint32_t *dbase = reinterpret_cast<uint32_t *>(rs_smem + RS_TILE * 8 + RS_WARPS * RS_RADIX * 4);
     uint32_t *delta = dbase + RS_RADIX;
     uint32_t *wtot = delta + RS_RADIX;
-    for (int i = threadIdx.x; i < WARPS * RS_RADIX; i += THREADS) (&wh[0][0])[i] = 0;
+    for (int i = threadIdx.x; i < RS_WARPS * RS_RADIX; i += RS_THREADS) (&wh[0][0])[i] = 0;
     __syncthreads();
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const uint32_t lt = (1u << lane) - 1u;
     const int64_t tile_base = (int64_t)blockIdx.x * RS_TILE;
-    const int64_t wbase = tile_base + (int64_t)wid * (32 * ITEMS);
-    uint64_t k[ITEMS];
-    uint16_t r[ITEMS];
+    const int64_t wbase = tile_base + (int64_t)wid * (32 * RS_ITEMS);
+    uint64_t k[RS_ITEMS];
+    uint16_t r[RS_ITEMS];
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
+    for (int j = 0; j < RS_ITEMS; ++j) {
         int64_t idx = wbase + j * 32 + lane;
         k[j] = (idx < T) ? in[idx] : 0ull;
     }
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
+    for (int j = 0; j < RS_ITEMS; ++j) {
         int64_t idx = wbase + j * 32 + lane;
         bool valid = idx < T;
         uint32_t d = valid ? ((uint32_t)(k[j] >> shift) & mask) : 0xffffffffu;
@@ -80,7 +79,7 @@ __global__ void __launch_bounds__(THREADS, MINB) rs_scatter_kernel(const uint64_
         uint32_t cnt = 0;
         const int d = threadIdx.x;
 #pragma unroll
-        for (int w = 0; w < WARPS; ++w) {
+        for (int w = 0; w < RS_WARPS; ++w) {
             uint32_t c = wh[w][d];
             wh[w][d] = cnt;
             cnt += c;
@@ -106,7 +105,7 @@ __global__ void __launch_bounds__(THREADS, MINB) rs_scatter_kernel(const uint64_
     }
     __syncthreads();
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
+    for (int j = 0; j < RS_ITEMS; ++j) {
         int64_t idx = wbase + j * 32 + lane;
         if (idx < T) {
             uint32_t d = (uint32_t)(k[j] >> shift) & mask;
@@ -117,8 +116,8 @@ __global__ void __launch_bounds__(THREADS, MINB) rs_scatter_kernel(const uint64_
     const int64_t remain = T - tile_base;
     const int count = remain < RS_TILE ? (int)remain : RS_TILE;
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-        int pos = j * THREADS + threadIdx.x;
+    for (int j = 0; j < RS_ITEMS; ++j) {
+        int pos = j * RS_THREADS + threadIdx.x;
         if (pos < count) {
             uint64_t rec = srec[pos];
             uint32_t d = (uint32_t)(rec >> shift) & mask;
@@ -126,8 +125,6 @@ __global__ void __launch_bounds__(THREADS, MINB) rs_scatter_kernel(const uint64_
         }
     }
 }
-
-int g_scatter_variant = 3;  // tuning knob 2: 256 threads x 16 records, 4 CTAs/SM (measured best)
 
 __global__ void rs_bucket_counts_kernel(const uint32_t *__restrict__ scanned, int64_t ntiles, int nb, int64_t T,
                                         int64_t *__restrict__ counts) {
@@ -149,63 +146,9 @@ __global__ void rs_bucket_counts_kernel(const uint32_t *__restrict__ scanned, in
 constexpr int OS_MAX_PASSES = 8;
 constexpr int OS_EXTRA_ELEMS = OS_MAX_PASSES * RS_RADIX * 2 + 64;   // global counts + bases + tickets
 
-struct PlainKeySrc {
-    const uint64_t *in;
-    // k[j] = record at first + j*32 (0 beyond T)
-    template <int ITEMS>
-    __device__ __forceinline__ void load(int64_t first, int64_t T, uint64_t (&k)[ITEMS]) const {
-#pragma unroll
-        for (int j = 0; j < ITEMS; ++j) {
-            const int64_t idx = first + j * 32;
-            k[j] = idx < T ? in[idx] : 0ull;
-        }
-    }
-};
-
-struct ProductKeyGen {
-    ProductKeySrc s;
-    __device__ __forceinline__ void locate(uint32_t idx, int &b, uint32_t &p, uint32_t &q) const {
-        b = 0;
-        while (b + 1 < s.nblk && idx >= s.rec_off[b + 1]) ++b;
-        const uint32_t local = idx - s.rec_off[b];
-        q = local / s.m_blk[b];
-        p = local - q * s.m_blk[b];
-    }
-    template <int ITEMS>
-    __device__ __forceinline__ void load(int64_t first, int64_t T, uint64_t (&k)[ITEMS]) const {
-        int b = 0;
-        uint32_t p = 0, q = 0;
-        if (first < T) locate((uint32_t)first, b, p, q);
-        const int sh = s.tb + 2;
-#pragma unroll
-        for (int j = 0; j < ITEMS; ++j) {
-            const int64_t idx = first + j * 32;
-            uint64_t rec = 0ull;
-            if (idx < T) {
-                const uint32_t pg = s.p0[b] + p, qg = s.q0[b] + q;
-                const uint64_t h = mix64(s.a_sk[pg] ^ s.b_sk[qg]) & s.key_mask;
-                rec = ((h >> sh) << sh) | (((uint64_t)qg * s.M_total + pg) << 2);
-                if (idx + 32 < T) {
-                    if ((uint32_t)(idx + 32) >= s.rec_off[b + 1]) {
-                        locate((uint32_t)(idx + 32), b, p, q);   // next item is in another block
-                    } else {
-                        p += 32;
-                        while (p >= s.m_blk[b]) {
-                            p -= s.m_blk[b];
-                            ++q;
-                        }
-                    }
-                }
-            }
-            k[j] = rec;
-        }
-    }
-};
-
-// histograms of all passes in one read (or one generation) of the keys; grid-stride over tiles
-template <class Src>
-__global__ void __launch_bounds__(RS_THREADS) os_hist_kernel(Src src, int64_t T, int begin_bit, int passes, int64_t ntiles,
-                                                              uint32_t *__restrict__ counts) {
+// histograms of all passes in one read of the keys; grid-stride over tiles
+__global__ void __launch_bounds__(RS_THREADS) os_hist_kernel(const uint64_t *in, int64_t T, int begin_bit, int passes,
+                                                              int64_t ntiles, uint32_t *__restrict__ counts) {
     __shared__ uint32_t h[OS_MAX_PASSES][RS_RADIX];
     for (int i = threadIdx.x; i < OS_MAX_PASSES * RS_RADIX; i += RS_THREADS) (&h[0][0])[i] = 0;
     __syncthreads();
@@ -213,7 +156,8 @@ __global__ void __launch_bounds__(RS_THREADS) os_hist_kernel(Src src, int64_t T,
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         uint64_t k[RS_ITEMS];
         const int64_t first = tile * RS_TILE + (int64_t)wid * (32 * RS_ITEMS) + lane;
-        src.template load<RS_ITEMS>(first, T, k);
+#pragma unroll
+        for (int j = 0; j < RS_ITEMS; ++j) k[j] = first + j * 32 < T ? in[first + j * 32] : 0ull;
 #pragma unroll
         for (int j = 0; j < RS_ITEMS; ++j) {
             if (first + j * 32 < T) {
@@ -260,33 +204,35 @@ __device__ __forceinline__ void st_volatile_u32(uint32_t *p, uint32_t v) {
 
 // One radix pass. state[tile][digit]: bits 31:30 = 0 not published / 1 tile count / 2 inclusive
 // prefix over tiles 0..tile; bits 29:0 = value (T < 2^30 on this path).
-template <class Src, int THREADS, int ITEMS, int MINB>
-__global__ void __launch_bounds__(THREADS, MINB) os_pass_kernel(Src src, uint64_t *__restrict__ out, int64_t T, int shift,
-                                                                 uint32_t mask, const uint32_t *__restrict__ bases,
-                                                                 uint32_t *__restrict__ state, uint32_t *__restrict__ ticket) {
-    static_assert(THREADS * ITEMS == RS_TILE, "tile size is fixed");
-    static_assert(THREADS >= RS_RADIX, "one look-back thread per digit");
-    constexpr int WARPS = THREADS / 32;
+__global__ void __launch_bounds__(RS_THREADS, RS_MIN_BLOCKS) os_pass_kernel(const uint64_t *in, uint64_t *__restrict__ out,
+                                                                            int64_t T, int shift, uint32_t mask,
+                                                                            const uint32_t *__restrict__ bases,
+                                                                            uint32_t *__restrict__ state, uint32_t *__restrict__ ticket) {
+    static_assert(RS_THREADS >= RS_RADIX, "one look-back thread per digit");
     extern __shared__ __align__(16) unsigned char rs_smem[];
     uint64_t *srec = reinterpret_cast<uint64_t *>(rs_smem);
     uint32_t(*wh)[RS_RADIX] = reinterpret_cast<uint32_t(*)[RS_RADIX]>(rs_smem + RS_TILE * 8);
-    uint32_t *dbase = reinterpret_cast<uint32_t *>(rs_smem + RS_TILE * 8 + WARPS * RS_RADIX * 4);
+    uint32_t *dbase = reinterpret_cast<uint32_t *>(rs_smem + RS_TILE * 8 + RS_WARPS * RS_RADIX * 4);
     uint32_t *delta = dbase + RS_RADIX;
     uint32_t *wtot = delta + RS_RADIX;
     uint32_t *s_tile = wtot + 32;
-    for (int i = threadIdx.x; i < WARPS * RS_RADIX; i += THREADS) (&wh[0][0])[i] = 0;
+    for (int i = threadIdx.x; i < RS_WARPS * RS_RADIX; i += RS_THREADS) (&wh[0][0])[i] = 0;
     if (threadIdx.x == 0) *s_tile = atomicAdd(ticket, 1u);
     __syncthreads();
     const uint32_t tile = *s_tile;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const uint32_t lt = (1u << lane) - 1u;
     const int64_t tile_base = (int64_t)tile * RS_TILE;
-    const int64_t wbase = tile_base + (int64_t)wid * (32 * ITEMS);
-    uint64_t k[ITEMS];
-    uint16_t r[ITEMS];
-    src.template load<ITEMS>(wbase + lane, T, k);
+    const int64_t wbase = tile_base + (int64_t)wid * (32 * RS_ITEMS);
+    uint64_t k[RS_ITEMS];
+    uint16_t r[RS_ITEMS];
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
+    for (int j = 0; j < RS_ITEMS; ++j) {
+        int64_t idx = wbase + j * 32 + lane;
+        k[j] = (idx < T) ? in[idx] : 0ull;
+    }
+#pragma unroll
+    for (int j = 0; j < RS_ITEMS; ++j) {
         int64_t idx = wbase + j * 32 + lane;
         bool valid = idx < T;
         uint32_t d = valid ? ((uint32_t)(k[j] >> shift) & mask) : 0xffffffffu;
@@ -308,7 +254,7 @@ __global__ void __launch_bounds__(THREADS, MINB) os_pass_kernel(Src src, uint64_
     if (threadIdx.x < RS_RADIX) {
         const int d = threadIdx.x;
 #pragma unroll
-        for (int w = 0; w < WARPS; ++w) {
+        for (int w = 0; w < RS_WARPS; ++w) {
             uint32_t c = wh[w][d];
             wh[w][d] = cnt;
             cnt += c;
@@ -338,7 +284,7 @@ __global__ void __launch_bounds__(THREADS, MINB) os_pass_kernel(Src src, uint64_
     // stage the tile in digit order first: it needs no global offsets, and the tiles this one is about to
     // wait for get that much closer to publishing theirs
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
+    for (int j = 0; j < RS_ITEMS; ++j) {
         int64_t idx = wbase + j * 32 + lane;
         if (idx < T) {
             uint32_t d = (uint32_t)(k[j] >> shift) & mask;
@@ -377,8 +323,8 @@ __global__ void __launch_bounds__(THREADS, MINB) os_pass_kernel(Src src, uint64_
     const int64_t remain = T - tile_base;
     const int count = remain < RS_TILE ? (int)remain : RS_TILE;
 #pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-        int pos = j * THREADS + threadIdx.x;
+    for (int j = 0; j < RS_ITEMS; ++j) {
+        int pos = j * RS_THREADS + threadIdx.x;
         if (pos < count) {
             uint64_t rec = srec[pos];
             uint32_t d = (uint32_t)(rec >> shift) & mask;
@@ -402,38 +348,25 @@ size_t record_hist_elems(int64_t T) {
     return h * (size_t)os_state_copies(ntiles) + scan_scratch_elems((int64_t)h) + 64 + OS_EXTRA_ELEMS;
 }
 
-template <class Src, int TH, int IT, int MB>
-static int os_launch_shape(const Src &src, uint64_t *out, int64_t T, int shift, uint32_t mask, const uint32_t *bases,
-                           uint32_t *state, uint32_t *ticket, int64_t ntiles, cudaStream_t st, bool clear_state) {
-    constexpr size_t smem = RS_TILE * 8 + (TH / 32) * RS_RADIX * 4 + 2 * RS_RADIX * 4 + 32 * 4 + 64;
+static int os_launch_pass(const uint64_t *in, uint64_t *out, int64_t T, int shift, uint32_t mask, const uint32_t *bases,
+                          uint32_t *state, uint32_t *ticket, int64_t ntiles, cudaStream_t st, bool clear_state) {
+    constexpr size_t smem = RS_TILE * 8 + RS_WARPS * RS_RADIX * 4 + 2 * RS_RADIX * 4 + 32 * 4 + 64;
     static bool attr_done[64] = {};   // per device
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-        SYM_CUDA_OK(cudaFuncSetAttribute(os_pass_kernel<Src, TH, IT, MB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        SYM_CUDA_OK(cudaFuncSetAttribute(os_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
     if (clear_state) SYM_CUDA_OK(cudaMemsetAsync(state, 0, sizeof(uint32_t) * (size_t)RS_RADIX * (size_t)ntiles, st));
-    os_pass_kernel<Src, TH, IT, MB><<<(unsigned)ntiles, TH, smem, st>>>(src, out, T, shift, mask, bases, state, ticket);
+    os_pass_kernel<<<(unsigned)ntiles, RS_THREADS, smem, st>>>(in, out, T, shift, mask, bases, state, ticket);
     SYM_LAUNCH_OK();
     return SYM_OK;
 }
 
-template <class Src>
-static int os_launch_pass(const Src &src, uint64_t *out, int64_t T, int shift, uint32_t mask, const uint32_t *bases,
-                          uint32_t *state, uint32_t *ticket, int64_t ntiles, cudaStream_t st, bool clear_state) {
-    switch (g_scatter_variant) {   // tuning knob 2 (CTA shape); 3 = 256 threads x 16 records, 4 CTAs/SM is the default
-        case 1: return os_launch_shape<Src, 512, 8, 2>(src, out, T, shift, mask, bases, state, ticket, ntiles, st, clear_state);
-        case 2: return os_launch_shape<Src, 512, 8, 3>(src, out, T, shift, mask, bases, state, ticket, ntiles, st, clear_state);
-        case 5: return os_launch_shape<Src, 256, 16, 5>(src, out, T, shift, mask, bases, state, ticket, ntiles, st, clear_state);
-        default: return os_launch_shape<Src, 256, 16, 4>(src, out, T, shift, mask, bases, state, ticket, ntiles, st, clear_state);
-    }
-}
-
-// keys of pass 0 come from `first` (a buffer or the product key generator), later passes ping-pong a <-> b
-template <class Src>
-static int onesweep_sort(const Src &first, uint64_t *a, uint64_t *b, int64_t T, int begin_bit, uint32_t *hist,
-                         uint64_t **result, cudaStream_t st) {
+// passes ping-pong a <-> b; pass 0 reads a
+static int onesweep_sort(uint64_t *a, uint64_t *b, int64_t T, int begin_bit, uint32_t *hist, uint64_t **result,
+                         cudaStream_t st) {
     const int passes = (64 - begin_bit + 7) / 8;
     const int64_t ntiles = (T + RS_TILE - 1) / RS_TILE;
     uint32_t *state = hist;
@@ -446,7 +379,7 @@ static int onesweep_sort(const Src &first, uint64_t *a, uint64_t *b, int64_t T, 
     else
         SYM_CUDA_OK(cudaMemsetAsync(extra, 0, sizeof(uint32_t) * OS_EXTRA_ELEMS, st));
     const unsigned hgrid = (unsigned)std::min<int64_t>(ntiles, (int64_t)num_sms() * 8);
-    os_hist_kernel<Src><<<hgrid, RS_THREADS, 0, st>>>(first, T, begin_bit, passes, ntiles, counts);
+    os_hist_kernel<<<hgrid, RS_THREADS, 0, st>>>(a, T, begin_bit, passes, ntiles, counts);
     SYM_LAUNCH_OK();
     os_bases_kernel<<<passes, RS_RADIX, 0, st>>>(counts, bases);
     SYM_LAUNCH_OK();
@@ -455,12 +388,7 @@ static int onesweep_sort(const Src &first, uint64_t *a, uint64_t *b, int64_t T, 
         const int width = (64 - bit) < 8 ? (64 - bit) : 8;
         const uint32_t mask = (1u << width) - 1u;
         uint32_t *state_ps = copies > 1 ? state + (size_t)ps * h : state;
-        if (ps == 0) {
-            SYM_TRY(os_launch_pass(first, b, T, bit, mask, bases + ps * RS_RADIX, state_ps, tickets + ps, ntiles, st, copies == 1));
-        } else {
-            PlainKeySrc src{a};
-            SYM_TRY(os_launch_pass(src, b, T, bit, mask, bases + ps * RS_RADIX, state_ps, tickets + ps, ntiles, st, copies == 1));
-        }
+        SYM_TRY(os_launch_pass(a, b, T, bit, mask, bases + ps * RS_RADIX, state_ps, tickets + ps, ntiles, st, copies == 1));
         uint64_t *t = a; a = b; b = t;
         bit += width;
     }
@@ -475,55 +403,17 @@ static int rs_pass(const uint64_t *in, uint64_t *out, int64_t T, int shift, uint
     rs_hist_kernel<<<(unsigned)ntiles, RS_THREADS, 0, st>>>(in, T, shift, mask, hist, ntiles);
     SYM_LAUNCH_OK();
     SYM_TRY(scan_exclusive_u32(hist, hist, hn, nullptr, scratch, st));
-#define RS_LAUNCH(TH, IT, MB)                                                                                     \
-    {                                                                                                             \
-        constexpr size_t smem = RS_TILE * 8 + (TH / 32) * RS_RADIX * 4 + 2 * RS_RADIX * 4 + 64;                   \
-        static bool attr_done[64] = {};                                                                           \
-        int dev_ = 0;                                                                                             \
-        cudaGetDevice(&dev_);                                                                                     \
-        if (dev_ >= 0 && dev_ < 64 && !attr_done[dev_]) {                                                         \
-            SYM_CUDA_OK(cudaFuncSetAttribute(rs_scatter_kernel<TH, IT, MB>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                             (int)smem));                                                         \
-            attr_done[dev_] = true;                                                                               \
-        }                                                                                                         \
-        rs_scatter_kernel<TH, IT, MB><<<(unsigned)ntiles, TH, smem, st>>>(in, out, T, shift, mask, hist, ntiles); \
+    constexpr size_t smem = RS_TILE * 8 + RS_WARPS * RS_RADIX * 4 + 2 * RS_RADIX * 4 + 64;
+    static bool attr_done[64] = {};   // per device
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 64 && !attr_done[dev]) {
+        SYM_CUDA_OK(cudaFuncSetAttribute(rs_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_done[dev] = true;
     }
-    switch (g_scatter_variant) {
-        case 1: RS_LAUNCH(512, 8, 2); break;
-        case 2: RS_LAUNCH(512, 8, 3); break;
-        case 3: RS_LAUNCH(256, 16, 4); break;
-        case 4: RS_LAUNCH(1024, 4, 1); break;
-        case 5: RS_LAUNCH(1024, 4, 2); break;
-        default: RS_LAUNCH(256, 16, 3); break;
-    }
-#undef RS_LAUNCH
+    rs_scatter_kernel<<<(unsigned)ntiles, RS_THREADS, smem, st>>>(in, out, T, shift, mask, hist, ntiles);
     SYM_LAUNCH_OK();
     return SYM_OK;
-}
-
-// materialise the generated records (fallback when the one-sweep path is off or T >= 2^30)
-__global__ void __launch_bounds__(RS_THREADS) os_materialise_kernel(ProductKeyGen gen, int64_t T, uint64_t *__restrict__ out) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int64_t first = (int64_t)blockIdx.x * RS_TILE + (int64_t)wid * (32 * RS_ITEMS) + lane;
-    uint64_t k[RS_ITEMS];
-    gen.template load<RS_ITEMS>(first, T, k);
-#pragma unroll
-    for (int j = 0; j < RS_ITEMS; ++j)
-        if (first + j * 32 < T) out[first + j * 32] = k[j];
-}
-
-int radix_sort_product_keys(const ProductKeySrc &src, uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit,
-                            uint32_t *hist, uint64_t **result, cudaStream_t st) {
-    *result = keys;
-    if (T <= 0) return SYM_OK;
-    if (begin_bit < 0) begin_bit = 0;
-    if (begin_bit > 63) begin_bit = 63;
-    ProductKeyGen gen{src};
-    if (T > 1 && g_onesweep && T < ((int64_t)1 << 30)) return onesweep_sort(gen, keys, alt, T, begin_bit, hist, result, st);
-    const int64_t ntiles = (T + RS_TILE - 1) / RS_TILE;
-    os_materialise_kernel<<<(unsigned)ntiles, RS_THREADS, 0, st>>>(gen, T, keys);
-    SYM_LAUNCH_OK();
-    return radix_sort_records(keys, alt, T, begin_bit, hist, result, st);
 }
 
 int radix_sort_records(uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit, uint32_t *hist, uint64_t **result,
@@ -532,10 +422,7 @@ int radix_sort_records(uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit, 
     if (T <= 1) return SYM_OK;
     if (begin_bit < 0) begin_bit = 0;
     if (begin_bit > 63) begin_bit = 63;
-    if (g_onesweep && T < ((int64_t)1 << 30)) {
-        PlainKeySrc src{keys};
-        return onesweep_sort(src, keys, alt, T, begin_bit, hist, result, st);
-    }
+    if (g_onesweep && T < ((int64_t)1 << 30)) return onesweep_sort(keys, alt, T, begin_bit, hist, result, st);
     uint64_t *a = keys, *b = alt;
     int bit = begin_bit;
     while (bit < 64) {

@@ -287,10 +287,8 @@ int dedup_plain_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const PlainRow
                      double *out_c, void *ws, size_t ws_bytes, cudaStream_t st);
 
 // ordered-tile mode (products only); blocks_host mirrors tm.blocks
-struct ProductKeySrc;   // sort.cuh: records generated inside the first radix pass (nullptr: recs already holds them)
-int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
-                             const ProductKeySrc *ksrc, double thr, int64_t *n_out, int64_t *n_out_host, void *ws,
-                             size_t ws_bytes, cudaStream_t st);
+int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, double thr,
+                             int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
 // class mode: `recs` is only scratch (the overflow array); a_sk / b_sk are the operand sketch tables and
 // class_ws holds the class tables (class_job_ws_bytes)
 int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, ClassJob &job,

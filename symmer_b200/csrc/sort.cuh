@@ -37,25 +37,6 @@ size_t record_hist_elems(int64_t T);
 int radix_sort_records(uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit, uint32_t *hist, uint64_t **result,
                        cudaStream_t st);
 
-// Records of a product generated on the fly (ordered-tile mode): record j of block b is
-//   [ mix64(a_sk[p] ^ b_sk[q]) & key_mask | t = q*M_total + p | 0 ],  local = j - rec_off[b],
-//   q = q0[b] + local / m_blk[b],  p = p0[b] + local % m_blk[b]
-// so that the first radix pass reads two sketch tables instead of an 8 B/record array that a
-// separate kernel would have had to write first. At most PKS_MAX_BLOCKS blocks (by value).
-constexpr int PKS_MAX_BLOCKS = 8;
-struct ProductKeySrc {
-    const uint64_t *a_sk, *b_sk;
-    uint32_t M_total;
-    uint64_t key_mask;
-    int tb;                                  // RecFmt::tb
-    int nblk;
-    uint32_t rec_off[PKS_MAX_BLOCKS + 1];    // rec_off[nblk] = T
-    uint32_t p0[PKS_MAX_BLOCKS], m_blk[PKS_MAX_BLOCKS], q0[PKS_MAX_BLOCKS];
-};
-// Same sort with the records of `src` as the (virtual) contents of `keys`: keys is only used as
-// the ping-pong partner of alt; the result lands where radix_sort_records would have put it.
-int radix_sort_product_keys(const ProductKeySrc &src, uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit,
-                            uint32_t *hist, uint64_t **result, cudaStream_t st);
 // One stable partition pass on the top `bits` (<= 8) bits; counts: device int64[1 << bits].
 int radix_partition_records(const uint64_t *keys, uint64_t *out, int64_t T, int bits, int64_t *counts, uint32_t *hist,
                             cudaStream_t st);
