@@ -758,7 +758,7 @@ static int dedup_plan(uint64_t *recs, int64_t T, RecFmt fmt, const Rows &rows, d
     }
     const int begin = sort_begin_bit(T, fmt);
     uint64_t *sr = nullptr;
-    SYM_TRY(radix_sort_records(recs, L.alt, T, begin, L.hist, &sr, st));
+    SYM_TRY(radix_sort(recs, nullptr, L.alt, nullptr, T, begin, L.hist, &sr, st));
 
     const unsigned nb = (unsigned)((T + 255) / 256);
     link_kernel<Rows><<<nb, 256, 0, st>>>(rows, fmt, sr, T, begin, L.flag, L.link);
@@ -989,7 +989,7 @@ int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const Produc
     }
     const int begin = sort_begin_bit(T, fmt);
     uint64_t *sr = nullptr;
-    SYM_TRY(radix_sort_records(recs, L.alt, T, begin, L.hist, &sr, st));
+    SYM_TRY(radix_sort(recs, nullptr, L.alt, nullptr, T, begin, L.hist, &sr, st));
     const unsigned nb = (unsigned)((T + 255) / 256);
     ProductRows rows_sum = rows;
     if (thr >= 0.0 && rows.N > 0) {
@@ -1291,7 +1291,8 @@ int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
             return SYM_E_CUDA;
         }
         uint64_t *sorted = nullptr;
-        SYM_TRY(radix_sort_records(over, reinterpret_cast<uint64_t *>(L.slot), (int64_t)n_over, 2, L.hist, &sorted, st));
+        SYM_TRY(radix_sort(over, nullptr, reinterpret_cast<uint64_t *>(L.slot), nullptr, (int64_t)n_over, 2, L.hist,
+                           &sorted, st));
         SYM_CUDA_OK(cudaMemcpyAsync(cand + n_cand, sorted, sizeof(uint64_t) * (size_t)n_over, cudaMemcpyDeviceToDevice, st));
         SYM_TRY(class_ord_to_t(job, cand + n_cand, n_over, st));
         SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, sort_shift, counters, counters + 3, L, thr, tm, st));

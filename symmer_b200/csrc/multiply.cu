@@ -336,7 +336,7 @@ extern "C" int sym_partition_records(const uint64_t *recs, int64_t T, int32_t lo
     }
     Arena ar(ws, ws_bytes);
     uint32_t *hist = ar.take<uint32_t>(record_hist_elems(T));
-    return radix_partition_records(recs, out_recs, T, log2_parts, counts, hist, (cudaStream_t)stream);
+    return radix_partition(recs, nullptr, out_recs, nullptr, T, log2_parts, counts, hist, (cudaStream_t)stream);
 }
 
 extern "C" size_t sym_dedup_records_ws_bytes(int64_t T, int32_t W) {

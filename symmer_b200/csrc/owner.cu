@@ -22,7 +22,7 @@ __device__ __forceinline__ uint32_t owner_of_sketch(uint64_t sk, int lg) {
     return cls;
 }
 
-// keys[row] = class << (64 - lg) (radix_partition_top splits on the top lg bits), vals[row] = row
+// keys[row] = class << (64 - lg) (radix_partition splits on the top lg bits), vals[row] = row
 __global__ void __launch_bounds__(256) owner_keys_kernel(const uint64_t *__restrict__ sk, int64_t M, int lg,
                                                           uint64_t *__restrict__ keys, uint32_t *__restrict__ vals,
                                                           uint8_t *__restrict__ cls_out) {
@@ -86,7 +86,7 @@ extern "C" int sym_gather_rows(const uint64_t *xz, const double *c, const uint32
 
 extern "C" size_t sym_class_partition_ws_bytes(int64_t M) {
     if (M < 1) M = 1;
-    return arena_need((size_t)M, 8) * 3 + arena_need((size_t)M, 4) * 2 + arena_need(sort_hist_elems(M), 4) + 2048;
+    return arena_need((size_t)M, 8) * 3 + arena_need((size_t)M, 4) * 2 + arena_need(record_hist_elems(M), 4) + 2048;
 }
 
 extern "C" int sym_class_partition(const uint64_t *xz, const double *c, int64_t M, int32_t W, int32_t log2_parts,
@@ -110,7 +110,7 @@ extern "C" int sym_class_partition(const uint64_t *xz, const double *c, int64_t 
     uint64_t *keys2 = ar.take<uint64_t>((size_t)M);
     uint32_t *vals = ar.take<uint32_t>((size_t)M);
     uint32_t *vals2 = ar.take<uint32_t>((size_t)M);
-    uint32_t *hist = ar.take<uint32_t>(sort_hist_elems(M));
+    uint32_t *hist = ar.take<uint32_t>(record_hist_elems(M));
     if (!hist) {
         set_error("workspace arena exhausted");
         return SYM_E_WORKSPACE;
@@ -120,7 +120,7 @@ extern "C" int sym_class_partition(const uint64_t *xz, const double *c, int64_t 
     SYM_LAUNCH_OK();
     const uint32_t *order = vals;
     if (log2_parts > 0) {
-        SYM_TRY(radix_partition_top(keys, vals, keys2, vals2, M, log2_parts, counts, hist, st));
+        SYM_TRY(radix_partition(keys, vals, keys2, vals2, M, log2_parts, counts, hist, st));
         order = vals2;
     } else {
         int64_t m = M;

@@ -1,6 +1,5 @@
-// Exclusive scan + stable LSD radix sort (uint64 key, uint32 value), hand-written for sm_100a.
-// HBM-bound integer work: coalesced 8/16-byte accesses, per-warp stable ranking with match.any,
-// grids sized by the data (thousands of CTAs >> 148 SMs).
+// Exclusive scan, hand-written for sm_100a, and the C ABI of the pair sort (record_sort.cu).
+// HBM-bound integer work: coalesced 16-byte accesses, grids sized by the data (thousands of CTAs >> 148 SMs).
 #include "sort.cuh"
 
 namespace symb {
@@ -226,170 +225,6 @@ int scan_exclusive_u32(const uint32_t *in, uint32_t *out, int64_t n, uint32_t *t
     return scan_impl<uint32_t>(in, out, n, total, scratch, st);
 }
 
-// ---------------------------------------------------------------------------------------------
-// radix sort
-// ---------------------------------------------------------------------------------------------
-constexpr int SORT_THREADS = 256;
-constexpr int SORT_WARPS = SORT_THREADS / 32;
-constexpr int SORT_ITEMS = 16;
-constexpr int SORT_TILE = SORT_THREADS * SORT_ITEMS;  // 4096 elements, warp w owns 512 consecutive
-constexpr int RADIX = 256;
-
-__global__ void __launch_bounds__(SORT_THREADS) radix_hist_kernel(const uint64_t *__restrict__ keys, int64_t T, int shift,
-                                                                   uint32_t mask, uint32_t *__restrict__ hist,
-                                                                   int64_t ntiles) {
-    __shared__ uint32_t h[RADIX];
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int64_t wbase = (int64_t)blockIdx.x * SORT_TILE + (int64_t)wid * (32 * SORT_ITEMS);
-#pragma unroll 4
-    for (int j = 0; j < SORT_ITEMS; ++j) {
-        int64_t idx = wbase + j * 32 + lane;
-        bool valid = idx < T;
-        uint32_t d = valid ? (uint32_t)((keys[idx] >> shift) & mask) : 0xffffffffu;
-        uint32_t peers = __match_any_sync(0xffffffffu, d);
-        if (valid && lane == (__ffs(peers) - 1)) atomicAdd(&h[d], __popc(peers));
-    }
-    __syncthreads();
-    hist[(int64_t)threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
-}
-
-__global__ void __launch_bounds__(SORT_THREADS) radix_scatter_kernel(const uint64_t *__restrict__ keys_in,
-                                                                      const uint32_t *__restrict__ vals_in,
-                                                                      uint64_t *__restrict__ keys_out,
-                                                                      uint32_t *__restrict__ vals_out, int64_t T, int shift,
-                                                                      uint32_t mask, const uint32_t *__restrict__ hist,
-                                                                      int64_t ntiles, int vals_iota) {
-    __shared__ uint32_t wh[SORT_WARPS][RADIX];
-    for (int i = threadIdx.x; i < SORT_WARPS * RADIX; i += SORT_THREADS) (&wh[0][0])[i] = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const uint32_t lt = (1u << lane) - 1u;
-    const int64_t wbase = (int64_t)blockIdx.x * SORT_TILE + (int64_t)wid * (32 * SORT_ITEMS);
-    uint64_t k[SORT_ITEMS];
-    uint32_t r[SORT_ITEMS];
-#pragma unroll
-    for (int j = 0; j < SORT_ITEMS; ++j) {
-        int64_t idx = wbase + j * 32 + lane;
-        k[j] = (idx < T) ? keys_in[idx] : 0ull;
-    }
-#pragma unroll
-    for (int j = 0; j < SORT_ITEMS; ++j) {
-        int64_t idx = wbase + j * 32 + lane;
-        bool valid = idx < T;
-        uint32_t d = valid ? (uint32_t)((k[j] >> shift) & mask) : 0xffffffffu;
-        uint32_t peers = __match_any_sync(0xffffffffu, d);
-        uint32_t before = valid ? wh[wid][d] : 0u;
-        r[j] = before + __popc(peers & lt);
-        __syncwarp();
-        if (valid && lane == (__ffs(peers) - 1)) wh[wid][d] = before + __popc(peers);
-        __syncwarp();
-    }
-    __syncthreads();
-    {
-        const int d = threadIdx.x;
-        uint32_t run = hist[(int64_t)d * ntiles + blockIdx.x];
-#pragma unroll
-        for (int w = 0; w < SORT_WARPS; ++w) {
-            uint32_t c = wh[w][d];
-            wh[w][d] = run;
-            run += c;
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < SORT_ITEMS; ++j) {
-        int64_t idx = wbase + j * 32 + lane;
-        if (idx < T) {
-            uint32_t d = (uint32_t)((k[j] >> shift) & mask);
-            uint32_t dst = wh[wid][d] + r[j];
-            keys_out[dst] = k[j];
-            vals_out[dst] = vals_iota ? (uint32_t)idx : vals_in[idx];
-        }
-    }
-}
-
-__global__ void bucket_counts_kernel(const uint32_t *__restrict__ scanned, int64_t ntiles, int nb, int64_t T,
-                                     int64_t *__restrict__ counts) {
-    int d = blockIdx.x * blockDim.x + threadIdx.x;
-    if (d < nb) {
-        int64_t lo = scanned[(int64_t)d * ntiles];
-        int64_t hi = (d + 1 < RADIX) ? (int64_t)scanned[(int64_t)(d + 1) * ntiles] : T;
-        // buckets >= nb are empty, so scanned[(d+1)*ntiles] == T for d == nb-1 as well
-        counts[d] = hi - lo;
-    }
-}
-
-size_t sort_hist_elems(int64_t T) {
-    int64_t ntiles = (T + SORT_TILE - 1) / SORT_TILE;
-    if (ntiles < 1) ntiles = 1;
-    size_t h = (size_t)RADIX * (size_t)ntiles;
-    return h + scan_scratch_elems((int64_t)h) + 64;
-}
-
-static int radix_pass(const uint64_t *kin, const uint32_t *vin, uint64_t *kout, uint32_t *vout, int64_t T, int shift,
-                      uint32_t mask, bool iota, uint32_t *hist, cudaStream_t st) {
-    int64_t ntiles = (T + SORT_TILE - 1) / SORT_TILE;
-    int64_t hn = (int64_t)RADIX * ntiles;
-    uint32_t *scratch = hist + hn;
-    radix_hist_kernel<<<(unsigned)ntiles, SORT_THREADS, 0, st>>>(kin, T, shift, mask, hist, ntiles);
-    SYM_LAUNCH_OK();
-    SYM_TRY(scan_exclusive_u32(hist, hist, hn, nullptr, scratch, st));
-    radix_scatter_kernel<<<(unsigned)ntiles, SORT_THREADS, 0, st>>>(kin, vin, kout, vout, T, shift, mask, hist, ntiles,
-                                                                     iota ? 1 : 0);
-    SYM_LAUNCH_OK();
-    return SYM_OK;
-}
-
-int radix_sort_pairs(uint64_t *keys, uint32_t *vals, uint64_t *keys_alt, uint32_t *vals_alt, int64_t T, int begin_bit,
-                     bool vals_iota, uint32_t *hist, cudaStream_t st) {
-    if (T <= 0) return SYM_OK;
-    if (begin_bit < 0) begin_bit = 0;
-    if (begin_bit > 63) begin_bit = 63;
-    int passes = (64 - begin_bit + 7) / 8;
-    // an even number of passes leaves the result in keys/vals; if odd, run the first pass on the
-    // lowest partial digit and copy back at the end.
-    uint64_t *ka = keys, *kb = keys_alt;
-    uint32_t *va = vals, *vb = vals_alt;
-    int bit = begin_bit;
-    for (int p = 0; p < passes; ++p) {
-        int width = (64 - bit) < 8 ? (64 - bit) : 8;
-        uint32_t mask = (1u << width) - 1u;
-        SYM_TRY(radix_pass(ka, va, kb, vb, T, bit, mask, vals_iota && p == 0, hist, st));
-        uint64_t *tk = ka; ka = kb; kb = tk;
-        uint32_t *tv = va; va = vb; vb = tv;
-        bit += width;
-    }
-    if (ka != keys) {
-        SYM_CUDA_OK(cudaMemcpyAsync(keys, ka, sizeof(uint64_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
-        SYM_CUDA_OK(cudaMemcpyAsync(vals, va, sizeof(uint32_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
-    }
-    return SYM_OK;
-}
-
-int radix_partition_top(const uint64_t *keys, const uint32_t *vals, uint64_t *out_keys, uint32_t *out_vals, int64_t T,
-                        int bits, int64_t *counts, uint32_t *hist, cudaStream_t st) {
-    int nb = 1 << bits;
-    if (T <= 0) {
-        SYM_CUDA_OK(cudaMemsetAsync(counts, 0, sizeof(int64_t) * nb, st));
-        return SYM_OK;
-    }
-    if (bits == 0) {
-        SYM_CUDA_OK(cudaMemcpyAsync(out_keys, keys, sizeof(uint64_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
-        SYM_CUDA_OK(cudaMemcpyAsync(out_vals, vals, sizeof(uint32_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
-        int64_t t = T;
-        SYM_CUDA_OK(cudaMemcpyAsync(counts, &t, sizeof(int64_t), cudaMemcpyHostToDevice, st));
-        SYM_CUDA_OK(cudaStreamSynchronize(st));
-        return SYM_OK;
-    }
-    SYM_TRY(radix_pass(keys, vals, out_keys, out_vals, T, 64 - bits, (1u << bits) - 1u, false, hist, st));
-    int64_t ntiles = (T + SORT_TILE - 1) / SORT_TILE;
-    bucket_counts_kernel<<<1, 256, 0, st>>>(hist, ntiles, nb, T, counts);
-    SYM_LAUNCH_OK();
-    return SYM_OK;
-}
-
 }  // namespace symb
 
 // ---------------------------------------------------------------------------------------------
@@ -399,7 +234,7 @@ using namespace symb;
 
 extern "C" size_t sym_sort_pairs_ws_bytes(int64_t T) {
     if (T < 1) T = 1;
-    return arena_need((size_t)T, 8) + arena_need((size_t)T, 4) + arena_need(sort_hist_elems(T), 4) + 1024;
+    return arena_need((size_t)T, 8) + arena_need((size_t)T, 4) + arena_need(record_hist_elems(T), 4) + 1024;
 }
 
 extern "C" int sym_sort_pairs(uint64_t *keys, uint32_t *vals, int64_t T, int32_t begin_bit, void *ws, size_t ws_bytes,
@@ -413,7 +248,13 @@ extern "C" int sym_sort_pairs(uint64_t *keys, uint32_t *vals, int64_t T, int32_t
     Arena ar(ws, ws_bytes);
     uint64_t *ka = ar.take<uint64_t>((size_t)T);
     uint32_t *va = ar.take<uint32_t>((size_t)T);
-    uint32_t *hist = ar.take<uint32_t>(sort_hist_elems(T));
-    return radix_sort_pairs(keys, vals, ka, va, T, begin_bit, false, hist, (cudaStream_t)stream);
+    uint32_t *hist = ar.take<uint32_t>(record_hist_elems(T));
+    cudaStream_t st = (cudaStream_t)stream;
+    uint64_t *sorted = keys;
+    SYM_TRY(radix_sort(keys, vals, ka, va, T, begin_bit, hist, &sorted, st));
+    if (sorted != keys) {   // an odd number of passes ends in the workspace
+        SYM_CUDA_OK(cudaMemcpyAsync(keys, ka, sizeof(uint64_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
+        SYM_CUDA_OK(cudaMemcpyAsync(vals, va, sizeof(uint32_t) * (size_t)T, cudaMemcpyDeviceToDevice, st));
+    }
+    return SYM_OK;
 }
-

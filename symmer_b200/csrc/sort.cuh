@@ -1,5 +1,5 @@
-// Device-wide primitives used by the dedup pipeline: exclusive scan and a stable LSD radix sort
-// of (uint64 key, uint32 value) pairs. Hand-written for sm_100a; no CUB/Thrust on the path.
+// Device-wide primitives used by the dedup pipeline: exclusive scan and a stable LSD radix sort of
+// 64-bit keys with optional 32-bit values. Hand-written for sm_100a; no CUB/Thrust on the path.
 #pragma once
 #include "common.cuh"
 
@@ -14,30 +14,18 @@ int scan_exclusive_u8(const uint8_t *in, uint32_t *out, int64_t n, uint32_t *tot
 int scan_exclusive_u32(const uint32_t *in, uint32_t *out, int64_t n, uint32_t *total, uint32_t *scratch,
                        cudaStream_t st);
 
-// Stable radix sort on key bits [begin_bit, 64), 8 bits per pass. Buffers: keys/vals hold the
-// input and receive the output; keys_alt/vals_alt are same-sized scratch. hist: uint32 scratch of
-// sort_hist_elems(T). If vals_iota is true the input values are taken to be 0..T-1 (vals need not
-// be initialised).
-size_t sort_hist_elems(int64_t T);
-int radix_sort_pairs(uint64_t *keys, uint32_t *vals, uint64_t *keys_alt, uint32_t *vals_alt, int64_t T,
-                     int begin_bit, bool vals_iota, uint32_t *hist, cudaStream_t st);
-
-// One stable partition pass on the top `bits` bits of the key (bits <= 8); counts[d] (device
-// int64[1<<bits]) receives the bucket sizes.
-int radix_partition_top(const uint64_t *keys, const uint32_t *vals, uint64_t *out_keys, uint32_t *out_vals,
-                        int64_t T, int bits, int64_t *counts, uint32_t *hist, cudaStream_t st);
-
-}  // namespace symb
-
-namespace symb {
-// Hot-path sort: stable LSD radix sort of single 64-bit records on bits [begin_bit, 64), shared-
-// memory staged so that every digit run of a tile leaves as one contiguous (coalesced) store.
-// `*result` receives whichever of keys/alt holds the sorted records (no copy-back).
+// Stable LSD radix sort (record_sort.cu) of 64-bit keys on bits [begin_bit, 64), 8 bits per pass; each key
+// optionally carries a 32-bit value (vals, vals_alt: null for keys alone). Tiles are staged in shared memory so
+// that every digit run of a tile leaves as one contiguous (coalesced) store. Passes ping-pong between keys/vals
+// and the same-sized alt/vals_alt; `*result` receives whichever of keys/alt holds the sorted keys (no copy-back),
+// and the sorted values are in the matching value buffer. hist: uint32 scratch of record_hist_elems(T).
 size_t record_hist_elems(int64_t T);
-int radix_sort_records(uint64_t *keys, uint64_t *alt, int64_t T, int begin_bit, uint32_t *hist, uint64_t **result,
-                       cudaStream_t st);
+int radix_sort(uint64_t *keys, uint32_t *vals, uint64_t *alt, uint32_t *vals_alt, int64_t T, int begin_bit,
+               uint32_t *hist, uint64_t **result, cudaStream_t st);
 
-// One stable partition pass on the top `bits` (<= 8) bits; counts: device int64[1 << bits].
-int radix_partition_records(const uint64_t *keys, uint64_t *out, int64_t T, int bits, int64_t *counts, uint32_t *hist,
-                            cudaStream_t st);
+// One stable partition pass on the top `bits` (<= 8) bits of the key, values (if not null) moving with their
+// keys; counts: device int64[1 << bits] receives the bucket sizes. hist as for radix_sort.
+int radix_partition(const uint64_t *keys, const uint32_t *vals, uint64_t *out, uint32_t *out_vals, int64_t T, int bits,
+                    int64_t *counts, uint32_t *hist, cudaStream_t st);
+
 }  // namespace symb

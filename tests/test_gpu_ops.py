@@ -49,17 +49,25 @@ def test_sketch_is_linear(ops):
 
 
 def test_sort_pairs(ops):
-    rng = np.random.default_rng(1)
-    for T in [1, 31, 4096, 4097, 100003]:
-        keys = rng.integers(0, 2**63 - 1, size=T, dtype=np.int64) * 2 + rng.integers(0, 2, size=T)
-        keys[::5] = keys[0]                       # many duplicates: checks stability
-        vals = np.arange(T, dtype=np.int32)
-        k = torch.from_numpy(keys.copy()).cuda()
-        v = torch.from_numpy(vals.copy()).cuda()
-        ops.sort_pairs(k, v, 0)
-        order = np.argsort(keys.view(np.uint64), kind="stable")
-        assert np.array_equal(k.cpu().numpy(), keys[order])
-        assert np.array_equal(v.cpu().numpy(), vals[order])
+    """Both pass forms (knob 8), nonzero begin_bit with an even and an odd (13: 7 passes, copied back) pass
+    count, and a size above 1024 tiles, where the one-sweep passes share one look-back state."""
+    try:
+        for onesweep in [1, 0]:
+            ops.set_tuning(8, onesweep)
+            rng = np.random.default_rng(1)
+            for T in [1, 31, 4096, 4097, 100003, 5_000_000]:
+                keys = rng.integers(0, 2**63 - 1, size=T, dtype=np.int64) * 2 + rng.integers(0, 2, size=T)
+                keys[::5] = keys[0]                       # many duplicates: checks stability
+                vals = np.arange(T, dtype=np.int32)
+                for begin_bit in [0, 4, 13]:
+                    k = torch.from_numpy(keys.copy()).cuda()
+                    v = torch.from_numpy(vals.copy()).cuda()
+                    ops.sort_pairs(k, v, begin_bit)
+                    order = np.argsort(keys.view(np.uint64) >> np.uint64(begin_bit), kind="stable")
+                    assert np.array_equal(k.cpu().numpy(), keys[order]), (onesweep, T, begin_bit)
+                    assert np.array_equal(v.cpu().numpy(), vals[order]), (onesweep, T, begin_bit)
+    finally:
+        ops.set_tuning(8, 1)
 
 
 @pytest.mark.parametrize("n,m1,m2", [(1, 3, 2), (5, 20, 7), (63, 12, 9), (64, 10, 13), (65, 9, 11), (130, 16, 5),
@@ -579,9 +587,9 @@ def test_owner_classes_are_linear_and_partition_is_stable(ops):
     """Ownership must be GF(2)-linear in the row (class(a^b) = class(a)^class(b)) and the class
     grouping a stable permutation with the right counts."""
     rng = np.random.default_rng(5)
-    for n in [3, 64, 200, 1000, 2100]:
-        a = rng.random((300, 2 * n)) < 0.3
-        b = rng.random((300, 2 * n)) < 0.3
+    for n, m in [(3, 300), (64, 300), (200, 300), (1000, 300), (2100, 300), (64, 10000), (1000, 10000)]:   # 10 000: 3 tiles
+        a = rng.random((m, 2 * n)) < 0.3
+        b = rng.random((m, 2 * n)) < 0.3
         for lg in [0, 1, 3, 8]:
             ca = ops.owner_classes(ops.pack(torch.from_numpy(a), n), lg).cpu().numpy()
             cb = ops.owner_classes(ops.pack(torch.from_numpy(b), n), lg).cpu().numpy()
@@ -590,7 +598,7 @@ def test_owner_classes_are_linear_and_partition_is_stable(ops):
             assert ca.max(initial=0) < (1 << lg)
         if n >= 64:
             assert len(np.unique(ca)) > 100                           # 8 bits of 300 random rows: well spread
-        coeff = rng.standard_normal(300) + 1j * rng.standard_normal(300)
+        coeff = rng.standard_normal(m) + 1j * rng.standard_normal(m)
         xz, c = dev_op(ops, a, coeff)
         cls = ops.owner_classes(xz, 3).cpu().numpy()
         p_xz, p_c, perm, counts = ops.class_partition(xz, c, 3)
