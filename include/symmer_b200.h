@@ -96,15 +96,30 @@ int sym_mul_blocks_count(const uint64_t *a_xz, const double *a_c, int64_t M_tota
                          double zero_threshold, int64_t *n_out, int64_t *n_out_host, void *ws,
                          size_t ws_bytes, void *stream);
 /* sym_mul_blocks_count with the sketch and Y-count tables of A supplied by the caller (what
- * sym_sketch_rows / sym_ycount would compute; both NULL = computed here). */
+ * sym_sketch_rows / sym_ycount would compute; both NULL = computed here).
+ * speculate (NULL = never; then n_out may be given): a large product whose duplicate detection runs
+ * class by class (ordered-tile class mode) may stop after a sampled first wave of classes that found
+ * no duplicate candidate, no class overflow and no coefficient that can fail zero_threshold. It then
+ * sets *speculate = 1 and *n_out_host = T (the cross-term count), and the caller allocates T rows
+ * and calls sym_mul_blocks_emit_spec instead of sym_mul_blocks_emit. Otherwise *speculate = 0 and
+ * the call is sym_mul_blocks_count. */
 int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a_c, const uint64_t *a_sketch,
                                 const int32_t *a_ycount, int64_t M_total, const uint64_t *b_xz,
                                 const double *b_c, int64_t N, int32_t W, const int64_t *blocks_host,
                                 int32_t nblk, double zero_threshold, int64_t *n_out, int64_t *n_out_host,
-                                void *ws, size_t ws_bytes, void *stream);
+                                int32_t *speculate, void *ws, size_t ws_bytes, void *stream);
 int sym_mul_blocks_emit(const uint64_t *a_xz, const double *a_c, int64_t M_total, const uint64_t *b_xz,
                         const double *b_c, int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk,
                         int64_t U, uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, void *stream);
+/* After a count that set *speculate: finishes the duplicate detection while the rows are written at
+ * their no-duplicate positions (out_xz / out_c hold T rows), sets *n_out_host = U and leaves the
+ * result in rows [0, U). U == T keeps the speculative rows; U < T rewrites rows [0, U) after them.
+ * Stream-ordered like the other calls: work queued on `stream` afterwards sees the finished rows.
+ * The same operands, blocks, zero_threshold and untouched ws as the count. */
+int sym_mul_blocks_emit_spec(const uint64_t *a_xz, const double *a_c, int64_t M_total, const uint64_t *b_xz,
+                             const double *b_c, int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk,
+                             double zero_threshold, uint64_t *out_xz, double *out_c, int64_t *n_out_host,
+                             void *ws, size_t ws_bytes, void *stream);
 
 /* ---- a5 cleanup: symplectic_cleanup (utils.py:230-279) / PauliwordOp.cleanup (base.py:617-638)
  * Unique rows with duplicates' coefficients summed in input order, then |c| > zero_threshold.

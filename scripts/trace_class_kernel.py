@@ -5,8 +5,9 @@ torch.profiler (CUPTI) trace of warmed steps, L2 flushed before each; the class 
 
 `span`: the operands of bench.py's secondary_dedup instead (both from the span of 28 generators, duplicate-heavy).
 
-Writes OUT_DIR/class_kernel_trace.json (device ms per step and kernel, sorted) and the chrome trace beside it.
-Run it on its own: tracing slows the host, so the step times of bench.py are taken without it."""
+Writes OUT_DIR/class_kernel_trace.json (device ms per step and kernel, sorted; per step, the start and end of the class
+kernel launches and of tile_emit_kernel relative to the step's first kernel, which shows whether they overlap) and the
+chrome trace beside it. Run it on its own: tracing slows the host, so the step times of bench.py are taken without it."""
 import json
 import os
 import sys
@@ -53,25 +54,37 @@ def main():
             del R
     trace = os.path.join(out_dir, "class_kernel.pt.trace.json")
     prof.export_chrome_trace(trace)
-    events = [e for e in json.load(open(trace))["traceEvents"] if e.get("cat") == "kernel"]
-    per_kernel = {}
+    events = sorted((e for e in json.load(open(trace))["traceEvents"] if e.get("cat") == "kernel"), key=lambda e: e["ts"])
+    per_kernel, timeline = {}, []
     for e in events:
         name = e["name"]
-        if "fill" in name.lower() and "symb" not in name:          # the L2 flush
+        if "fill" in name.lower() and "symb" not in name:          # the L2 flush: a step starts after it
+            timeline.append({"t0": None, "kernels": []})
             continue
         per_kernel.setdefault(name, []).append(e["dur"] / 1e3)
+        if timeline:
+            step = timeline[-1]
+            if step["t0"] is None:
+                step["t0"] = e["ts"]
+            if "class_dedup" in name or "tile_emit" in name:
+                step["kernels"].append({"name": name.split("(")[0].replace("void symb::", ""),
+                                        "start_ms": round((e["ts"] - step["t0"]) / 1e3, 4),
+                                        "end_ms": round((e["ts"] + e["dur"] - step["t0"]) / 1e3, 4)})
     rows = sorted(((sum(v) / steps, len(v) / steps, k) for k, v in per_kernel.items()), reverse=True)
     result = {
         "gpu": torch.cuda.get_device_name(0), "steps": steps,
         "kernel_ms_per_step": sum(r[0] for r in rows),
         "kernels": [{"ms_per_step": ms, "launches_per_step": n, "name": k} for ms, n, k in rows],
         "class_kernel_ms": [float(np.round(d, 4)) for k, v in per_kernel.items() if "class_dedup" in k for d in v],
+        "timeline": [step["kernels"] for step in timeline],
     }
     with open(os.path.join(out_dir, "class_kernel_trace.json"), "w") as f:
         json.dump(result, f, indent=1)
     for ms, n, k in rows[:8]:
         print(f"{ms:8.3f} ms  x{n:g}  {k[:110]}")
     print("class kernel per step (ms):", result["class_kernel_ms"])
+    for k in result["timeline"][-1]:
+        print(f"{k['start_ms']:8.3f} -> {k['end_ms']:8.3f} ms  {k['name']}")
 
 
 if __name__ == "__main__":

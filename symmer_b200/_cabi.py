@@ -31,9 +31,11 @@ SIGNATURES = {
     "sym_mul_blocks_count": (ctypes.c_int, [c_p, c_p, c_i64, c_p, c_p, c_i64, c_i32, c_p, c_i32, c_f64, c_p, c_p, c_p,
                                             c_sz, c_p]),
     "sym_mul_blocks_count_tables": (ctypes.c_int, [c_p, c_p, c_p, c_p, c_i64, c_p, c_p, c_i64, c_i32, c_p, c_i32, c_f64,
-                                                   c_p, c_p, c_p, c_sz, c_p]),
+                                                   c_p, c_p, c_p, c_p, c_sz, c_p]),
     "sym_mul_blocks_emit": (ctypes.c_int, [c_p, c_p, c_i64, c_p, c_p, c_i64, c_i32, c_p, c_i32, c_i64, c_p, c_p, c_p,
                                            c_sz, c_p]),
+    "sym_mul_blocks_emit_spec": (ctypes.c_int, [c_p, c_p, c_i64, c_p, c_p, c_i64, c_i32, c_p, c_i32, c_f64, c_p, c_p, c_p,
+                                                c_p, c_sz, c_p]),
     "sym_cleanup_ws_bytes": (c_sz, [c_i64, c_i32]),
     "sym_cleanup_count": (ctypes.c_int, [c_p, c_p, c_i64, c_i32, c_f64, c_p, c_p, c_p, c_sz, c_p]),
     "sym_cleanup_emit": (ctypes.c_int, [c_p, c_p, c_i64, c_i32, c_i64, c_p, c_p, c_p, c_sz, c_p]),

@@ -300,7 +300,7 @@ constexpr int CD_SMALL_GROUP = 16;  // hash groups up to this size are ordered b
 template <int THREADS, int CAP, int LOG_SLOTS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB) class_dedup_kernel(ClassJob J, ProductRows rows, TileMap tm, double thr,
                                                                      uint64_t *__restrict__ cand, uint64_t *__restrict__ over,
-                                                                     uint32_t *__restrict__ counters) {
+                                                                     uint32_t *__restrict__ counters, uint32_t c0, uint32_t c1) {
     constexpr int SLOTS = 1 << LOG_SLOTS;
     constexpr int RPT = CAP / THREADS;
     static_assert(CAP % THREADS == 0 && CAP <= 65536 && CAP <= SLOTS, "record ids are 16 bits; candidates are sorted inside the table");
@@ -314,14 +314,13 @@ __global__ void __launch_bounds__(THREADS, MINB) class_dedup_kernel(ClassJob J, 
     __shared__ uint32_t s_warp[33];
     const int tid = threadIdx.x, lane = tid & 31;
     const uint32_t lt = (1u << lane) - 1u;
-    const uint32_t K = 1u << J.k;
     const bool check_thr = !(thr < 0.0 || rows.all_pass());
     const uint32_t bm_words = (((uint32_t)J.nblk << (J.k + 1)) + 31u) / 32u;
     const bool bm_shared = bm_words <= (uint32_t)CD_BM_WORDS;
     if (bm_shared)
         for (uint32_t i = tid; i < bm_words; i += THREADS) s_bits[i] = J.bits[i];
 
-    for (uint32_t c = blockIdx.x; c < K; c += gridDim.x) {
+    for (uint32_t c = c0 + blockIdx.x; c < c1; c += gridDim.x) {
         if (tid == 0) {
             s_count = 0;
             s_ncand = 0;
@@ -560,7 +559,7 @@ __device__ __forceinline__ uint32_t cd_filter_index(uint64_t key) {
 template <int THREADS, int CAP, int LOG_SLOTS, int PRE_LOG>
 __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, ProductRows rows, TileMap tm, double thr,
                                                                     uint64_t *__restrict__ cand, uint64_t *__restrict__ over,
-                                                                    uint32_t *__restrict__ counters, int vbits) {
+                                                                    uint32_t *__restrict__ counters, int vbits, uint32_t c0, uint32_t c1) {
     constexpr int SLOTS = 1 << LOG_SLOTS;
     constexpr int RPT = CAP / THREADS;
     constexpr int PRE_WORDS = PRE_LOG > 0 ? (1 << PRE_LOG) / 32 : 0;
@@ -579,7 +578,6 @@ __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, P
     __shared__ uint32_t s_count, s_nsurv, s_ncand, s_base;
     __shared__ uint32_t s_warp[33];
     const int tid = threadIdx.x;
-    const uint32_t K = 1u << J.k;
     const uint32_t vmask = (1u << vbits) - 1u;
     const bool check_thr = !(thr < 0.0 || rows.all_pass());
     const uint32_t bm_words = (((uint32_t)J.nblk << (J.k + 1)) + 31u) / 32u;
@@ -597,7 +595,7 @@ __global__ void __launch_bounds__(THREADS, 1) class_dedup32_kernel(ClassJob J, P
         if (!keep_test(re, im, thr)) tm.mark_dropped(t);
     };
 
-    for (uint32_t c = blockIdx.x; c < K; c += gridDim.x) {
+    for (uint32_t c = c0 + blockIdx.x; c < c1; c += gridDim.x) {
         if (tid == 0) {
             s_count = 0;
             s_nsurv = 0;
@@ -911,7 +909,7 @@ int g_class_variant = 2;    // tuning knob 11: class kernel (0: 512 threads x 2 
 
 template <int THREADS, int CAP, int LOG_SLOTS, int MINB>
 static int cd_launch(const ClassJob &J, const ProductRows &rows, const TileMap &tm, double thr, uint64_t *cand, uint64_t *over,
-                     uint32_t *counters, cudaStream_t st) {
+                     uint32_t *counters, uint32_t c0, uint32_t c1, uint32_t sms, cudaStream_t st) {
     constexpr size_t smem = ((size_t)1 << LOG_SLOTS) * 8 + (size_t)CAP * 8 + CAP + (size_t)CD_BM_WORDS * 4;
     auto kern = class_dedup_kernel<THREADS, CAP, LOG_SLOTS, MINB>;
     static bool attr_done[64] = {};
@@ -921,45 +919,59 @@ static int cd_launch(const ClassJob &J, const ProductRows &rows, const TileMap &
         SYM_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
-    const uint32_t K = 1u << J.k;
-    const unsigned grid = (unsigned)std::min<uint32_t>(K, (uint32_t)num_sms() * (uint32_t)MINB);
-    kern<<<grid, THREADS, smem, st>>>(J, rows, tm, thr, cand, over, counters);
+    const unsigned grid = (unsigned)std::min<uint32_t>(c1 - c0, sms * (uint32_t)MINB);
+    kern<<<grid, THREADS, smem, st>>>(J, rows, tm, thr, cand, over, counters, c0, c1);
     SYM_LAUNCH_OK();
     return SYM_OK;
 }
 
-// Builds the class tables in `ws` and runs the class kernel. cand / over: capacity T records each.
-int class_dedup_run(ClassJob &J, const uint64_t *a_sk, const uint64_t *b_sk, const ProductRows &rows, const TileMap &tm,
-                    double thr, uint64_t *cand, uint64_t *over, uint32_t *counters, void *ws, size_t ws_bytes,
-                    cudaStream_t st) {
+// The class tables in `ws` (and the scratch of their build): carves the arena and points J at the tables.
+struct CdTables {
+    uint32_t *off, *cursor, *bits, *scratch, *lookp, *vkey, *vq;
+    uint64_t *look8, *vsk;
+};
+static int cd_carve(ClassJob &J, const uint64_t *b_sk, void *ws, size_t ws_bytes, CdTables &t) {
     Arena ar(ws, ws_bytes);
     const size_t tab = cd_table_elems(J);
     const size_t ne = J.n_entries ? J.n_entries : 1, nv = J.n_visits ? J.n_visits : 1;
-    uint32_t *off = ar.take<uint32_t>(2 * tab + 64);
-    uint32_t *cursor = ar.take<uint32_t>(2 * tab + 64);
-    uint32_t *bits = ar.take<uint32_t>(tab / 32 + 64);
-    uint32_t *scratch = ar.take<uint32_t>(scan_scratch_elems((int64_t)(2 * tab)));
-    uint64_t *look8 = ar.take<uint64_t>(ne);
-    uint32_t *lookp = ar.take<uint32_t>(ne);
-    const size_t nvp = cd_padded_visits(J.n_visits);
-    uint32_t *vkey = ar.take<uint32_t>(nvp);
-    uint32_t *vq = ar.take<uint32_t>(nv);
-    uint64_t *vsk = ar.take<uint64_t>(nv);
-    if (!vsk) {
+    t.off = ar.take<uint32_t>(2 * tab + 64);
+    t.cursor = ar.take<uint32_t>(2 * tab + 64);
+    t.bits = ar.take<uint32_t>(tab / 32 + 64);
+    t.scratch = ar.take<uint32_t>(scan_scratch_elems((int64_t)(2 * tab)));
+    t.look8 = ar.take<uint64_t>(ne);
+    t.lookp = ar.take<uint32_t>(ne);
+    t.vkey = ar.take<uint32_t>(cd_padded_visits(J.n_visits));
+    t.vq = ar.take<uint32_t>(nv);
+    t.vsk = ar.take<uint64_t>(nv);
+    if (!t.vsk) {
         set_error("workspace arena exhausted (class tables)");
         return SYM_E_WORKSPACE;
     }
-    SYM_CUDA_OK(cudaMemsetAsync(off, 0, sizeof(uint32_t) * (2 * tab + 64), st));
-    SYM_CUDA_OK(cudaMemsetAsync(cursor, 0, sizeof(uint32_t) * (2 * tab + 64), st));
-    SYM_CUDA_OK(cudaMemsetAsync(counters, 0, sizeof(uint32_t) * 4, st));
     J.b_sk = b_sk;
-    J.off = off;
-    J.bits = bits;
-    J.look8 = look8;
-    J.lookp = lookp;
-    J.vkey = vkey;
-    J.vq = vq;
-    J.vsk = vsk;
+    J.off = t.off;
+    J.bits = t.bits;
+    J.look8 = t.look8;
+    J.lookp = t.lookp;
+    J.vkey = t.vkey;
+    J.vq = t.vq;
+    J.vsk = t.vsk;
+    return SYM_OK;
+}
+
+int class_dedup_bind(ClassJob &J, const uint64_t *b_sk, void *ws, size_t ws_bytes) {
+    CdTables t;
+    return cd_carve(J, b_sk, ws, ws_bytes, t);
+}
+
+int class_dedup_tables(ClassJob &J, const uint64_t *a_sk, const uint64_t *b_sk, uint32_t *counters, void *ws, size_t ws_bytes,
+                       cudaStream_t st) {
+    CdTables t;
+    SYM_TRY(cd_carve(J, b_sk, ws, ws_bytes, t));
+    const size_t tab = cd_table_elems(J);
+    const size_t nvp = cd_padded_visits(J.n_visits);
+    SYM_CUDA_OK(cudaMemsetAsync(t.off, 0, sizeof(uint32_t) * (2 * tab + 64), st));
+    SYM_CUDA_OK(cudaMemsetAsync(t.cursor, 0, sizeof(uint32_t) * (2 * tab + 64), st));
+    SYM_CUDA_OK(cudaMemsetAsync(counters, 0, sizeof(uint32_t) * 4, st));
     // many rows of A per table entry: privatised counters (the visits still take the plain kernels, with no rows of A)
     const bool priv = tab <= 12288 && (size_t)J.n_entries >= 16 * tab && J.n_entries >= (1u << 18);
     const uint32_t n_rows_a = priv ? 0u : J.n_entries;
@@ -971,46 +983,54 @@ int class_dedup_run(ClassJob &J, const uint64_t *a_sk, const uint64_t *b_sk, con
             SYM_CUDA_OK(cudaFuncSetAttribute(cd_place_priv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 12288 * 4));
             attr_done[dev] = true;
         }
-        cd_hist_priv_kernel<<<(J.n_entries + CD_CHUNK - 1) / CD_CHUNK, 1024, tab * 4, st>>>(J, a_sk, off, (uint32_t)tab);
+        cd_hist_priv_kernel<<<(J.n_entries + CD_CHUNK - 1) / CD_CHUNK, 1024, tab * 4, st>>>(J, a_sk, t.off, (uint32_t)tab);
         SYM_LAUNCH_OK();
     }
     const uint32_t n1 = n_rows_a > J.n_visits ? n_rows_a : J.n_visits;
     if (n1) {
-        cd_hist_kernel<<<(n1 + 255) / 256, 256, 0, st>>>(J, a_sk, off, (uint32_t)tab, n_rows_a);
+        cd_hist_kernel<<<(n1 + 255) / 256, 256, 0, st>>>(J, a_sk, t.off, (uint32_t)tab, n_rows_a);
         SYM_LAUNCH_OK();
     }
-    SYM_TRY(scan_exclusive_u32(off, off, (int64_t)(2 * tab), nullptr, scratch, st));
+    SYM_TRY(scan_exclusive_u32(t.off, t.off, (int64_t)(2 * tab), nullptr, t.scratch, st));
     if (priv) {
-        cd_place_priv_kernel<<<(J.n_entries + CD_CHUNK - 1) / CD_CHUNK, 1024, 2 * tab * 4, st>>>(J, a_sk, off, cursor, (uint32_t)tab,
-                                                                                                 look8, lookp);
+        cd_place_priv_kernel<<<(J.n_entries + CD_CHUNK - 1) / CD_CHUNK, 1024, 2 * tab * 4, st>>>(J, a_sk, t.off, t.cursor,
+                                                                                                 (uint32_t)tab, t.look8, t.lookp);
         SYM_LAUNCH_OK();
     }
     uint32_t n2 = n1 > (uint32_t)((tab + 31) / 32) ? n1 : (uint32_t)((tab + 31) / 32);
     if (n2 < (uint32_t)nvp) n2 = (uint32_t)nvp;
-    cd_place_kernel<<<(n2 + 255) / 256, 256, 0, st>>>(J, a_sk, off, cursor, (uint32_t)tab, look8, lookp, vkey, vq, vsk, bits,
-                                                     (uint32_t)nvp, n_rows_a);
+    cd_place_kernel<<<(n2 + 255) / 256, 256, 0, st>>>(J, a_sk, t.off, t.cursor, (uint32_t)tab, t.look8, t.lookp, t.vkey, t.vq,
+                                                     t.vsk, t.bits, (uint32_t)nvp, n_rows_a);
     SYM_LAUNCH_OK();
-    if (J.variant == 2 || J.variant == 3) {
-        constexpr int CAP = 18432;
-        constexpr size_t smem = ((size_t)1 << 15) * 4 + (size_t)CAP * 4 + CAP / 8 + (size_t)CD32_BM_WORDS * 4;   // both shapes
-        auto kern_pre = class_dedup32_kernel<1024, CAP, 14, 18>;   // 64 KB table + 2 x 32 KB presence maps
-        auto kern_old = class_dedup32_kernel<1024, CAP, 15, 0>;    // 128 KB table (tuning knob 11 = 3)
-        static bool attr_done[64] = {};
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-            SYM_CUDA_OK(cudaFuncSetAttribute(kern_pre, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            SYM_CUDA_OK(cudaFuncSetAttribute(kern_old, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            attr_done[dev] = true;
+    return SYM_OK;
+}
+
+int class_dedup_classes(const ClassJob &J, const ProductRows &rows, const TileMap &tm, double thr, uint64_t *cand, uint64_t *over,
+                        uint32_t *counters, uint32_t c0, uint32_t c1, uint32_t sms, cudaStream_t st) {
+    if (c0 < c1) {
+        if (J.variant == 2 || J.variant == 3) {
+            constexpr int CAP = 18432;
+            constexpr size_t smem = ((size_t)1 << 15) * 4 + (size_t)CAP * 4 + CAP / 8 + (size_t)CD32_BM_WORDS * 4;   // both shapes
+            auto kern_pre = class_dedup32_kernel<1024, CAP, 14, 18>;   // 64 KB table + 2 x 32 KB presence maps
+            auto kern_old = class_dedup32_kernel<1024, CAP, 15, 0>;    // 128 KB table (tuning knob 11 = 3)
+            static bool attr_done[64] = {};
+            int dev = 0;
+            cudaGetDevice(&dev);
+            if (dev >= 0 && dev < 64 && !attr_done[dev]) {
+                SYM_CUDA_OK(cudaFuncSetAttribute(kern_pre, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                SYM_CUDA_OK(cudaFuncSetAttribute(kern_old, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                attr_done[dev] = true;
+            }
+            const unsigned grid = (unsigned)std::min<uint32_t>(c1 - c0, sms);
+            const int vbits = cd_bits_for((uint32_t)cd_padded_visits(J.n_visits));
+            if (J.variant == 2) kern_pre<<<grid, 1024, smem, st>>>(J, rows, tm, thr, cand, over, counters, vbits, c0, c1);
+            else kern_old<<<grid, 1024, smem, st>>>(J, rows, tm, thr, cand, over, counters, vbits, c0, c1);
+            SYM_LAUNCH_OK();
+        } else if (class_cap(J.variant) == 9216) {
+            SYM_TRY((cd_launch<1024, 9216, 14, 1>(J, rows, tm, thr, cand, over, counters, c0, c1, sms, st)));
+        } else {
+            SYM_TRY((cd_launch<512, 4096, 13, 2>(J, rows, tm, thr, cand, over, counters, c0, c1, sms, st)));
         }
-        const unsigned grid = (unsigned)std::min<uint32_t>(1u << J.k, (uint32_t)num_sms());
-        if (J.variant == 2) kern_pre<<<grid, 1024, smem, st>>>(J, rows, tm, thr, cand, over, counters, cd_bits_for((uint32_t)nvp));
-        else kern_old<<<grid, 1024, smem, st>>>(J, rows, tm, thr, cand, over, counters, cd_bits_for((uint32_t)nvp));
-        SYM_LAUNCH_OK();
-    } else if (class_cap(J.variant) == 9216) {
-        SYM_TRY((cd_launch<1024, 9216, 14, 1>(J, rows, tm, thr, cand, over, counters, st)));
-    } else {
-        SYM_TRY((cd_launch<512, 4096, 13, 2>(J, rows, tm, thr, cand, over, counters, st)));
     }
     cd_total_kernel<<<1, 1, 0, st>>>(counters);
     SYM_LAUNCH_OK();

@@ -868,8 +868,15 @@ __global__ void __launch_bounds__(256) seg_count_kernel(TileMap tm) {
 // 4-bit field per row and XOR-shuffle-reduced over the W lanes of the row (all UN rows in one
 // word), then 3*(Ya+Yb) is added. Lane u of a row group writes the coefficient a[p]*b[q]*i^e of row
 // u; group sums overwrite theirs in the fix-up pass. The kernel stays HBM-write bound.
-template <int LW>
-__global__ void __launch_bounds__((TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 256)
+// SPEC (speculative emission of a class-mode product, see dedup_product_spec_classes): nothing is dropped, so row j of
+// segment (ql, ptile) goes to slot t_base + ql * m_blk + ptile * TILE_ROWS + j. The kernel then reads neither `drop`
+// nor `segoff`, which the duplicate detection is still writing while it runs; rows and coefficients are those the
+// plain form writes when no drop bit is set.
+// The SPEC form is held to the plain form's occupancy (at LW = 4, 4 CTAs of 256 threads per SM): left alone, ptxas
+// gives it 75 registers and 3 CTAs per SM there.
+template <int LW, bool SPEC>
+__global__ void __launch_bounds__((TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 256,
+                                  SPEC ? (LW <= 1 ? 2048 : 1024) / ((TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 256) : 0)
     tile_emit_kernel(const uint64_t *__restrict__ A, const double2 *__restrict__ Ac, const int32_t *__restrict__ Ay,
                      const uint64_t *__restrict__ B, const double2 *__restrict__ Bc, const int32_t *__restrict__ By,
                      TileBlock first, const TileBlock *__restrict__ blocks, uint32_t qg, const uint32_t *__restrict__ drop,
@@ -908,8 +915,8 @@ __global__ void __launch_bounds__((TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 
     for (uint32_t ql = q_lo; ql < q_hi; ++ql) {
         const uint32_t s = blk.seg_base + ql * blk.ptiles + ptile;
         const size_t qrow = (size_t)(blk.q0 + ql);
-        const uint4 d = reinterpret_cast<const uint4 *>(drop)[s];
-        const uint32_t base = segoff[s];
+        const uint4 d = SPEC ? make_uint4(0u, 0u, 0u, 0u) : reinterpret_cast<const uint4 *>(drop)[s];
+        const uint32_t base = SPEC ? blk.t_base + ql * blk.m_blk + ptile * TILE_ROWS : segoff[s];
         const uint64_t xb = B[qrow * (2 * W) + c], zb = B[qrow * (2 * W) + W + c];
         const uint32_t yb3 = (3u * (uint32_t)By[qrow]) & 3u;
         const uint32_t k[4] = {vm[0] & ~d.x, vm[1] & ~d.y, vm[2] & ~d.z, vm[3] & ~d.w};
@@ -1246,36 +1253,15 @@ static int class_group_pass(const ProductRows &rows, const ProductRows &rows_sum
     return SYM_OK;
 }
 
-// Class mode of the ordered-tile product (class_dedup.cu): no record array, no global sort. The candidate
-// array (L.alt) holds, class by class, the records that have a same-hash mate, sorted by (hash, t); the
-// group pass runs over all of them with device-side counts, so the common case (no class overflow) costs
-// one stream synchronisation like the sort path. Overflowed classes take the global sort afterwards and
-// are appended to the candidate array.
-int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, ClassJob &job,
-                               const uint64_t *a_sk, const uint64_t *b_sk, const int32_t *a_y, const int32_t *b_y, void *class_ws,
-                               size_t class_ws_bytes, double thr, int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes,
-                               cudaStream_t st) {
-    if (ws_bytes < dedup_ws_bytes(T)) {
-        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
-    ProductRows rows_sum = rows;
-    if (thr >= 0.0 && rows.N > 0) {
-        SYM_TRY(launch_min_abs_flag(reinterpret_cast<const double2 *>(rows.Ac), (int64_t)rows.M,
-                                    reinterpret_cast<const double2 *>(rows.Bc), (int64_t)rows.N, thr,
-                                    reinterpret_cast<unsigned long long *>(L.scratch), L.total + 2, st));
-        rows_sum.pass_all = L.total + 2;
-    }
+// Survivor counts per segment and their scan, read on the host; overflowed classes then take the global sort on
+// (hash, t), are appended behind the candidates and get their own group pass. The candidates of the classes have had
+// theirs. U = survivors.
+static int class_count(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const ProductRows &rows_sum,
+                       const TileMap &tm, const ClassJob &job, const int32_t *a_y, const int32_t *b_y, double thr,
+                       const DedupLayout &L, int64_t *n_out, uint32_t &U, cudaStream_t st) {
     uint32_t *counters = L.total + 8;
     uint64_t *cand = L.alt, *over = recs;
-    SYM_TRY(class_dedup_run(job, a_sk, b_sk, rows_sum, tm, thr, cand, over, counters, class_ws, class_ws_bytes, st));
     const int sort_shift = 64 - job.hbits;
-    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, sort_shift, nullptr, counters, L, thr, tm, st));
     uint32_t host[12] = {0};
     for (int attempt = 0; attempt < 2; ++attempt) {
         seg_count_kernel<<<(tm.n_seg + 255) / 256, 256, 0, st>>>(tm);
@@ -1285,7 +1271,6 @@ int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
         SYM_CUDA_OK(cudaStreamSynchronize(st));
         const uint32_t n_cand = host[8], n_over = host[9];
         if (attempt == 1 || n_over == 0u) break;
-        // overflowed classes: global sort of their records on (hash, t), appended behind the candidates
         if ((int64_t)n_cand + (int64_t)n_over > T) {
             set_error("class dedup wrote more records than cross terms");
             return SYM_E_CUDA;
@@ -1301,25 +1286,79 @@ int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
         total_to_i64_kernel<<<1, 1, 0, st>>>(L.total, n_out);
         SYM_LAUNCH_OK();
     }
-    if (n_out_host) *n_out_host = (int64_t)host[0];
+    U = host[0];
     return SYM_OK;
 }
 
-int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
-                             const TileBlock *blocks_host, const int32_t *a_y, const int32_t *b_y, int64_t U,
-                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, bool class_mode, cudaStream_t st) {
-    if (T == 0 || U == 0) return SYM_OK;
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
+static int class_layout(int64_t T, void *ws, size_t ws_bytes, DedupLayout &L) {
+    if (ws_bytes < dedup_ws_bytes(T)) {
+        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
+        return SYM_E_WORKSPACE;
+    }
+    L = dedup_layout(ws, ws_bytes, T);
     if (!L.ok) {
         set_error("workspace arena exhausted");
         return SYM_E_WORKSPACE;
     }
-    const uint64_t *sr = class_mode ? L.alt : ((T > 1 && sorted_in_alt(sort_begin_bit(T, fmt))) ? L.alt : recs);
+    return SYM_OK;
+}
+
+// Class mode of the ordered-tile product (class_dedup.cu): no record array, no global sort. The candidate
+// array (L.alt) holds, class by class, the records that have a same-hash mate, sorted by (hash, t); the
+// group pass runs over all of them with device-side counts, so the common case (no class overflow) costs
+// one stream synchronisation like the sort path. Overflowed classes take the global sort afterwards and
+// are appended to the candidate array.
+// speculate != nullptr: the product may take the speculative emission (dedup_product_spec_classes). The class kernel
+// first runs one wave, one class per SM, as a sample; the host reads its candidate and overflow counts and the
+// pass_all flag. All clean: *speculate = true, *n_out_host = T, and the rest of the classes is left to
+// dedup_product_spec_classes. Otherwise the rest runs here as it does without the sample, one host round trip later.
+int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, ClassJob &job,
+                               const uint64_t *a_sk, const uint64_t *b_sk, const int32_t *a_y, const int32_t *b_y, void *class_ws,
+                               size_t class_ws_bytes, double thr, int64_t *n_out, int64_t *n_out_host, bool *speculate, void *ws,
+                               size_t ws_bytes, cudaStream_t st) {
+    DedupLayout L;
+    SYM_TRY(class_layout(T, ws, ws_bytes, L));
+    ProductRows rows_sum = rows;
+    if (thr >= 0.0 && rows.N > 0) {
+        SYM_TRY(launch_min_abs_flag(reinterpret_cast<const double2 *>(rows.Ac), (int64_t)rows.M,
+                                    reinterpret_cast<const double2 *>(rows.Bc), (int64_t)rows.N, thr,
+                                    reinterpret_cast<unsigned long long *>(L.scratch), L.total + 2, st));
+        rows_sum.pass_all = L.total + 2;
+    }
+    uint32_t *counters = L.total + 8;
+    uint64_t *cand = L.alt, *over = recs;
+    SYM_TRY(class_dedup_tables(job, a_sk, b_sk, counters, class_ws, class_ws_bytes, st));
+    const uint32_t K = 1u << job.k, sms = (uint32_t)num_sms();
+    uint32_t c0 = 0;
+    if (speculate) *speculate = false;
+    if (speculate && K > sms) {
+        SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, counters, 0, sms, sms, st));
+        uint32_t host[12] = {0};
+        SYM_CUDA_OK(cudaMemcpyAsync(host, L.total, sizeof(host), cudaMemcpyDeviceToHost, st));
+        SYM_CUDA_OK(cudaStreamSynchronize(st));
+        c0 = sms;
+        const bool all_pass = thr < 0.0 || host[2] != 0u;
+        if (host[8] == 0u && host[9] == 0u && all_pass) {
+            *speculate = true;
+            if (n_out_host) *n_out_host = T;
+            return SYM_OK;
+        }
+    }
+    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, counters, c0, K, sms, st));
+    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, 64 - job.hbits, nullptr, counters, L, thr, tm, st));
+    uint32_t U = 0;
+    SYM_TRY(class_count(recs, T, fmt, rows, rows_sum, tm, job, a_y, b_y, thr, L, n_out, U, st));
+    if (n_out_host) *n_out_host = (int64_t)U;
+    return SYM_OK;
+}
+
+// tile_emit_kernel over every block of the list on stream st, between the optional emission events
+template <bool SPEC>
+static int launch_tile_emit(const ProductRows &rows, const TileMap &tm, const TileBlock *blocks_host, const int32_t *a_y,
+                            const int32_t *b_y, uint64_t *out_xz, double2 *oc, cudaStream_t st) {
     const int chunks = rows.words / 2;
     const double2 *Ac = reinterpret_cast<const double2 *>(rows.Ac), *Bc = reinterpret_cast<const double2 *>(rows.Bc);
-    double2 *oc = reinterpret_cast<double2 *>(out_c);
     const uint32_t qg = (uint32_t)(g_tile_qgroup < 1 ? 1 : g_tile_qgroup);
-    if (g_emit_ev0) SYM_CUDA_OK(cudaEventRecord(g_emit_ev0, st));
     uint32_t gx = 0, gy = 0;
     for (int b = 0; b < tm.nblk; ++b) {
         const TileBlock blk = blocks_host[b];
@@ -1331,10 +1370,11 @@ int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const 
         set_error("too many B rows for one tile launch");
         return SYM_E_UNSUPPORTED;
     }
+    if (g_emit_ev0) SYM_CUDA_OK(cudaEventRecord(g_emit_ev0, st));
     if (gx > 0 && gy > 0) {
         dim3 grid(gx, gy, (unsigned)tm.nblk);
 #define TILE_EMIT(LW) \
-    tile_emit_kernel<LW><<<grid, (TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 256, 0, st>>>(                 \
+    tile_emit_kernel<LW, SPEC><<<grid, (TILE_ROWS << LW) < 256 ? (TILE_ROWS << LW) : 256, 0, st>>>(             \
         rows.A, Ac, a_y, rows.B, Bc, b_y, tm.first, tm.blocks, qg, tm.drop, tm.segoff, out_xz, oc)
         switch (chunks) {
             case 1: TILE_EMIT(0); break;
@@ -1348,10 +1388,93 @@ int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const 
         SYM_LAUNCH_OK();
     }
     if (g_emit_ev1) SYM_CUDA_OK(cudaEventRecord(g_emit_ev1, st));
+    return SYM_OK;
+}
+
+int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
+                             const TileBlock *blocks_host, const int32_t *a_y, const int32_t *b_y, int64_t U,
+                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, bool class_mode, cudaStream_t st) {
+    if (T == 0 || U == 0) return SYM_OK;
+    DedupLayout L = dedup_layout(ws, ws_bytes, T);
+    if (!L.ok) {
+        set_error("workspace arena exhausted");
+        return SYM_E_WORKSPACE;
+    }
+    const uint64_t *sr = class_mode ? L.alt : ((T > 1 && sorted_in_alt(sort_begin_bit(T, fmt))) ? L.alt : recs);
+    double2 *oc = reinterpret_cast<double2 *>(out_c);
+    SYM_TRY(launch_tile_emit<false>(rows, tm, blocks_host, a_y, b_y, out_xz, oc, st));
     const WorkList wl = class_mode ? class_worklist(L, T, nullptr, L.total + 11) : tile_worklist(L, T);
     tile_fixup_kernel<<<wl.nreg * WORK_SPLIT, 256, 0, st>>>(tm, fmt, sr, wl, L.multi, L.acc, oc);
     SYM_LAUNCH_OK();
     return SYM_OK;
+}
+
+// Library-owned stream (non-blocking: it must not serialise with a legacy default stream) and events of the current
+// device for the speculative emission. One per device, created on first use and shared by every call: like the emission
+// events and the kernel attribute flags, this assumes one host thread issues the products of a device at a time.
+struct SideStream {
+    cudaStream_t s;
+    cudaEvent_t ready, done;
+};
+static int side_stream(SideStream *&out) {
+    static SideStream per_dev[64] = {};
+    int dev = 0;
+    SYM_CUDA_OK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) {
+        set_error("device ordinal %d out of range", dev);
+        return SYM_E_UNSUPPORTED;
+    }
+    SideStream &ss = per_dev[dev];
+    if (!ss.s) {
+        SYM_CUDA_OK(cudaEventCreateWithFlags(&ss.ready, cudaEventDisableTiming));
+        SYM_CUDA_OK(cudaEventCreateWithFlags(&ss.done, cudaEventDisableTiming));
+        SYM_CUDA_OK(cudaStreamCreateWithFlags(&ss.s, cudaStreamNonBlocking));
+    }
+    out = &ss;
+    return SYM_OK;
+}
+
+// Speculative emission of a class-mode product whose sampled first wave was clean (dedup_product_plan_classes set
+// *speculate): out_xz / out_c hold T rows. The rest of the classes runs on the caller's stream as persistent CTAs on a
+// quarter of the SMs, followed by the group pass and the survivor count, while tile_emit_kernel<SPEC> writes every
+// cross term at its no-drop slot from a library stream on the other SMs (and on the class SMs as they free up). The
+// class CTAs are launched first and hold their SMs (1024 threads x 64 registers fill one); on the bench product (B200)
+// the 37 of them finish the classes 3.7 ms into the emission's 5.3 ms, and the emission, which writes at ~91 % of its
+// full-GPU rate on the 111 SMs left to it, takes 0.35 ms longer than alone. The guess was right
+// iff U == T: a group of equal rows, or a row that fails the threshold, always drops at least one row. Then the output
+// is final, and the group pass and the fix-up had nothing to do.
+// U < T: duplicates (or exact cancellations) in classes the sample did not see. The caller's stream waits for the
+// speculative emission, and the plain emission + fix-up write rows [0, U) of the same buffer: such a product pays one
+// extra emission. It needs the duplicates to be sparse enough that ~1/55 of the classes (bench shape) showed none.
+// Either way the caller's stream waits for the library stream before this returns, so work the caller queues after it
+// (and the reuse of out / ws by torch's caching allocator) sees the finished rows.
+int dedup_product_spec_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
+                               const TileBlock *blocks_host, ClassJob &job, const uint64_t *b_sk, const int32_t *a_y,
+                               const int32_t *b_y, void *class_ws, size_t class_ws_bytes, double thr, uint64_t *out_xz,
+                               double *out_c, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st) {
+    DedupLayout L;
+    SYM_TRY(class_layout(T, ws, ws_bytes, L));
+    ProductRows rows_sum = rows;
+    if (thr >= 0.0 && rows.N > 0) rows_sum.pass_all = L.total + 2;   // set by dedup_product_plan_classes
+    SYM_TRY(class_dedup_bind(job, b_sk, class_ws, class_ws_bytes));
+    SideStream *side = nullptr;
+    SYM_TRY(side_stream(side));
+    uint32_t *counters = L.total + 8;
+    const uint32_t K = 1u << job.k, sms = (uint32_t)num_sms();
+    // operand tables and block list were written on st before this point
+    SYM_CUDA_OK(cudaEventRecord(side->ready, st));
+    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, L.alt, recs, counters, std::min(sms, K), K, std::max(1u, sms / 4), st));
+    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, L.alt, T, 64 - job.hbits, nullptr, counters, L, thr, tm, st));
+    SYM_CUDA_OK(cudaStreamWaitEvent(side->s, side->ready, 0));
+    SYM_TRY(launch_tile_emit<true>(rows, tm, blocks_host, a_y, b_y, out_xz, reinterpret_cast<double2 *>(out_c), side->s));
+    SYM_CUDA_OK(cudaEventRecord(side->done, side->s));
+    uint32_t U = 0;
+    const int rc = class_count(recs, T, fmt, rows, rows_sum, tm, job, a_y, b_y, thr, L, nullptr, U, st);
+    SYM_CUDA_OK(cudaStreamWaitEvent(st, side->done, 0));
+    SYM_TRY(rc);
+    if (n_out_host) *n_out_host = (int64_t)U;
+    if ((int64_t)U == T) return SYM_OK;
+    return dedup_product_emit_tiles(recs, T, fmt, rows, tm, blocks_host, a_y, b_y, (int64_t)U, out_xz, out_c, ws, ws_bytes, true, st);
 }
 
 int dedup_product_plan(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, bool by_t, double thr,

@@ -485,6 +485,7 @@ static int mul_blocks_plan(int64_t M_total, int64_t N, int32_t W, const int64_t 
         tb.nq = (uint32_t)(q[3] - q[2]);
         tb.ptiles = (tb.m_blk + TILE_ROWS - 1) / TILE_ROWS;
         tb.seg_base = (uint32_t)segs;
+        tb.t_base = (uint32_t)P.T;
         segs += (int64_t)tb.nq * tb.ptiles;
         P.T += (int64_t)tb.m_blk * tb.nq;
     }
@@ -554,15 +555,17 @@ extern "C" int sym_mul_blocks_count(const uint64_t *a_xz, const double *a_c, int
                                     double zero_threshold, int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes,
                                     void *stream) {
     return sym_mul_blocks_count_tables(a_xz, a_c, nullptr, nullptr, M_total, b_xz, b_c, N, W, blocks_host, nblk,
-                                       zero_threshold, n_out, n_out_host, ws, ws_bytes, stream);
+                                       zero_threshold, n_out, n_out_host, nullptr, ws, ws_bytes, stream);
 }
 
 extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a_c, const uint64_t *a_sketch,
                                            const int32_t *a_ycount, int64_t M_total, const uint64_t *b_xz, const double *b_c,
                                            int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk,
-                                           double zero_threshold, int64_t *n_out, int64_t *n_out_host, void *ws,
-                                           size_t ws_bytes, void *stream) {
+                                           double zero_threshold, int64_t *n_out, int64_t *n_out_host, int32_t *speculate,
+                                           void *ws, size_t ws_bytes, void *stream) {
     SYM_REQUIRE((a_sketch == nullptr) == (a_ycount == nullptr), "a_sketch and a_ycount come together");
+    SYM_REQUIRE(speculate == nullptr || n_out == nullptr, "a speculating count leaves no device count");
+    if (speculate) *speculate = 0;
     MulBlocksPlan P;
     SYM_TRY(mul_blocks_plan(M_total, N, W, blocks_host, nblk, ws, ws_bytes, P));
     cudaStream_t st = (cudaStream_t)stream;
@@ -620,8 +623,12 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
             set_error("workspace arena exhausted (class tables)");
             return SYM_E_WORKSPACE;
         }
-        return dedup_product_plan_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.job, P.a_sk, P.b_sk, P.a_y, P.b_y,
-                                          P.class_ws, P.class_ws_bytes, zero_threshold, n_out, n_out_host, P.rest, P.rest_bytes, st);
+        bool spec = false;
+        SYM_TRY(dedup_product_plan_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.job, P.a_sk, P.b_sk, P.a_y, P.b_y,
+                                           P.class_ws, P.class_ws_bytes, zero_threshold, n_out, n_out_host,
+                                           speculate ? &spec : nullptr, P.rest, P.rest_bytes, st));
+        if (speculate) *speculate = spec ? 1 : 0;
+        return SYM_OK;
     }
     if (P.mode == MODE_TILES)
         return dedup_product_plan_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), zero_threshold, n_out, n_out_host,
@@ -649,6 +656,25 @@ extern "C" int sym_mul_blocks_emit(const uint64_t *a_xz, const double *a_c, int6
                                         out_c, P.rest, P.rest_bytes, P.class_mode, (cudaStream_t)stream);
     return dedup_product_emit(P.recs, P.T, fmt, rows, P.mode == MODE_BY_T, U, out_xz, out_c, P.rest, P.rest_bytes,
                               (cudaStream_t)stream);
+}
+
+extern "C" int sym_mul_blocks_emit_spec(const uint64_t *a_xz, const double *a_c, int64_t M_total, const uint64_t *b_xz,
+                                        const double *b_c, int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk,
+                                        double zero_threshold, uint64_t *out_xz, double *out_c, int64_t *n_out_host, void *ws,
+                                        size_t ws_bytes, void *stream) {
+    MulBlocksPlan P;
+    SYM_TRY(mul_blocks_plan(M_total, N, W, blocks_host, nblk, ws, ws_bytes, P));
+    SYM_REQUIRE(P.class_mode && P.T > 0, "this product takes no speculative emission");
+    if (ws == nullptr || ws_bytes < P.need || P.class_ws == nullptr) {
+        set_error("workspace too small: need %zu bytes, got %zu", P.need, ws_bytes);
+        return SYM_E_WORKSPACE;
+    }
+    ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
+    rows.Minv = fastdiv_magic((uint32_t)M_total);
+    RecFmt fmt{t_bits_for(M_total * N)};
+    return dedup_product_spec_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.blocks, P.job, P.b_sk, P.a_y, P.b_y,
+                                      P.class_ws, P.class_ws_bytes, zero_threshold, out_xz, out_c, n_out_host, P.rest,
+                                      P.rest_bytes, (cudaStream_t)stream);
 }
 
 // the whole product = one block

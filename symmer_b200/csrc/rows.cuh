@@ -164,6 +164,7 @@ constexpr int TILE_ROWS = 128;
 
 struct TileBlock {
     uint32_t p0, m_blk, q0, nq, ptiles, seg_base;
+    uint32_t t_base;   // cross terms of the blocks before this one: the block's first output row when nothing is dropped
 };
 
 __host__ __device__ __forceinline__ uint32_t tile_valid_word(uint32_t m_blk, uint32_t ptile, int w) {
@@ -266,10 +267,17 @@ bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t 
 size_t class_job_ws_bytes(const ClassJob &J);
 // overflow records carry their enumeration position in the term field while they are sorted; this puts t back
 int class_ord_to_t(const ClassJob &J, uint64_t *recs, uint32_t n, cudaStream_t st);
-// cand / over: T records each; counters: device uint32[4] = {candidates, overflow records, overflowed classes, sum}
-int class_dedup_run(ClassJob &J, const uint64_t *a_sk, const uint64_t *b_sk, const ProductRows &rows, const TileMap &tm,
-                    double thr, uint64_t *cand, uint64_t *over, uint32_t *counters, void *ws, size_t ws_bytes,
-                    cudaStream_t st);
+// Builds the class tables in `ws`, points J at them and zeroes counters: device uint32[4] = {candidates, overflow
+// records, overflowed classes, sum}
+int class_dedup_tables(ClassJob &J, const uint64_t *a_sk, const uint64_t *b_sk, uint32_t *counters, void *ws, size_t ws_bytes,
+                       cudaStream_t st);
+// points J at the tables an earlier class_dedup_tables built in the same `ws`
+int class_dedup_bind(ClassJob &J, const uint64_t *b_sk, void *ws, size_t ws_bytes);
+// Runs the class kernel over classes [c0, c1) on at most `sms` SMs, then sets counters[3]. Every class appends its
+// candidates / overflow records at atomically claimed offsets, so launches over disjoint ranges fill cand / over
+// (T records each) exactly as one launch over their union does.
+int class_dedup_classes(const ClassJob &J, const ProductRows &rows, const TileMap &tm, double thr, uint64_t *cand, uint64_t *over,
+                        uint32_t *counters, uint32_t c0, uint32_t c1, uint32_t sms, cudaStream_t st);
 
 // Dedup driver (dedup.cu), split where the survivor count is known so the caller can allocate
 // exact-size outputs. `recs` holds T records (clobbered). by_t: the t fields are a permutation of
@@ -290,11 +298,17 @@ int dedup_plain_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const PlainRow
 int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, double thr,
                              int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
 // class mode: `recs` is only scratch (the overflow array); a_sk / b_sk are the operand sketch tables and
-// class_ws holds the class tables (class_job_ws_bytes)
+// class_ws holds the class tables (class_job_ws_bytes). speculate != nullptr: the product may stop after a sampled
+// first wave of classes with *speculate = true and *n_out_host = T; dedup_product_spec_classes then finishes it.
 int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, ClassJob &job,
                                const uint64_t *a_sk, const uint64_t *b_sk, const int32_t *a_y, const int32_t *b_y, void *class_ws,
-                               size_t class_ws_bytes, double thr, int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes,
-                               cudaStream_t st);
+                               size_t class_ws_bytes, double thr, int64_t *n_out, int64_t *n_out_host, bool *speculate, void *ws,
+                               size_t ws_bytes, cudaStream_t st);
+// the rest of a speculating class-mode product and its output (T rows of capacity); *n_out_host = U
+int dedup_product_spec_classes(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
+                               const TileBlock *blocks_host, ClassJob &job, const uint64_t *b_sk, const int32_t *a_y,
+                               const int32_t *b_y, void *class_ws, size_t class_ws_bytes, double thr, uint64_t *out_xz,
+                               double *out_c, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
 int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
                              const TileBlock *blocks_host, const int32_t *a_y, const int32_t *b_y, int64_t U,
                              uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, bool class_mode, cudaStream_t st);

@@ -176,6 +176,37 @@ def _thr(zero_threshold):
     return -1.0 if zero_threshold is None else float(zero_threshold)
 
 
+def _mul_blocks(a_xz, a_c, b_xz, b_c, flat, nblk, ws, zero_threshold, a_sketch=None, a_ycount=None):
+    """Count + emission of a block-list product; returns (xz[U,2W], c[U]). When the count offers the speculative
+    emission (a large product whose sampled classes showed no duplicate), the output is allocated at T rows and the
+    rows are written while the duplicate detection finishes; a product that turns out to have duplicates after all
+    comes back as the first U rows of that buffer."""
+    M, W = _rows(a_xz)
+    N, _ = _rows(b_xz)
+    L = lib()
+    U = ctypes.c_int64(0)
+    spec = ctypes.c_int32(0)
+    _cabi.check(L.sym_mul_blocks_count_tables(_p(a_xz), _p(_coeff(a_c)), _p(a_sketch), _p(a_ycount), M, _p(b_xz),
+                                              _p(_coeff(b_c)), N, W, flat, nblk, _thr(zero_threshold), None,
+                                              ctypes.byref(U), ctypes.byref(spec), _p(ws), ws.numel(), _stream()))
+    U = U.value
+    out_xz = torch.empty((U, 2 * W), dtype=torch.int64, device=a_xz.device)
+    out_c = torch.empty(U, dtype=torch.complex128, device=a_xz.device)
+    ev = _emit_begin()
+    if spec.value:
+        n = ctypes.c_int64(0)
+        _cabi.check(L.sym_mul_blocks_emit_spec(_p(a_xz), _p(a_c), M, _p(b_xz), _p(b_c), N, W, flat, nblk,
+                                               _thr(zero_threshold), _p(out_xz), _p(out_c), ctypes.byref(n), _p(ws),
+                                               ws.numel(), _stream()))
+        if n.value < U:
+            out_xz, out_c = out_xz[:n.value], out_c[:n.value]
+    else:
+        _cabi.check(L.sym_mul_blocks_emit(_p(a_xz), _p(a_c), M, _p(b_xz), _p(b_c), N, W, flat, nblk, U, _p(out_xz),
+                                          _p(out_c), _p(ws), ws.numel(), _stream()))
+    _emit_end(ev)
+    return out_xz, out_c
+
+
 def mul_cleanup(a_xz, a_c, b_xz, b_c, zero_threshold=1e-15):
     """Fused A*B + cleanup; returns (xz[U,2W], c[U]) in first-occurrence order of t = q*M + p."""
     M, W = _rows(a_xz)
@@ -185,20 +216,8 @@ def mul_cleanup(a_xz, a_c, b_xz, b_c, zero_threshold=1e-15):
     if M * N == 0:
         return (torch.empty((0, 2 * W), dtype=torch.int64, device=dev),
                 torch.empty(0, dtype=torch.complex128, device=dev))
-    L = lib()
-    nbytes = L.sym_mul_cleanup_ws_bytes(M, N, W)
-    ws = workspace(nbytes)
-    U = ctypes.c_int64(0)
-    _cabi.check(L.sym_mul_cleanup_count(_p(a_xz), _p(_coeff(a_c)), M, _p(b_xz), _p(_coeff(b_c)), N, W,
-                                        _thr(zero_threshold), None, ctypes.byref(U), _p(ws), ws.numel(), _stream()))
-    U = U.value
-    out_xz = torch.empty((U, 2 * W), dtype=torch.int64, device=dev)
-    out_c = torch.empty(U, dtype=torch.complex128, device=dev)
-    ev = _emit_begin()
-    _cabi.check(L.sym_mul_cleanup_emit(_p(a_xz), _p(a_c), M, _p(b_xz), _p(b_c), N, W, U, _p(out_xz), _p(out_c),
-                                       _p(ws), ws.numel(), _stream()))
-    _emit_end(ev)
-    return out_xz, out_c
+    ws = workspace(lib().sym_mul_cleanup_ws_bytes(M, N, W))
+    return _mul_blocks(a_xz, a_c, b_xz, b_c, (ctypes.c_int64 * 4)(0, M, 0, N), 1, ws, zero_threshold)
 
 
 def mul_blocks_cleanup(a_xz, a_c, b_xz, b_c, blocks, zero_threshold=1e-15, a_sketch=None, a_ycount=None):
@@ -215,22 +234,11 @@ def mul_blocks_cleanup(a_xz, a_c, b_xz, b_c, blocks, zero_threshold=1e-15, a_ske
         return (torch.empty((0, 2 * W), dtype=torch.int64, device=dev),
                 torch.empty(0, dtype=torch.complex128, device=dev), 0)
     flat = (ctypes.c_int64 * (4 * len(blocks)))(*[v for blk in blocks for v in blk])
-    L = lib()
-    nbytes = L.sym_mul_blocks_ws_bytes(M, N, W, flat, len(blocks))
+    nbytes = lib().sym_mul_blocks_ws_bytes(M, N, W, flat, len(blocks))
     if nbytes == 0:
         _cabi.check(-1)
     ws = workspace(nbytes)
-    U = ctypes.c_int64(0)
-    _cabi.check(L.sym_mul_blocks_count_tables(_p(a_xz), _p(_coeff(a_c)), _p(a_sketch), _p(a_ycount), M, _p(b_xz),
-                                              _p(_coeff(b_c)), N, W, flat, len(blocks), _thr(zero_threshold), None,
-                                              ctypes.byref(U), _p(ws), ws.numel(), _stream()))
-    U = U.value
-    out_xz = torch.empty((U, 2 * W), dtype=torch.int64, device=dev)
-    out_c = torch.empty(U, dtype=torch.complex128, device=dev)
-    ev = _emit_begin()
-    _cabi.check(L.sym_mul_blocks_emit(_p(a_xz), _p(a_c), M, _p(b_xz), _p(b_c), N, W, flat, len(blocks), U, _p(out_xz),
-                                      _p(out_c), _p(ws), ws.numel(), _stream()))
-    _emit_end(ev)
+    out_xz, out_c = _mul_blocks(a_xz, a_c, b_xz, b_c, flat, len(blocks), ws, zero_threshold, a_sketch, a_ycount)
     return out_xz, out_c, T
 
 
