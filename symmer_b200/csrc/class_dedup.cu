@@ -835,9 +835,6 @@ int class_ord_to_t(const ClassJob &J, uint64_t *recs, uint32_t n, cudaStream_t s
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-int g_class_dedup = 1;   // tuning knob 10: 1 (default) = class-local duplicate detection for ordered-tile products, 0 = global record sort
-
-extern int g_class_variant;
 static int cd_bits_for(uint32_t n) {   // bits that hold every index below n
     int b = 1;
     while (b < 32 && (1ull << b) < n) ++b;
@@ -845,9 +842,9 @@ static int cd_bits_for(uint32_t n) {   // bits that hold every index below n
 }
 static int class_cap(int variant) { return (variant == 2 || variant == 3) ? 18432 : (variant == 1 ? 9216 : 4096); }
 
-bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t T, int tb, uint64_t key_mask, ClassJob &J,
-                    bool ignore_knob) {   // ignore_knob: workspace sizing — the shape with the larger tables
-    if ((!g_class_dedup && !ignore_knob) || nblk < 1 || nblk > CD_MAX_BLOCKS || T < 1 || T >= ((int64_t)1 << 32)) return false;
+bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t T, int tb, uint64_t key_mask, int variant,
+                    ClassJob &J) {
+    if (nblk < 1 || nblk > CD_MAX_BLOCKS || T < 1 || T >= ((int64_t)1 << 32)) return false;
     int64_t entries = 0, visits = 0, recs = 0;
     for (int b = 0; b < nblk; ++b) {
         J.entry_base[b] = (uint32_t)entries;
@@ -872,7 +869,7 @@ bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t 
     if (entries >= ((int64_t)1 << 31) || visits >= ((int64_t)1 << 31)) return false;
     // classes: the average class fills at most 85 % of a CTA's pair list; small products still get enough classes
     // to occupy the GPU
-    J.variant = ignore_knob ? 0 : g_class_variant;
+    J.variant = variant;
     if ((J.variant == 2 || J.variant == 3) && cd_bits_for((uint32_t)entries) + cd_bits_for((uint32_t)cd_padded_visits((uint32_t)visits)) > 32) J.variant = 1;
     int64_t target = (int64_t)(0.85 * class_cap(J.variant));
     if (T / 1024 < target) target = T / 1024 > 256 ? T / 1024 : 256;
@@ -902,10 +899,6 @@ size_t class_job_ws_bytes(const ClassJob &J) {
     return 2 * arena_need(2 * tab + 64, 4) + arena_need(tab / 32 + 64, 4) + arena_need(scan_scratch_elems((int64_t)(2 * tab)), 4) +
            arena_need(ne, 8) + arena_need(ne, 4) + arena_need(cd_padded_visits(J.n_visits), 4) + arena_need(nv, 4) + arena_need(nv, 8) + 1024;
 }
-
-int g_class_variant = 2;    // tuning knob 11: class kernel (0: 512 threads x 2 CTAs/SM, 4096 records; 1: 1024 threads, 9216 records;
-                            // 2 (default): compact 4-byte entries, 1024 threads, 18432 records per class, presence filter;
-                            // 3: the same without the filter and with a 32768-slot table)
 
 template <int THREADS, int CAP, int LOG_SLOTS, int MINB>
 static int cd_launch(const ClassJob &J, const ProductRows &rows, const TileMap &tm, double thr, uint64_t *cand, uint64_t *over,

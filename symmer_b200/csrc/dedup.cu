@@ -570,21 +570,6 @@ __global__ void min_abs_flag_finish_kernel(const unsigned long long *__restrict_
     *flag = (isfinite(prod) && prod > 4.0 * thr) ? 1u : 0u;
 }
 
-// mins: two uint64 of scratch (free until the scans run); flag: device uint32
-static int launch_min_abs_flag(const double2 *a, int64_t M, const double2 *b, int64_t N, double thr, unsigned long long *mins,
-                               uint32_t *flag, cudaStream_t st) {
-    SYM_CUDA_OK(cudaMemsetAsync(mins, 0xff, 2 * sizeof(unsigned long long), st));
-    const unsigned ga = (unsigned)std::max<int64_t>(1, std::min<int64_t>((M + 255) / 256, (int64_t)num_sms() * 8));
-    const unsigned gb = (unsigned)std::max<int64_t>(1, std::min<int64_t>((N + 255) / 256, (int64_t)num_sms() * 8));
-    min_abs_kernel<<<ga, 256, 0, st>>>(a, M, mins);
-    SYM_LAUNCH_OK();
-    min_abs_kernel<<<gb, 256, 0, st>>>(b, N, mins + 1);
-    SYM_LAUNCH_OK();
-    min_abs_flag_finish_kernel<<<1, 1, 0, st>>>(mins, thr, flag);
-    SYM_LAUNCH_OK();
-    return SYM_OK;
-}
-
 // Compaction (emit phase): kept_t[slot] = term index of the survivor, out_c[slot] = its coefficient,
 // so that the row-emission kernel has a two-step dependency chain (kept_t -> rows) only.
 template <class Rows, bool BY_T>
@@ -671,6 +656,15 @@ __global__ void __launch_bounds__(256) emit_generic_kernel(Rows rows, const uint
     out_xz[g] = rows.chunk(kept_t[rec], (int)c);
 }
 
+// What a count leaves for the host and for the emission besides its arrays. The class counters, which the class
+// kernels update atomically, have a 32-byte sector of their own.
+struct DedupWords {
+    uint32_t total;                     // survivor count: total of the last exclusive scan
+    uint32_t pass_all;                  // pass_all_flag: no single cross term can fail |c| > thr
+    alignas(32) uint32_t counters[4];   // TILES_CLASS (class_dedup_tables): candidates, overflow records, overflowed
+                                        // classes, end of the candidate array
+};
+
 size_t dedup_ws_bytes(int64_t T) {
     if (T < 1) T = 1;
     size_t n = (size_t)T;
@@ -684,7 +678,7 @@ size_t dedup_ws_bytes(int64_t T) {
            + arena_need(n, 4)                        // slot
            + arena_need(n, 4)                        // kept
            + arena_need(scan_scratch_elems(T), 4)    // scan scratch
-           + arena_need(16, 4) + 4096;
+           + arena_need(1, sizeof(DedupWords)) + 4096;
 }
 
 // Sort on log2(T) + SORT_EXTRA_BITS hash bits, rounded up to whole 8-bit passes. A sort bucket then
@@ -700,14 +694,10 @@ static int sort_begin_bit(int64_t T, RecFmt fmt) {
     return begin;
 }
 
-static bool sorted_in_alt(int begin_bit) {
-    int passes = (64 - begin_bit + 7) / 8;
-    return (passes & 1) != 0;
-}
-
+// The dedup workspace: what the count hands to the emission.
 struct DedupLayout {
-    uint64_t *alt;
-    uint32_t *hist;
+    uint64_t *alt;           // radix sort buffer; TILES_CLASS: the candidate array
+    uint32_t *hist;          // radix histograms
     uint8_t *flag;
     uint32_t *link;
     double2 *acc;
@@ -716,13 +706,29 @@ struct DedupLayout {
     uint32_t *slot;
     uint32_t *kept;
     uint32_t *scratch;
-    uint32_t *total;
-    bool ok;
+    DedupWords *words;
+    uint32_t *total, *pass_all, *counters, *cand_end;   // in *words
+    // ordered-tile paths: the worklist regions in slot + kept (adjacent, both unused there), their counters in hist
+    // (free once the sort is done)
+    uint32_t *work, *work_counts;
+    size_t work_elems;
+
+    // Where the count leaves the records the emission reads again: the candidates of TILES_CLASS, else the sorted
+    // records, which the radix sort leaves in alt after an odd number of passes.
+    template <class R>
+    R *records(Path path, R *recs, int64_t T, RecFmt fmt) const {
+        if (path == Path::TILES_CLASS) return alt;
+        const int passes = (64 - sort_begin_bit(T, fmt) + 7) / 8;
+        return (T > 1 && (passes & 1) != 0) ? alt : recs;
+    }
 };
 
-static DedupLayout dedup_layout(void *ws, size_t ws_bytes, int64_t T) {
+static int dedup_layout_checked(void *ws, size_t ws_bytes, int64_t T, DedupLayout &L) {
+    if (ws_bytes < dedup_ws_bytes(T)) {
+        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
+        return SYM_E_WORKSPACE;
+    }
     Arena ar(ws, ws_bytes);
-    DedupLayout L;
     L.alt = ar.take<uint64_t>((size_t)T);
     L.hist = ar.take<uint32_t>(record_hist_elems(T));
     L.flag = ar.take<uint8_t>((size_t)T);
@@ -733,10 +739,46 @@ static DedupLayout dedup_layout(void *ws, size_t ws_bytes, int64_t T) {
     L.slot = ar.take<uint32_t>((size_t)T);
     L.kept = ar.take<uint32_t>((size_t)T);
     L.scratch = ar.take<uint32_t>(scan_scratch_elems(T));
-    L.total = ar.take<uint32_t>(16);   // [0] scan total, [2] pass_all flag, [8..11] class-mode counters
-    L.ok = L.total != nullptr;
-    return L;
+    L.words = ar.take<DedupWords>(1);
+    L.total = &L.words->total;
+    L.pass_all = &L.words->pass_all;
+    L.counters = L.words->counters;
+    L.cand_end = L.words->counters + 3;
+    L.work = L.slot;
+    L.work_counts = L.hist;
+    L.work_elems = 2 * (arena_need((size_t)T, 4) / 4);
+    return SYM_OK;
 }
+
+// The record sort of a count: sr = its output, which must be where the emission looks for it (L.records).
+static int sort_records(const DedupLayout &L, Path path, uint64_t *recs, int64_t T, RecFmt fmt, uint64_t *&sr,
+                        cudaStream_t st) {
+    SYM_TRY(radix_sort(recs, nullptr, L.alt, nullptr, T, sort_begin_bit(T, fmt), L.hist, &sr, st));
+    if (sr == L.records(path, recs, T, fmt)) return SYM_OK;
+    set_error("internal: the record sort left its output where the emission does not read it");
+    return SYM_E_INVALID;
+}
+
+// The pass_all flag of a product (min_abs_kernel) when the threshold is on; rows_sum = rows reading it.
+static int pass_all_flag(const ProductRows &rows, double thr, const DedupLayout &L, ProductRows &rows_sum, cudaStream_t st) {
+    rows_sum = rows;
+    if (thr < 0.0 || rows.N == 0) return SYM_OK;
+    unsigned long long *mins = reinterpret_cast<unsigned long long *>(L.scratch);   // free until the scans run
+    const int64_t M = rows.M, N = rows.N;
+    SYM_CUDA_OK(cudaMemsetAsync(mins, 0xff, 2 * sizeof(unsigned long long), st));
+    const unsigned ga = (unsigned)std::max<int64_t>(1, std::min<int64_t>((M + 255) / 256, (int64_t)num_sms() * 8));
+    const unsigned gb = (unsigned)std::max<int64_t>(1, std::min<int64_t>((N + 255) / 256, (int64_t)num_sms() * 8));
+    min_abs_kernel<<<ga, 256, 0, st>>>(reinterpret_cast<const double2 *>(rows.Ac), M, mins);
+    SYM_LAUNCH_OK();
+    min_abs_kernel<<<gb, 256, 0, st>>>(reinterpret_cast<const double2 *>(rows.Bc), N, mins + 1);
+    SYM_LAUNCH_OK();
+    min_abs_flag_finish_kernel<<<1, 1, 0, st>>>(mins, thr, L.pass_all);
+    SYM_LAUNCH_OK();
+    rows_sum.pass_all = L.pass_all;
+    return SYM_OK;
+}
+
+static int count_tail(const TileMap *tm, const DedupLayout &L, int64_t *n_out, DedupWords &h, cudaStream_t st);
 
 // Phase 1: everything up to the survivor count (synchronises the stream once to read it).
 template <class Rows, bool BY_T>
@@ -747,18 +789,11 @@ static int dedup_plan(uint64_t *recs, int64_t T, RecFmt fmt, const Rows &rows, d
         if (n_out_host) *n_out_host = 0;
         return SYM_OK;
     }
-    if (ws_bytes < dedup_ws_bytes(T)) {
-        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
+    DedupLayout L;
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
     const int begin = sort_begin_bit(T, fmt);
     uint64_t *sr = nullptr;
-    SYM_TRY(radix_sort(recs, nullptr, L.alt, nullptr, T, begin, L.hist, &sr, st));
+    SYM_TRY(sort_records(L, BY_T ? Path::BY_T : Path::SORTED, recs, T, fmt, sr, st));
 
     const unsigned nb = (unsigned)((T + 255) / 256);
     link_kernel<Rows><<<nb, 256, 0, st>>>(rows, fmt, sr, T, begin, L.flag, L.link);
@@ -768,26 +803,14 @@ static int dedup_plan(uint64_t *recs, int64_t T, RecFmt fmt, const Rows &rows, d
     constexpr bool DIRECT = !BY_T || std::is_same<Rows, PlainRows>::value;
     SYM_CUDA_OK(cudaMemsetAsync(L.multi, 0, (size_t)T, st));
     Rows rows_sum = rows;
-    if constexpr (std::is_same<Rows, ProductRows>::value && !BY_T) {
-        if (thr >= 0.0 && rows.N > 0) {
-            SYM_TRY(launch_min_abs_flag(reinterpret_cast<const double2 *>(rows.Ac), (int64_t)rows.M,
-                                        reinterpret_cast<const double2 *>(rows.Bc), (int64_t)rows.N, thr,
-                                        reinterpret_cast<unsigned long long *>(L.scratch), L.total + 2, st));
-            rows_sum.pass_all = L.total + 2;
-        }
-    }
+    if constexpr (std::is_same<Rows, ProductRows>::value && !BY_T) SYM_TRY(pass_all_flag(rows, thr, L, rows_sum, st));
     sum_kernel<Rows, BY_T, DIRECT><<<nb, 256, 0, st>>>(rows_sum, fmt, sr, T, begin, L.flag, L.link, thr, L.acc, L.keep,
                                                       L.multi);
     SYM_LAUNCH_OK();
     SYM_TRY(scan_exclusive_u8(L.keep, L.slot, T, L.total, L.scratch, st));
-    if (n_out) {
-        total_to_i64_kernel<<<1, 1, 0, st>>>(L.total, n_out);
-        SYM_LAUNCH_OK();
-    }
-    uint32_t U32 = 0;
-    SYM_CUDA_OK(cudaMemcpyAsync(&U32, L.total, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    SYM_CUDA_OK(cudaStreamSynchronize(st));
-    if (n_out_host) *n_out_host = (int64_t)U32;
+    DedupWords h;
+    SYM_TRY(count_tail(nullptr, L, n_out, h, st));
+    if (n_out_host) *n_out_host = (int64_t)h.total;
     return SYM_OK;
 }
 
@@ -797,12 +820,9 @@ template <class Rows, bool BY_T>
 static int dedup_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const Rows &rows, int64_t U, uint64_t *out_xz,
                       double *out_c, void *ws, size_t ws_bytes, cudaStream_t st) {
     if (T == 0 || U == 0) return SYM_OK;
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
-    const uint64_t *sr = (T > 1 && sorted_in_alt(sort_begin_bit(T, fmt))) ? L.alt : recs;
+    DedupLayout L;
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
+    const uint64_t *sr = L.records(BY_T ? Path::BY_T : Path::SORTED, recs, T, fmt);
     const uint32_t chunks = (uint32_t)(rows.words / 2);
     uint4 *o = reinterpret_cast<uint4 *>(out_xz);
     double2 *oc = reinterpret_cast<double2 *>(out_c);
@@ -856,6 +876,23 @@ __global__ void __launch_bounds__(256) seg_count_kernel(TileMap tm) {
     const uint4 d = reinterpret_cast<const uint4 *>(tm.drop)[s];
     tm.segoff[s] = __popc(tile_valid_word(blk.m_blk, ptile, 0) & ~d.x) + __popc(tile_valid_word(blk.m_blk, ptile, 1) & ~d.y) +
                    __popc(tile_valid_word(blk.m_blk, ptile, 2) & ~d.z) + __popc(tile_valid_word(blk.m_blk, ptile, 3) & ~d.w);
+}
+
+// End of a count: for an ordered-tile product (tm != nullptr) the survivors per segment and their scan, then the
+// device count (n_out != nullptr) and the count words on the host (one stream synchronisation).
+static int count_tail(const TileMap *tm, const DedupLayout &L, int64_t *n_out, DedupWords &h, cudaStream_t st) {
+    if (tm) {
+        seg_count_kernel<<<(tm->n_seg + 255) / 256, 256, 0, st>>>(*tm);
+        SYM_LAUNCH_OK();
+        SYM_TRY(scan_exclusive_u32(tm->segoff, tm->segoff, (int64_t)tm->n_seg, L.total, L.scratch, st));
+    }
+    if (n_out) {
+        total_to_i64_kernel<<<1, 1, 0, st>>>(L.total, n_out);
+        SYM_LAUNCH_OK();
+    }
+    SYM_CUDA_OK(cudaMemcpyAsync(&h, L.words, sizeof(DedupWords), cudaMemcpyDeviceToHost, st));
+    SYM_CUDA_OK(cudaStreamSynchronize(st));
+    return SYM_OK;
 }
 
 // Row + coefficient emission of one block, CTA = (tile of TILE_ROWS rows of A) x (QG rows of B).
@@ -969,15 +1006,13 @@ __global__ void __launch_bounds__(256) tile_fixup_kernel(TileMap tm, RecFmt fmt,
     }
 }
 
-// worklist storage: L.slot and L.kept (adjacent, both unused in this mode) hold the regions, the
-// radix histogram buffer (free once the sort is done) holds the counters
 static WorkList tile_worklist(const DedupLayout &L, int64_t T) {
     const int64_t nb = (T + CLS_TILE - 1) / CLS_TILE;   // CTAs of tile_classify_kernel
     WorkList wl;
     wl.nreg = (uint32_t)std::max<int64_t>(1, std::min<int64_t>(2048, nb));
     wl.cap = (uint32_t)std::min<int64_t>(((nb + wl.nreg - 1) / wl.nreg) * CLS_TILE, T);
-    wl.work = L.slot;
-    wl.counts = L.hist;
+    wl.work = L.work;
+    wl.counts = L.work_counts;
     return wl;
 }
 
@@ -985,29 +1020,16 @@ int g_tile_qgroup = 16;   // tuning knob 7: B rows per CTA of tile_emit_kernel
 
 int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm, double thr,
                              int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st) {
-    if (ws_bytes < dedup_ws_bytes(T)) {
-        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
+    DedupLayout L;
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
     const int begin = sort_begin_bit(T, fmt);
     uint64_t *sr = nullptr;
-    SYM_TRY(radix_sort(recs, nullptr, L.alt, nullptr, T, begin, L.hist, &sr, st));
-    const unsigned nb = (unsigned)((T + 255) / 256);
-    ProductRows rows_sum = rows;
-    if (thr >= 0.0 && rows.N > 0) {
-        SYM_TRY(launch_min_abs_flag(reinterpret_cast<const double2 *>(rows.Ac), (int64_t)rows.M,
-                                    reinterpret_cast<const double2 *>(rows.Bc), (int64_t)rows.N, thr,
-                                    reinterpret_cast<unsigned long long *>(L.scratch), L.total + 2, st));
-        rows_sum.pass_all = L.total + 2;
-    }
+    SYM_TRY(sort_records(L, Path::TILES_SORT, recs, T, fmt, sr, st));
+    ProductRows rows_sum;
+    SYM_TRY(pass_all_flag(rows, thr, L, rows_sum, st));
     // worklist of the records that share a sort bucket
     const WorkList wl = tile_worklist(L, T);
-    if ((size_t)wl.nreg * wl.cap > 2 * (arena_need((size_t)T, 4) / 4)) {
+    if ((size_t)wl.nreg * wl.cap > L.work_elems) {
         set_error("worklist does not fit its arena slice");
         return SYM_E_WORKSPACE;
     }
@@ -1021,17 +1043,9 @@ int dedup_product_plan_tiles(uint64_t *recs, int64_t T, RecFmt fmt, const Produc
     SYM_LAUNCH_OK();
     sum_work_kernel<ProductRows><<<wl.nreg * WORK_SPLIT, 256, 0, st>>>(rows_sum, fmt, sr, T, begin, wl, L.flag, L.link, thr, L.acc, L.multi, tm);
     SYM_LAUNCH_OK();
-    seg_count_kernel<<<(tm.n_seg + 255) / 256, 256, 0, st>>>(tm);
-    SYM_LAUNCH_OK();
-    SYM_TRY(scan_exclusive_u32(tm.segoff, tm.segoff, (int64_t)tm.n_seg, L.total, L.scratch, st));
-    if (n_out) {
-        total_to_i64_kernel<<<1, 1, 0, st>>>(L.total, n_out);
-        SYM_LAUNCH_OK();
-    }
-    uint32_t U32 = 0;
-    SYM_CUDA_OK(cudaMemcpyAsync(&U32, L.total, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    SYM_CUDA_OK(cudaStreamSynchronize(st));
-    if (n_out_host) *n_out_host = (int64_t)U32;
+    DedupWords h;
+    SYM_TRY(count_tail(&tm, L, n_out, h, st));
+    if (n_out_host) *n_out_host = (int64_t)h.total;
     return SYM_OK;
 }
 
@@ -1259,47 +1273,29 @@ static int class_group_pass(const ProductRows &rows, const ProductRows &rows_sum
 static int class_count(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const ProductRows &rows_sum,
                        const TileMap &tm, const ClassJob &job, const int32_t *a_y, const int32_t *b_y, double thr,
                        const DedupLayout &L, int64_t *n_out, uint32_t &U, cudaStream_t st) {
-    uint32_t *counters = L.total + 8;
     uint64_t *cand = L.alt, *over = recs;
     const int sort_shift = 64 - job.hbits;
-    uint32_t host[12] = {0};
+    DedupWords h;
     for (int attempt = 0; attempt < 2; ++attempt) {
-        seg_count_kernel<<<(tm.n_seg + 255) / 256, 256, 0, st>>>(tm);
-        SYM_LAUNCH_OK();
-        SYM_TRY(scan_exclusive_u32(tm.segoff, tm.segoff, (int64_t)tm.n_seg, L.total, L.scratch, st));
-        SYM_CUDA_OK(cudaMemcpyAsync(host, L.total, sizeof(host), cudaMemcpyDeviceToHost, st));
-        SYM_CUDA_OK(cudaStreamSynchronize(st));
-        const uint32_t n_cand = host[8], n_over = host[9];
+        SYM_TRY(count_tail(&tm, L, nullptr, h, st));
+        const uint32_t n_cand = h.counters[0], n_over = h.counters[1];
         if (attempt == 1 || n_over == 0u) break;
         if ((int64_t)n_cand + (int64_t)n_over > T) {
             set_error("class dedup wrote more records than cross terms");
             return SYM_E_CUDA;
         }
-        uint64_t *sorted = nullptr;
-        SYM_TRY(radix_sort(over, nullptr, reinterpret_cast<uint64_t *>(L.slot), nullptr, (int64_t)n_over, 2, L.hist,
+        uint64_t *sorted = nullptr;   // the worklist storage holds 8 bytes per cross term: the sort's second buffer
+        SYM_TRY(radix_sort(over, nullptr, reinterpret_cast<uint64_t *>(L.work), nullptr, (int64_t)n_over, 2, L.hist,
                            &sorted, st));
         SYM_CUDA_OK(cudaMemcpyAsync(cand + n_cand, sorted, sizeof(uint64_t) * (size_t)n_over, cudaMemcpyDeviceToDevice, st));
         SYM_TRY(class_ord_to_t(job, cand + n_cand, n_over, st));
-        SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, sort_shift, counters, counters + 3, L, thr, tm, st));
+        SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, sort_shift, L.counters, L.cand_end, L, thr, tm, st));
     }
     if (n_out) {
         total_to_i64_kernel<<<1, 1, 0, st>>>(L.total, n_out);
         SYM_LAUNCH_OK();
     }
-    U = host[0];
-    return SYM_OK;
-}
-
-static int class_layout(int64_t T, void *ws, size_t ws_bytes, DedupLayout &L) {
-    if (ws_bytes < dedup_ws_bytes(T)) {
-        set_error("workspace too small: need %zu bytes, got %zu", dedup_ws_bytes(T), ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
-    L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
+    U = h.total;
     return SYM_OK;
 }
 
@@ -1317,35 +1313,29 @@ int dedup_product_plan_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
                                size_t class_ws_bytes, double thr, int64_t *n_out, int64_t *n_out_host, bool *speculate, void *ws,
                                size_t ws_bytes, cudaStream_t st) {
     DedupLayout L;
-    SYM_TRY(class_layout(T, ws, ws_bytes, L));
-    ProductRows rows_sum = rows;
-    if (thr >= 0.0 && rows.N > 0) {
-        SYM_TRY(launch_min_abs_flag(reinterpret_cast<const double2 *>(rows.Ac), (int64_t)rows.M,
-                                    reinterpret_cast<const double2 *>(rows.Bc), (int64_t)rows.N, thr,
-                                    reinterpret_cast<unsigned long long *>(L.scratch), L.total + 2, st));
-        rows_sum.pass_all = L.total + 2;
-    }
-    uint32_t *counters = L.total + 8;
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
+    ProductRows rows_sum;
+    SYM_TRY(pass_all_flag(rows, thr, L, rows_sum, st));
     uint64_t *cand = L.alt, *over = recs;
-    SYM_TRY(class_dedup_tables(job, a_sk, b_sk, counters, class_ws, class_ws_bytes, st));
+    SYM_TRY(class_dedup_tables(job, a_sk, b_sk, L.counters, class_ws, class_ws_bytes, st));
     const uint32_t K = 1u << job.k, sms = (uint32_t)num_sms();
     uint32_t c0 = 0;
     if (speculate) *speculate = false;
     if (speculate && K > sms) {
-        SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, counters, 0, sms, sms, st));
-        uint32_t host[12] = {0};
-        SYM_CUDA_OK(cudaMemcpyAsync(host, L.total, sizeof(host), cudaMemcpyDeviceToHost, st));
-        SYM_CUDA_OK(cudaStreamSynchronize(st));
+        SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, L.counters, 0, sms, sms, st));
+        DedupWords h;
+        SYM_TRY(count_tail(nullptr, L, nullptr, h, st));
         c0 = sms;
-        const bool all_pass = thr < 0.0 || host[2] != 0u;
-        if (host[8] == 0u && host[9] == 0u && all_pass) {
+        const bool all_pass = thr < 0.0 || h.pass_all != 0u;
+        if (h.counters[0] == 0u && h.counters[1] == 0u && all_pass) {
             *speculate = true;
             if (n_out_host) *n_out_host = T;
             return SYM_OK;
         }
     }
-    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, counters, c0, K, sms, st));
-    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, 64 - job.hbits, nullptr, counters, L, thr, tm, st));
+    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, cand, over, L.counters, c0, K, sms, st));
+    // the group pass over the candidates of the classes: positions [0, counters[0])
+    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, cand, T, 64 - job.hbits, nullptr, L.counters, L, thr, tm, st));
     uint32_t U = 0;
     SYM_TRY(class_count(recs, T, fmt, rows, rows_sum, tm, job, a_y, b_y, thr, L, n_out, U, st));
     if (n_out_host) *n_out_host = (int64_t)U;
@@ -1391,19 +1381,16 @@ static int launch_tile_emit(const ProductRows &rows, const TileMap &tm, const Ti
     return SYM_OK;
 }
 
-int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
+int dedup_product_emit_tiles(Path path, const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
                              const TileBlock *blocks_host, const int32_t *a_y, const int32_t *b_y, int64_t U,
-                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, bool class_mode, cudaStream_t st) {
+                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, cudaStream_t st) {
     if (T == 0 || U == 0) return SYM_OK;
-    DedupLayout L = dedup_layout(ws, ws_bytes, T);
-    if (!L.ok) {
-        set_error("workspace arena exhausted");
-        return SYM_E_WORKSPACE;
-    }
-    const uint64_t *sr = class_mode ? L.alt : ((T > 1 && sorted_in_alt(sort_begin_bit(T, fmt))) ? L.alt : recs);
+    DedupLayout L;
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
+    const uint64_t *sr = L.records(path, recs, T, fmt);
     double2 *oc = reinterpret_cast<double2 *>(out_c);
     SYM_TRY(launch_tile_emit<false>(rows, tm, blocks_host, a_y, b_y, out_xz, oc, st));
-    const WorkList wl = class_mode ? class_worklist(L, T, nullptr, L.total + 11) : tile_worklist(L, T);
+    const WorkList wl = path == Path::TILES_CLASS ? class_worklist(L, T, nullptr, L.cand_end) : tile_worklist(L, T);
     tile_fixup_kernel<<<wl.nreg * WORK_SPLIT, 256, 0, st>>>(tm, fmt, sr, wl, L.multi, L.acc, oc);
     SYM_LAUNCH_OK();
     return SYM_OK;
@@ -1453,18 +1440,17 @@ int dedup_product_spec_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
                                const int32_t *b_y, void *class_ws, size_t class_ws_bytes, double thr, uint64_t *out_xz,
                                double *out_c, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st) {
     DedupLayout L;
-    SYM_TRY(class_layout(T, ws, ws_bytes, L));
+    SYM_TRY(dedup_layout_checked(ws, ws_bytes, T, L));
     ProductRows rows_sum = rows;
-    if (thr >= 0.0 && rows.N > 0) rows_sum.pass_all = L.total + 2;   // set by dedup_product_plan_classes
+    if (thr >= 0.0 && rows.N > 0) rows_sum.pass_all = L.pass_all;   // the count's pass_all_flag
     SYM_TRY(class_dedup_bind(job, b_sk, class_ws, class_ws_bytes));
     SideStream *side = nullptr;
     SYM_TRY(side_stream(side));
-    uint32_t *counters = L.total + 8;
     const uint32_t K = 1u << job.k, sms = (uint32_t)num_sms();
     // operand tables and block list were written on st before this point
     SYM_CUDA_OK(cudaEventRecord(side->ready, st));
-    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, L.alt, recs, counters, std::min(sms, K), K, std::max(1u, sms / 4), st));
-    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, L.alt, T, 64 - job.hbits, nullptr, counters, L, thr, tm, st));
+    SYM_TRY(class_dedup_classes(job, rows_sum, tm, thr, L.alt, recs, L.counters, std::min(sms, K), K, std::max(1u, sms / 4), st));
+    SYM_TRY(class_group_pass(rows, rows_sum, a_y, b_y, fmt, L.alt, T, 64 - job.hbits, nullptr, L.counters, L, thr, tm, st));
     SYM_CUDA_OK(cudaStreamWaitEvent(side->s, side->ready, 0));
     SYM_TRY(launch_tile_emit<true>(rows, tm, blocks_host, a_y, b_y, out_xz, reinterpret_cast<double2 *>(out_c), side->s));
     SYM_CUDA_OK(cudaEventRecord(side->done, side->s));
@@ -1474,18 +1460,19 @@ int dedup_product_spec_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
     SYM_TRY(rc);
     if (n_out_host) *n_out_host = (int64_t)U;
     if ((int64_t)U == T) return SYM_OK;
-    return dedup_product_emit_tiles(recs, T, fmt, rows, tm, blocks_host, a_y, b_y, (int64_t)U, out_xz, out_c, ws, ws_bytes, true, st);
+    return dedup_product_emit_tiles(Path::TILES_CLASS, recs, T, fmt, rows, tm, blocks_host, a_y, b_y, (int64_t)U, out_xz, out_c,
+                                    ws, ws_bytes, st);
 }
 
-int dedup_product_plan(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, bool by_t, double thr,
+int dedup_product_plan(Path path, uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, double thr,
                        int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st) {
-    if (by_t) return dedup_plan<ProductRows, true>(recs, T, fmt, rows, thr, n_out, n_out_host, ws, ws_bytes, st);
+    if (path == Path::BY_T) return dedup_plan<ProductRows, true>(recs, T, fmt, rows, thr, n_out, n_out_host, ws, ws_bytes, st);
     return dedup_plan<ProductRows, false>(recs, T, fmt, rows, thr, n_out, n_out_host, ws, ws_bytes, st);
 }
 
-int dedup_product_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, bool by_t, int64_t U,
+int dedup_product_emit(Path path, const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, int64_t U,
                        uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, cudaStream_t st) {
-    if (by_t) return dedup_emit<ProductRows, true>(recs, T, fmt, rows, U, out_xz, out_c, ws, ws_bytes, st);
+    if (path == Path::BY_T) return dedup_emit<ProductRows, true>(recs, T, fmt, rows, U, out_xz, out_c, ws, ws_bytes, st);
     return dedup_emit<ProductRows, false>(recs, T, fmt, rows, U, out_xz, out_c, ws, ws_bytes, st);
 }
 

@@ -353,7 +353,7 @@ extern "C" int sym_dedup_records_count(uint64_t *recs, int64_t T, const uint64_t
     SYM_REQUIRE(M_total * N < (int64_t)4000000000LL, "M_total*N must be < 4e9");
     ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
     RecFmt fmt{t_bits_for(M_total * N)};
-    return dedup_product_plan(recs, T, fmt, rows, false, zero_threshold, n_out, n_out_host, ws, ws_bytes,
+    return dedup_product_plan(Path::SORTED, recs, T, fmt, rows, zero_threshold, n_out, n_out_host, ws, ws_bytes,
                               (cudaStream_t)stream);
 }
 
@@ -364,7 +364,7 @@ extern "C" int sym_dedup_records_emit(const uint64_t *recs, int64_t T, const uin
     SYM_REQUIRE(M_total >= 1 && N >= 1 && W >= 1, "bad size");
     ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
     RecFmt fmt{t_bits_for(M_total * N)};
-    return dedup_product_emit(recs, T, fmt, rows, false, U, out_xz, out_c, ws, ws_bytes, (cudaStream_t)stream);
+    return dedup_product_emit(Path::SORTED, recs, T, fmt, rows, U, out_xz, out_c, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int sym_dedup_records(uint64_t *recs, int64_t T, const uint64_t *a_xz, const double *a_c, int64_t M_total,
@@ -382,17 +382,23 @@ extern "C" int sym_dedup_records(uint64_t *recs, int64_t T, const uint64_t *a_xz
     return sym_dedup_records_emit(recs, T, a_xz, a_c, M_total, b_xz, b_c, N, W, U, out_xz, out_c, ws, ws_bytes, stream);
 }
 
-// Below this many cross terms the product is emitted in first-occurrence (reference) order; above,
-// in sorted-hash order, which keeps every pass of the dedup streaming (no T-sized scatters).
-static int64_t g_by_t_limit = (int64_t)1 << 22;
-// tuning knob 6: 1 (default) = products above the limit use the ordered-tile mode (first-occurrence
-// order at every size, streaming tiled row emission); 0 = the sorted-hash order path
-static int g_ordered_tiles = 1;
-namespace symb { extern int g_apply_variant; extern int g_rref_variant; extern int g_tile_qgroup; extern int g_onesweep; extern int g_class_dedup; extern int g_class_variant; }
+// Tuning knobs that select the path of a product (mul_blocks_plan reads them, nothing else does):
+//   0  by_t_limit: below this many cross terms a whole product is emitted in first-occurrence (reference) order by t;
+//      above, in the ordered-tile mode or in sorted-hash order, which keeps every pass of the dedup streaming (no
+//      T-sized scatters)
+//   6  ordered_tiles: 1 (default) = products above the limit use the ordered-tile mode (first-occurrence order at every
+//      size, streaming tiled row emission); 0 = the sorted-hash order path
+//   10 class_dedup: 1 (default) = class-local duplicate detection for ordered-tile products, 0 = global record sort
+//   11 class_variant: class kernel (0: 512 threads x 2 CTAs/SM, 4096 records; 1: 1024 threads, 9216 records;
+//      2 (default): compact 4-byte entries, 1024 threads, 18432 records per class, presence filter;
+//      3: the same without the filter and with a 32768-slot table)
+struct PathKnobs { int64_t by_t_limit; int ordered_tiles, class_dedup, class_variant; };
+static PathKnobs g_path_knobs = {(int64_t)1 << 22, 1, 1, 2};
+namespace symb { extern int g_apply_variant; extern int g_rref_variant; extern int g_tile_qgroup; extern int g_onesweep; }
 
 extern "C" int sym_set_tuning(int32_t which, int64_t value) {
     if (which == 0) {
-        g_by_t_limit = value;
+        g_path_knobs.by_t_limit = value;
         return SYM_OK;
     }
     if (which == 4) {
@@ -404,7 +410,7 @@ extern "C" int sym_set_tuning(int32_t which, int64_t value) {
         return SYM_OK;
     }
     if (which == 6) {
-        g_ordered_tiles = (int)value;
+        g_path_knobs.ordered_tiles = (int)value;
         return SYM_OK;
     }
     if (which == 7) {
@@ -416,11 +422,11 @@ extern "C" int sym_set_tuning(int32_t which, int64_t value) {
         return SYM_OK;
     }
     if (which == 10) {
-        symb::g_class_dedup = (int)value;
+        g_path_knobs.class_dedup = (int)value;
         return SYM_OK;
     }
     if (which == 11) {
-        symb::g_class_variant = (int)value;
+        g_path_knobs.class_variant = (int)value;
         return SYM_OK;
     }
     set_error("unknown tuning knob %d", which);
@@ -435,11 +441,10 @@ extern "C" int sym_set_emit_events(void *before_event, void *after_event) {
 // ---------------------------------------------------------------------------------------------
 // product + cleanup of a list of rectangular blocks of A x B (one block = the whole product)
 // ---------------------------------------------------------------------------------------------
-enum MulMode { MODE_BY_T = 0, MODE_SORTED = 1, MODE_TILES = 2 };
-
 struct MulBlocksPlan {
-    MulMode mode;
+    Path path;
     int64_t T;
+    RecFmt fmt;
     int nblk;
     uint32_t n_seg;
     TileBlock blocks[256];
@@ -447,26 +452,28 @@ struct MulBlocksPlan {
     uint64_t *a_sk, *b_sk;
     int32_t *a_y, *b_y;
     uint64_t *recs;
-    TileBlock *d_blocks;
+    TileBlock *d_blocks;   // ordered-tile paths
     uint32_t *drop;
     uint32_t *segoff;
-    bool class_mode;     // ordered tiles with class-local duplicate detection (class_dedup.cu) instead of the record sort
-    ClassJob job;
+    ClassJob job;          // TILES_CLASS
     void *class_ws;
     size_t class_ws_bytes;
     void *rest;
     size_t rest_bytes;
     size_t need;
+
+    bool tiles() const { return path == Path::TILES_SORT || path == Path::TILES_CLASS; }
 };
 
 static int mul_blocks_plan(int64_t M_total, int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk, void *ws,
-                           size_t ws_bytes, MulBlocksPlan &P) {
+                           size_t ws_bytes, MulBlocksPlan &P, const PathKnobs &knobs = g_path_knobs) {
     SYM_REQUIRE(M_total >= 0 && N >= 0 && W >= 1, "bad size");
     SYM_REQUIRE(nblk >= 0 && nblk <= 256, "at most 256 blocks");
     SYM_REQUIRE(M_total * N < (int64_t)4000000000LL, "M_total*N must be < 4e9 cross terms per call");
     SYM_REQUIRE(nblk == 0 || blocks_host != nullptr, "blocks_host is NULL");
     P.nblk = nblk;
     P.T = 0;
+    P.fmt = RecFmt{t_bits_for(M_total * N)};
     int64_t segs = 0;
     for (int b = 0; b < nblk; ++b) {
         const int64_t *q = blocks_host + 4 * b;
@@ -491,12 +498,15 @@ static int mul_blocks_plan(int64_t M_total, int64_t N, int32_t W, const int64_t 
     }
     const bool whole = nblk == 1 && P.blocks[0].p0 == 0 && P.blocks[0].q0 == 0 && P.blocks[0].m_blk == M_total &&
                        P.blocks[0].nq == N;
-    const bool tiles_ok = g_ordered_tiles != 0 && (W == 1 || W == 2 || W == 4 || W == 8 || W == 16) &&
+    const bool tiles_ok = knobs.ordered_tiles != 0 && (W == 1 || W == 2 || W == 4 || W == 8 || W == 16) &&
                           segs * TILE_ROWS <= 4 * P.T + 4096 && segs < (int64_t)1 << 31;
-    if (whole && P.T <= g_by_t_limit) P.mode = MODE_BY_T;
-    else if (tiles_ok) P.mode = MODE_TILES;
-    else P.mode = MODE_SORTED;
-    P.n_seg = P.mode == MODE_TILES ? (uint32_t)segs : 0u;
+    if (whole && P.T <= knobs.by_t_limit) P.path = Path::BY_T;
+    else if (!tiles_ok) P.path = Path::SORTED;
+    else if (knobs.class_dedup != 0 && class_job_plan(M_total, P.blocks, nblk, P.T, P.fmt.tb, g_key_mask,
+                                                      knobs.class_variant, P.job))
+        P.path = Path::TILES_CLASS;
+    else P.path = Path::TILES_SORT;
+    P.n_seg = P.tiles() ? (uint32_t)segs : 0u;
 
     Arena ar(ws, ws ? ws_bytes : 0);
     const size_t m = (size_t)(M_total > 0 ? M_total : 1), n = (size_t)(N > 0 ? N : 1), t = (size_t)(P.T > 0 ? P.T : 1);
@@ -509,21 +519,19 @@ static int mul_blocks_plan(int64_t M_total, int64_t N, int32_t W, const int64_t 
     P.d_blocks = nullptr;
     P.drop = nullptr;
     P.segoff = nullptr;
-    P.class_mode = false;
     P.class_ws = nullptr;
     P.class_ws_bytes = 0;
-    if (P.mode == MODE_TILES) {
+    if (P.tiles()) {
         const size_t sg = (size_t)P.n_seg;
         need += arena_need(256, sizeof(TileBlock)) + arena_need(4 * sg, 4) + arena_need(sg + 1, 4);
         P.d_blocks = ar.take<TileBlock>(256);
         P.drop = ar.take<uint32_t>(4 * sg);
         P.segoff = ar.take<uint32_t>(sg + 1);
-        P.class_mode = class_job_plan(M_total, P.blocks, nblk, P.T, t_bits_for(M_total * N), g_key_mask, P.job);
-        if (P.class_mode) {
-            P.class_ws_bytes = class_job_ws_bytes(P.job);
-            need += arena_need(P.class_ws_bytes, 1);
-            P.class_ws = ar.take<unsigned char>(P.class_ws_bytes);
-        }
+    }
+    if (P.path == Path::TILES_CLASS) {
+        P.class_ws_bytes = class_job_ws_bytes(P.job);
+        need += arena_need(P.class_ws_bytes, 1);
+        P.class_ws = ar.take<unsigned char>(P.class_ws_bytes);
     }
     P.rest = ws ? (void *)(ar.base + ar.off) : nullptr;
     P.rest_bytes = (ws && ws_bytes > ar.off) ? ws_bytes - ar.off : 0;
@@ -542,6 +550,14 @@ static TileMap tile_map_of(const MulBlocksPlan &P, int64_t M_total) {
     tm.drop = P.drop;
     tm.segoff = P.segoff;
     return tm;
+}
+
+static int check_ws(const MulBlocksPlan &P, const void *ws, size_t ws_bytes) {
+    if (ws == nullptr || ws_bytes < P.need) {
+        set_error("workspace too small: need %zu bytes, got %zu", P.need, ws_bytes);
+        return SYM_E_WORKSPACE;
+    }
+    return SYM_OK;
 }
 
 extern "C" size_t sym_mul_blocks_ws_bytes(int64_t M_total, int64_t N, int32_t W, const int64_t *blocks_host, int32_t nblk) {
@@ -574,10 +590,7 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
         if (n_out_host) *n_out_host = 0;
         return SYM_OK;
     }
-    if (ws == nullptr || ws_bytes < P.need) {
-        set_error("workspace too small: need %zu bytes, got %zu", P.need, ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
+    SYM_TRY(check_ws(P, ws, ws_bytes));
     if (a_sketch) {   // the caller already has A's tables (sym_rotate_split): two reads of A saved
         SYM_CUDA_OK(cudaMemcpyAsync(P.a_sk, a_sketch, sizeof(uint64_t) * (size_t)M_total, cudaMemcpyDeviceToDevice, st));
         SYM_CUDA_OK(cudaMemcpyAsync(P.a_y, a_ycount, sizeof(int32_t) * (size_t)M_total, cudaMemcpyDeviceToDevice, st));
@@ -586,16 +599,16 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
     } else {
         SYM_TRY(operand_tables(a_xz, M_total, b_xz, N, W, P.a_sk, P.a_y, P.b_sk, P.b_y, st));
     }
-    RecFmt fmt{t_bits_for(M_total * N)};
-    if (P.mode == MODE_TILES) {
+    if (P.tiles()) {
         if (P.nblk > 1)   // block 0 travels inside the TileMap kernel argument
             SYM_CUDA_OK(cudaMemcpyAsync(P.d_blocks, P.blocks, sizeof(TileBlock) * (size_t)P.nblk, cudaMemcpyHostToDevice, st));
         SYM_CUDA_OK(cudaMemsetAsync(P.drop, 0, sizeof(uint32_t) * 4 * (size_t)P.n_seg, st));
     }
+    const RecFmt fmt = P.fmt;
     size_t off = 0;
-    for (int b = 0; b < P.nblk && !P.class_mode; ++b) {
+    for (int b = 0; b < P.nblk && P.path != Path::TILES_CLASS; ++b) {
         const TileBlock &tb = P.blocks[b];
-        if (P.mode == MODE_TILES) {
+        if (P.path == Path::TILES_SORT) {
             // a separate kernel writes the records before the sort: generating them inside the first radix pass
             // measured slower on B200 (10.06 vs 9.65 ms per 1.25e8 cross terms: a key costs two 64-bit multiplies
             // and is generated twice, in the histogram and in pass 0, against 0.15 ms for writing 1 GB once)
@@ -618,23 +631,23 @@ extern "C" int sym_mul_blocks_count_tables(const uint64_t *a_xz, const double *a
     }
     ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
     rows.Minv = fastdiv_magic((uint32_t)M_total);
-    if (P.class_mode) {
-        if (P.class_ws == nullptr) {
-            set_error("workspace arena exhausted (class tables)");
-            return SYM_E_WORKSPACE;
+    switch (P.path) {
+        case Path::BY_T:
+        case Path::SORTED:
+            return dedup_product_plan(P.path, P.recs, P.T, fmt, rows, zero_threshold, n_out, n_out_host, P.rest, P.rest_bytes, st);
+        case Path::TILES_SORT:
+            return dedup_product_plan_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), zero_threshold, n_out, n_out_host,
+                                            P.rest, P.rest_bytes, st);
+        case Path::TILES_CLASS: {
+            bool spec = false;
+            SYM_TRY(dedup_product_plan_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.job, P.a_sk, P.b_sk, P.a_y,
+                                               P.b_y, P.class_ws, P.class_ws_bytes, zero_threshold, n_out, n_out_host,
+                                               speculate ? &spec : nullptr, P.rest, P.rest_bytes, st));
+            if (speculate) *speculate = spec ? 1 : 0;
+            return SYM_OK;
         }
-        bool spec = false;
-        SYM_TRY(dedup_product_plan_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.job, P.a_sk, P.b_sk, P.a_y, P.b_y,
-                                           P.class_ws, P.class_ws_bytes, zero_threshold, n_out, n_out_host,
-                                           speculate ? &spec : nullptr, P.rest, P.rest_bytes, st));
-        if (speculate) *speculate = spec ? 1 : 0;
-        return SYM_OK;
     }
-    if (P.mode == MODE_TILES)
-        return dedup_product_plan_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), zero_threshold, n_out, n_out_host,
-                                        P.rest, P.rest_bytes, st);
-    return dedup_product_plan(P.recs, P.T, fmt, rows, P.mode == MODE_BY_T, zero_threshold, n_out, n_out_host, P.rest,
-                              P.rest_bytes, st);
+    return SYM_E_INVALID;
 }
 
 extern "C" int sym_mul_blocks_emit(const uint64_t *a_xz, const double *a_c, int64_t M_total, const uint64_t *b_xz,
@@ -644,18 +657,20 @@ extern "C" int sym_mul_blocks_emit(const uint64_t *a_xz, const double *a_c, int6
     SYM_TRY(mul_blocks_plan(M_total, N, W, blocks_host, nblk, ws, ws_bytes, P));
     if (P.T == 0 || U == 0) return SYM_OK;
     SYM_REQUIRE(U >= 0 && U <= P.T, "bad survivor count");
-    if (ws == nullptr || ws_bytes < P.need) {
-        set_error("workspace too small: need %zu bytes, got %zu", P.need, ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
+    SYM_TRY(check_ws(P, ws, ws_bytes));
     ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
     rows.Minv = fastdiv_magic((uint32_t)M_total);
-    RecFmt fmt{t_bits_for(M_total * N)};
-    if (P.mode == MODE_TILES)
-        return dedup_product_emit_tiles(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.blocks, P.a_y, P.b_y, U, out_xz,
-                                        out_c, P.rest, P.rest_bytes, P.class_mode, (cudaStream_t)stream);
-    return dedup_product_emit(P.recs, P.T, fmt, rows, P.mode == MODE_BY_T, U, out_xz, out_c, P.rest, P.rest_bytes,
-                              (cudaStream_t)stream);
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (P.path) {
+        case Path::BY_T:
+        case Path::SORTED:
+            return dedup_product_emit(P.path, P.recs, P.T, P.fmt, rows, U, out_xz, out_c, P.rest, P.rest_bytes, st);
+        case Path::TILES_SORT:
+        case Path::TILES_CLASS:
+            return dedup_product_emit_tiles(P.path, P.recs, P.T, P.fmt, rows, tile_map_of(P, M_total), P.blocks, P.a_y, P.b_y, U,
+                                            out_xz, out_c, P.rest, P.rest_bytes, st);
+    }
+    return SYM_E_INVALID;
 }
 
 extern "C" int sym_mul_blocks_emit_spec(const uint64_t *a_xz, const double *a_c, int64_t M_total, const uint64_t *b_xz,
@@ -664,35 +679,29 @@ extern "C" int sym_mul_blocks_emit_spec(const uint64_t *a_xz, const double *a_c,
                                         size_t ws_bytes, void *stream) {
     MulBlocksPlan P;
     SYM_TRY(mul_blocks_plan(M_total, N, W, blocks_host, nblk, ws, ws_bytes, P));
-    SYM_REQUIRE(P.class_mode && P.T > 0, "this product takes no speculative emission");
-    if (ws == nullptr || ws_bytes < P.need || P.class_ws == nullptr) {
-        set_error("workspace too small: need %zu bytes, got %zu", P.need, ws_bytes);
-        return SYM_E_WORKSPACE;
-    }
+    SYM_REQUIRE(P.path == Path::TILES_CLASS && P.T > 0, "this product takes no speculative emission");
+    SYM_TRY(check_ws(P, ws, ws_bytes));
     ProductRows rows{a_xz, b_xz, a_c, b_c, (uint32_t)M_total, 2 * W, (uint32_t)N};
     rows.Minv = fastdiv_magic((uint32_t)M_total);
-    RecFmt fmt{t_bits_for(M_total * N)};
-    return dedup_product_spec_classes(P.recs, P.T, fmt, rows, tile_map_of(P, M_total), P.blocks, P.job, P.b_sk, P.a_y, P.b_y,
+    return dedup_product_spec_classes(P.recs, P.T, P.fmt, rows, tile_map_of(P, M_total), P.blocks, P.job, P.b_sk, P.a_y, P.b_y,
                                       P.class_ws, P.class_ws_bytes, zero_threshold, out_xz, out_c, n_out_host, P.rest,
                                       P.rest_bytes, (cudaStream_t)stream);
 }
 
-// the whole product = one block
+// The whole product = one block. Sized for every path a tuning-knob change can select for the shape (BY_T needs what
+// SORTED needs, the class tables grow with the class count of knob 11's shape), so that a knob change between calls
+// never invalidates a workspace.
 extern "C" size_t sym_mul_cleanup_ws_bytes(int64_t M, int64_t N, int32_t W) {
     const int64_t blk[4] = {0, M, 0, N};
-    // sized for either mode, so that a tuning-knob change between calls never invalidates a workspace
-    const int64_t T = M * N > 0 ? M * N : 1;
-    const size_t segs = (size_t)(N > 0 ? N : 1) * (size_t)((M + TILE_ROWS - 1) / TILE_ROWS + 1);
-    (void)blk;
-    size_t class_bytes = 0;
-    {
-        TileBlock tb{0u, (uint32_t)(M > 0 ? M : 0), 0u, (uint32_t)(N > 0 ? N : 0), 0u, 0u};
-        ClassJob job;
-        if (M > 0 && N > 0 && class_job_plan(M, &tb, 1, T, t_bits_for(T), ~0ull, job, true))
-            class_bytes = arena_need(class_job_ws_bytes(job), 1);
+    size_t need = 0;
+    for (int tiles = 0; tiles <= 1; ++tiles) {
+        for (int variant = -1; variant <= 3; ++variant) {   // -1: knob 10 = 0
+            const PathKnobs knobs{-1, tiles, variant >= 0, variant >= 0 ? variant : 0};
+            MulBlocksPlan P;
+            if (mul_blocks_plan(M, N, W, blk, 1, nullptr, 0, P, knobs) == SYM_OK && P.need > need) need = P.need;
+        }
     }
-    return sym_pair_records_ws_bytes(M, N, W) + arena_need((size_t)T, 8) + dedup_ws_bytes(T) + class_bytes +
-           arena_need(256, sizeof(TileBlock)) + arena_need(4 * segs, 4) + arena_need(segs + 1, 4) + 2048;
+    return need;
 }
 
 extern "C" int sym_mul_cleanup_count(const uint64_t *a_xz, const double *a_c, int64_t M, const uint64_t *b_xz,

@@ -261,9 +261,10 @@ struct ClassJob {
     const uint32_t *vkey, *vq;                 // rows of B ("visits") in table-entry order: table index, row index q
     const uint64_t *vsk;                       //                                           sketch
 };
-// false: this product takes the global record sort instead (too many blocks, B much larger than A, knob 10 = 0)
-bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t T, int tb, uint64_t key_mask, ClassJob &J,
-                    bool ignore_knob = false);
+// false: this product takes the global record sort instead (too many blocks, B much larger than A).
+// variant: CTA shape of the class kernel (tuning knob 11)
+bool class_job_plan(int64_t M_total, const TileBlock *blocks, int nblk, int64_t T, int tb, uint64_t key_mask, int variant,
+                    ClassJob &J);
 size_t class_job_ws_bytes(const ClassJob &J);
 // overflow records carry their enumeration position in the term field while they are sorted; this puts t back
 int class_ord_to_t(const ClassJob &J, uint64_t *recs, uint32_t n, cudaStream_t st);
@@ -279,15 +280,21 @@ int class_dedup_bind(ClassJob &J, const uint64_t *b_sk, void *ws, size_t ws_byte
 int class_dedup_classes(const ClassJob &J, const ProductRows &rows, const TileMap &tm, double thr, uint64_t *cand, uint64_t *over,
                         uint32_t *counters, uint32_t c0, uint32_t c1, uint32_t sms, cudaStream_t st);
 
+// The path of a product through the dedup, decided once per call by mul_blocks_plan (multiply.cu):
+//   BY_T         the t fields are a permutation of 0..T-1 and the survivors are written in increasing-t
+//                (first occurrence) order;
+//   SORTED       survivors in sorted-hash order;
+//   TILES_SORT   ordered-tile mode, duplicates found by the global record sort;
+//   TILES_CLASS  ordered-tile mode, duplicates found class by class (class_dedup.cu): no record array.
+enum class Path { BY_T, SORTED, TILES_SORT, TILES_CLASS };
+
 // Dedup driver (dedup.cu), split where the survivor count is known so the caller can allocate
-// exact-size outputs. `recs` holds T records (clobbered). by_t: the t fields are a permutation of
-// 0..T-1 and the output is written in increasing-t (first occurrence) order; otherwise the output
-// is in sorted-hash order.
+// exact-size outputs. `recs` holds T records (clobbered). path: BY_T or SORTED.
 size_t dedup_ws_bytes(int64_t T);
 void set_emit_events(cudaEvent_t before, cudaEvent_t after);
-int dedup_product_plan(uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, bool by_t, double thr,
+int dedup_product_plan(Path path, uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, double thr,
                        int64_t *n_out, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
-int dedup_product_emit(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, bool by_t, int64_t U,
+int dedup_product_emit(Path path, const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, int64_t U,
                        uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, cudaStream_t st);
 int dedup_plain_plan(uint64_t *recs, int64_t T, RecFmt fmt, const PlainRows &rows, double thr, int64_t *n_out,
                      int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
@@ -309,8 +316,9 @@ int dedup_product_spec_classes(uint64_t *recs, int64_t T, RecFmt fmt, const Prod
                                const TileBlock *blocks_host, ClassJob &job, const uint64_t *b_sk, const int32_t *a_y,
                                const int32_t *b_y, void *class_ws, size_t class_ws_bytes, double thr, uint64_t *out_xz,
                                double *out_c, int64_t *n_out_host, void *ws, size_t ws_bytes, cudaStream_t st);
-int dedup_product_emit_tiles(const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
+// path: TILES_SORT or TILES_CLASS
+int dedup_product_emit_tiles(Path path, const uint64_t *recs, int64_t T, RecFmt fmt, const ProductRows &rows, const TileMap &tm,
                              const TileBlock *blocks_host, const int32_t *a_y, const int32_t *b_y, int64_t U,
-                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, bool class_mode, cudaStream_t st);
+                             uint64_t *out_xz, double *out_c, void *ws, size_t ws_bytes, cudaStream_t st);
 
 }  // namespace symb
