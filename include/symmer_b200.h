@@ -286,6 +286,24 @@ int sym_project(const uint64_t *xz, const double *c, int64_t M, int32_t W, int32
                 int32_t n_free, uint64_t *out_xz, double *out_c, int64_t *n_out, int64_t *n_out_host,
                 void *ws, size_t ws_bytes, void *stream);
 
+/* ---- noncontextual ground state (CS-VQE: NoncontextualOp.solve, symmer/operators/noncontextual_op.py).
+ * A noncontextual operator decomposes as P_t = s_t * G^{J_t} * C_{i_t}: k commuting generators G, N pairwise
+ * anticommuting clique representatives C (no C for the symmetry terms, i_t = -1), s_t = +-1.
+ * sym_nc_signs: s_t from the rows (xz: uint64[M][2W], gen_xz: uint64[k][2W], rep_xz: uint64[N][2W]), J: uint64[M][Jw]
+ *   (bit j of row t set <=> G_j is a factor of P_t), clique: int32[M] in [-1, N). signs: double[M] receives s_t, or 0
+ *   where the product is not +-P_t (the decomposition does not hold for that term).
+ * sym_nc_min: minimum over the 2^f assignments m (bit j set <=> nu_j = -1) of
+ *     E(m) = a(m) - sqrt(sum_i w_i(m)^2),  a = sum_{clique[t] = -1} v_t (-1)^{|J_t & m|},  w_i = sum_{clique[t] = i} v_t (-1)^{|J_t & m|}
+ *   J: uint64[M] free-bit masks (bits >= f are ignored), v: double[M] (= h_t s_t), clique: int32[M] in [-1, N) (terms
+ *   outside are ignored), 0 <= f <= 62, N <= 4094. best: device 16 bytes {double E; uint64_t m}, ties to the smaller m;
+ *   best_host (may be NULL; forces one stream synchronise) receives a copy. Deterministic: no floating-point atomics,
+ *   terms summed in (clique, J) order, one ordered final reduction. */
+int sym_nc_signs(const uint64_t *xz, int64_t M, int32_t W, const uint64_t *gen_xz, int32_t k, const uint64_t *rep_xz,
+                 int32_t N, const uint64_t *J, int32_t Jw, const int32_t *clique, double *signs, void *stream);
+size_t sym_nc_min_ws_bytes(int64_t M, int32_t N);
+int sym_nc_min(const uint64_t *J, const double *v, const int32_t *clique, int64_t M, int32_t N, int32_t f, void *best,
+               void *best_host, void *ws, size_t ws_bytes, void *stream);
+
 /* out[i] = words[perm[i] * pitch_words + column] (perm NULL = identity): one 64-bit word column of a row-major matrix
  * in a given row order. Key of one pass of the word-by-word lexicographic sort that replaces
  * `np.lexsort(symp_matrix.T)` (symmer/operators/base.py:469-470) and of `__eq__` (base.py:640-662). */

@@ -8,7 +8,7 @@ from . import _cabi  # noqa: F401  (raises if the CUDA library is missing and ca
 
 __all__ = ["PauliwordOp", "QuantumState", "IndependentOp", "QubitTapering", "S3Projection", "single_term_expval",
            "get_PauliwordOp_projector", "get_ij_operator", "change_of_basis_XY_to_Z", "CircuitSymmerlator",
-           "exact_gs_energy", "trotter"]
+           "exact_gs_energy", "trotter", "NoncontextualOp"]
 _BASE_NAMES = ("PauliwordOp", "QuantumState", "single_term_expval", "get_PauliwordOp_projector", "get_ij_operator",
                "change_of_basis_XY_to_Z")
 
@@ -20,6 +20,9 @@ def __getattr__(name):
     if name == "IndependentOp":
         from .independent_op import IndependentOp
         return IndependentOp
+    if name == "NoncontextualOp":
+        from .noncontextual_op import NoncontextualOp
+        return NoncontextualOp
     if name in ("QubitTapering", "S3Projection"):
         from . import projection
         return getattr(projection, name)

@@ -73,6 +73,9 @@ SIGNATURES = {
     "sym_project_ws_bytes": (c_sz, [c_i64, c_i32]),
     "sym_project": (ctypes.c_int, [c_p, c_p, c_i64, c_i32, c_i32, c_p, c_p, c_i32, c_p, c_i32, c_p, c_p, c_p, c_p, c_p,
                                    c_sz, c_p]),
+    "sym_nc_signs": (ctypes.c_int, [c_p, c_i64, c_i32, c_p, c_i32, c_p, c_i32, c_p, c_i32, c_p, c_p, c_p]),
+    "sym_nc_min_ws_bytes": (c_sz, [c_i64, c_i32]),
+    "sym_nc_min": (ctypes.c_int, [c_p, c_p, c_p, c_i64, c_i32, c_i32, c_p, c_p, c_p, c_sz, c_p]),
     "sym_pair_records_ws_bytes": (c_sz, [c_i64, c_i64, c_i32]),
     "sym_pair_records": (ctypes.c_int, [c_p, c_i64, c_i64, c_i64, c_p, c_i64, c_i32, c_p, c_p, c_sz, c_p]),
     "sym_pair_records_blocks": (ctypes.c_int, [c_p, c_i64, c_p, c_i64, c_i32, c_p, c_i32, c_p, c_p, c_sz, c_p]),

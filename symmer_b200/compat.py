@@ -1,6 +1,6 @@
 """`import symmer` served by this engine: `install_as_symmer()` registers module objects named like the reference's
-packages (`symmer`, `symmer.operators`, `symmer.operators.utils`, `symmer.operators.base`, `symmer.projection`,
-`symmer.evolution[.gate_library|.exponentiation|.circuit_symmerlator]`, `symmer.utils`) whose attributes are the
+packages (`symmer`, `symmer.operators`, `symmer.operators.utils`, `symmer.operators.base`,
+`symmer.operators.independent_op`, `symmer.operators.noncontextual_op`, `symmer.projection`, `symmer.evolution[.gate_library|.exponentiation|.circuit_symmerlator]`, `symmer.utils`) whose attributes are the
 device-resident classes and functions of `symmer_b200`, so code written against UCL-CCS/symmer — including the
 reference's own test files — runs unmodified on the B200 engine. Only what this repository implements is exposed
 (INTEGRATION.md §3); anything else raises AttributeError / ImportError as usual.
@@ -12,8 +12,8 @@ import sys
 import types
 
 _NAMES = ["symmer", "symmer.operators", "symmer.operators.utils", "symmer.operators.base",
-          "symmer.operators.independent_op", "symmer.projection", "symmer.projection.qubit_tapering",
-          "symmer.projection.base", "symmer.evolution", "symmer.evolution.gate_library",
+          "symmer.operators.independent_op", "symmer.operators.noncontextual_op", "symmer.projection",
+          "symmer.projection.qubit_tapering", "symmer.projection.base", "symmer.evolution", "symmer.evolution.gate_library",
           "symmer.evolution.exponentiation", "symmer.evolution.circuit_symmerlator", "symmer.utils"]
 
 
@@ -30,17 +30,18 @@ def install_as_symmer():
     """Register the alias modules; returns the top-level `symmer` module object."""
     if "symmer" in sys.modules and not getattr(sys.modules["symmer"], "__symmer_b200_alias__", False):
         raise ImportError("a real `symmer` package is already imported; use symmer_b200.patch.install() instead")
-    from . import base, circuit_symmerlator, evolution, independent_op, projection, symmer_utils, utils
+    from . import base, circuit_symmerlator, evolution, independent_op, noncontextual_op, projection, symmer_utils, utils
     mods = {name: types.ModuleType(name) for name in _NAMES}
     for m in mods.values():
         m.__symmer_b200_alias__ = True
     mods["symmer.operators.utils"].__dict__.update(_public(utils))
     mods["symmer.operators.base"].__dict__.update(_public(base))
     mods["symmer.operators.independent_op"].__dict__.update(IndependentOp=independent_op.IndependentOp)
+    mods["symmer.operators.noncontextual_op"].__dict__.update(NoncontextualOp=noncontextual_op.NoncontextualOp)
     ops_ns = mods["symmer.operators"].__dict__
     ops_ns.update(_public(utils))
     ops_ns.update(_public(base))
-    ops_ns.update(IndependentOp=independent_op.IndependentOp)
+    ops_ns.update(IndependentOp=independent_op.IndependentOp, NoncontextualOp=noncontextual_op.NoncontextualOp)
     mods["symmer.projection"].__dict__.update(QubitTapering=projection.QubitTapering, S3Projection=projection.S3Projection)
     mods["symmer.projection.qubit_tapering"].__dict__.update(QubitTapering=projection.QubitTapering)
     mods["symmer.projection.base"].__dict__.update(S3Projection=projection.S3Projection)

@@ -672,6 +672,38 @@ def or_rows(bits, rows=None):
     return out
 
 
+# ---------------------------------------------------------------------------------- noncontextual
+def nc_signs(xz, gen_xz, rep_xz, J, clique):
+    """float64[M] device: s_t of P_t = s_t * G^{J_t} * C_{clique[t]} (0 where the product is not +-P_t).
+    J: int64[M, Jw] device bit rows over the k generators; clique: int32[M] device, -1 for symmetry terms."""
+    M, W = _rows(xz)
+    k, N = int(gen_xz.shape[0]), int(rep_xz.shape[0])
+    assert J.dtype == torch.int64 and J.dim() == 2 and J.shape[0] == M and J.is_contiguous()
+    assert clique.dtype == torch.int32 and clique.numel() == M and clique.is_contiguous()
+    signs = torch.empty(M, dtype=torch.float64, device=xz.device)
+    _cabi.check(lib().sym_nc_signs(_p(xz), M, W, _p(gen_xz.contiguous()), k, _p(rep_xz.contiguous()), N, _p(J),
+                                   int(J.shape[1]), _p(clique), _p(signs), _stream()))
+    return signs
+
+
+def nc_min(J, v, clique, n_cliques, f):
+    """(E, m): the minimum over the 2^f assignments m of a(m) - ||w(m)|| (see sym_nc_min), ties to the smaller m.
+    J: int64[M] free-bit masks, v: float64[M], clique: int32[M] (device). One 16-byte copy back."""
+    M = int(J.numel())
+    assert J.dtype == torch.int64 and v.dtype == torch.float64 and clique.dtype == torch.int32
+    assert v.numel() == M and clique.numel() == M
+    L = lib()
+    nbytes = L.sym_nc_min_ws_bytes(M, int(n_cliques))
+    if nbytes == 0:
+        _cabi.check(-1)
+    ws = workspace(nbytes)
+    best = torch.empty(2, dtype=torch.int64, device=ws.device)
+    host = (ctypes.c_uint64 * 2)()
+    _cabi.check(L.sym_nc_min(_p(J.contiguous()), _p(v.contiguous()), _p(clique.contiguous()), M, int(n_cliques), int(f),
+                             _p(best), ctypes.cast(host, ctypes.c_void_p), _p(ws), ws.numel(), _stream()))
+    return float(np.frombuffer(bytes(host), dtype=np.float64)[0]), int(host[1])
+
+
 # ---------------------------------------------------------------------------------- sort / records
 def sort_pairs(keys, vals, begin_bit=0):
     """Stable sort of (int64-as-uint64 keys, int32-as-uint32 vals) in place; returns (keys, vals)."""
