@@ -145,7 +145,10 @@ int sym_commute_mma(const uint64_t *a_xz, int64_t M, const uint64_t *b_xz, int64
                     uint8_t *out, void *ws, size_t ws_bytes, void *stream);
 /* Same with out_pitch bytes between output rows (out_pitch >= N). A pitch that is a multiple of 32
  * keeps every row 16-byte aligned, so ragged N (NaCl: 42 599 terms) takes the 32-byte vector stores
- * instead of per-byte stores (measured 10x at 36 qubits); bytes N..out_pitch-1 of a row are scratch. */
+ * instead of per-byte stores (measured 10x at 36 qubits). A call writes bytes [0, min(out_pitch, ceil32(N))) of
+ * each of its M rows and nothing else: bytes N..ceil32(N)-1 may be overwritten, bytes from ceil32(N) on are never
+ * touched (so a block of an upper triangle, out + i0*(pitch+1) with N = M - i0, stays inside its rows). Any M
+ * below 2^31 (A runs in slabs of 65535*128 rows). */
 int sym_commute_mma_pitched(const uint64_t *a_xz, int64_t M, const uint64_t *b_xz, int64_t N, int32_t W,
                             uint8_t *out, int64_t out_pitch, void *ws, size_t ws_bytes, void *stream);
 /* Mirrors the blocks on and above the block diagonal (square blocks of `block_rows` rows, a multiple of 32) of a

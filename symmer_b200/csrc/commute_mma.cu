@@ -84,8 +84,10 @@ __device__ __forceinline__ void umma_i8(uint32_t d_tmem, uint64_t a_desc, uint64
 // 16 packed bits -> 16 operand bytes: nibble * 0x00204081 puts bit k of the nibble at the LEAST SIGNIFICANT bit of byte k
 // (the copies n, n<<7, n<<14, n<<21 do not overlap, so no carries). The higher bits of every byte are left as they
 // fall: only the PARITY of the int32 dot product is used, and the parity of sum(a_i * b_i) depends on the low bits of
-// a_i and b_i alone (bytes are unsigned and <= 227, so the sum stays below 2^31 up to ~20 000 qubits). Dropping
-// the `& 0x01010101` of the 0/1 encoding saves a third of the expansion's ALU work, which is what limits the kernel.
+// a_i and b_i alone. Bytes are unsigned and <= 227, so two all-Y rows pass 2^31 from ~38 500 qubits on; the int32
+// accumulation wraps there rather than saturating, which keeps the parity exact at any width (measured on a B200 at
+// 40 000 qubits, tests/test_gpu_bitmatrix.py). Dropping the `& 0x01010101` of the 0/1 encoding saves a third of the
+// expansion's ALU work, which is what limits the kernel.
 __device__ __forceinline__ uint4 expand16(uint32_t bits) {
     uint4 v;
     v.x = (bits & 0xFu) * 0x00204081u;
@@ -253,8 +255,10 @@ __global__ void __launch_bounds__(MMA_THREADS + 32, 2) commute_mma_ws_kernel(con
                       "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
                     : "r"(taddr));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (row < M) {
-                    const uint32_t jbase = j0 + col_half + cb;
+                const uint32_t jbase = j0 + col_half + cb;
+                // a chunk starting at or past N holds no result: storing it would write up to 224 bytes past
+                // ceil32(N), i.e. past the row in commute_self's sub-views and past the matrix in its last row
+                if (row < M && jbase < N) {
                     uint8_t *dst = out + (size_t)row * pitch + jbase;
                     if (jbase + 32 <= pitch && ((reinterpret_cast<uintptr_t>(dst) & 15) == 0)) {
                         uint32_t p[8];
@@ -284,8 +288,12 @@ __global__ void __launch_bounds__(MMA_THREADS + 32, 2) commute_mma_ws_kernel(con
 
 using namespace symb;
 
+// grid.y is limited to 65535 row tiles: A runs in slabs of at most this many rows, which share one transposed copy
+constexpr int64_t MMA_SLAB_ROWS = (int64_t)65535 * MMA_M;
+
 extern "C" size_t sym_commute_mma_ws_bytes(int64_t M, int64_t N, int32_t W) {
-    return arena_need((size_t)(M > 0 ? M : 1) * 2 * W, 8) + arena_need((size_t)(N > 0 ? N : 1) * 2 * W, 8) + 1024;
+    const int64_t slab = M < MMA_SLAB_ROWS ? M : MMA_SLAB_ROWS;
+    return arena_need((size_t)(slab > 0 ? slab : 1) * 2 * W, 8) + arena_need((size_t)(N > 0 ? N : 1) * 2 * W, 8) + 1024;
 }
 
 extern "C" int sym_commute_mma(const uint64_t *a_xz, int64_t M, const uint64_t *b_xz, int64_t N, int32_t W, uint8_t *out,
@@ -298,22 +306,13 @@ extern "C" int sym_commute_mma_pitched(const uint64_t *a_xz, int64_t M, const ui
     SYM_REQUIRE(M >= 0 && N >= 0 && W >= 1, "bad size");
     SYM_REQUIRE(out_pitch >= N, "out_pitch must be >= N");
     SYM_REQUIRE(M < ((int64_t)1 << 31) && N < ((int64_t)1 << 31), "operand too large");
+    SYM_REQUIRE(W <= 65535 * 16, "operand too wide for one transpose launch");
     if (M == 0 || N == 0) return SYM_OK;
     if (ws_bytes < sym_commute_mma_ws_bytes(M, N, W)) {
         set_error("workspace too small");
         return SYM_E_WORKSPACE;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    Arena ar(ws, ws_bytes);
-    uint64_t *a_t = ar.take<uint64_t>((size_t)M * 2 * W);
-    uint64_t *b_t = ar.take<uint64_t>((size_t)N * 2 * W);
-    const int words = 2 * W;
-    transpose_words_kernel<<<dim3((unsigned)((M + 31) / 32), (unsigned)((words + 31) / 32)), 256, 0, st>>>(a_xz, (uint32_t)M,
-                                                                                                        words, 0, a_t);
-    SYM_LAUNCH_OK();
-    transpose_words_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((words + 31) / 32)), 256, 0, st>>>(b_xz, (uint32_t)N,
-                                                                                                        words, 1, b_t);
-    SYM_LAUNCH_OK();
     constexpr size_t smem = MMA_STAGES * (A_STAGE_BYTES + B_STAGE_BYTES) + 128;
     static bool attr_done[64] = {};   // per device
     int dev = 0;
@@ -322,10 +321,23 @@ extern "C" int sym_commute_mma_pitched(const uint64_t *a_xz, int64_t M, const ui
         SYM_CUDA_OK(cudaFuncSetAttribute(commute_mma_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
-    const int64_t tiles_m = (M + MMA_M - 1) / MMA_M;
-    SYM_REQUIRE(tiles_m <= 65535, "too many A rows for one launch (slice A)");
-    dim3 grid((unsigned)((N + MMA_N - 1) / MMA_N), (unsigned)tiles_m);
-    commute_mma_ws_kernel<<<grid, MMA_THREADS + 32, smem, st>>>(a_t, (uint32_t)M, b_t, (uint32_t)N, W, out, (size_t)out_pitch);
+    Arena ar(ws, ws_bytes);
+    uint64_t *a_t = ar.take<uint64_t>((size_t)(M < MMA_SLAB_ROWS ? M : MMA_SLAB_ROWS) * 2 * W);
+    uint64_t *b_t = ar.take<uint64_t>((size_t)N * 2 * W);
+    const int words = 2 * W;
+    transpose_words_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((words + 31) / 32)), 256, 0, st>>>(b_xz, (uint32_t)N,
+                                                                                                        words, 1, b_t);
     SYM_LAUNCH_OK();
+    // one transpose and one launch per slab of A; a_t is reused in stream order
+    for (int64_t done = 0; done < M; done += MMA_SLAB_ROWS) {
+        const int64_t rows = M - done < MMA_SLAB_ROWS ? M - done : MMA_SLAB_ROWS;
+        transpose_words_kernel<<<dim3((unsigned)((rows + 31) / 32), (unsigned)((words + 31) / 32)), 256, 0, st>>>(
+            a_xz + (size_t)done * words, (uint32_t)rows, words, 0, a_t);
+        SYM_LAUNCH_OK();
+        dim3 grid((unsigned)((N + MMA_N - 1) / MMA_N), (unsigned)((rows + MMA_M - 1) / MMA_M));
+        commute_mma_ws_kernel<<<grid, MMA_THREADS + 32, smem, st>>>(a_t, (uint32_t)rows, b_t, (uint32_t)N, W,
+                                                                    out + (size_t)done * (size_t)out_pitch, (size_t)out_pitch);
+        SYM_LAUNCH_OK();
+    }
     return SYM_OK;
 }

@@ -85,11 +85,13 @@ template <bool FROM_DENSE>
 static int wht_run(const double2 *src, double2 *dst, int64_t K, int n, cudaStream_t st) {
     const int L = n < WHT_SMEM_BITS ? n : WHT_SMEM_BITS;
     const size_t smem = sizeof(double2) << L;
-    static bool configured[2] = {false, false};
-    if (!configured[FROM_DENSE ? 1 : 0]) {
+    static bool attr_done[64] = {};   // per device (one array per instantiation)
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 64 && !attr_done[dev]) {
         SYM_CUDA_OK(cudaFuncSetAttribute(wht_tile_kernel<FROM_DENSE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)(sizeof(double2) << WHT_SMEM_BITS)));
-        configured[FROM_DENSE ? 1 : 0] = true;
+        attr_done[dev] = true;
     }
     const int64_t side = (int64_t)1 << n;
     const int64_t ctas = K * (side >> L);

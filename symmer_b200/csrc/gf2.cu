@@ -275,11 +275,13 @@ extern "C" int sym_rref(uint64_t *bits, int64_t R, int64_t C, int64_t Cw, int32_
         return SYM_OK;
     }
     const size_t smem = (size_t)R * (size_t)Cw * 8;
+    int dev = 0;
+    cudaGetDevice(&dev);
     if (smem <= 200 * 1024) {
-        static bool attr_set = false;
-        if (!attr_set) {
+        static bool attr_done[64] = {};   // per device
+        if (dev >= 0 && dev < 64 && !attr_done[dev]) {
             SYM_CUDA_OK(cudaFuncSetAttribute(rref_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            attr_set = true;
+            attr_done[dev] = true;
         }
         rref_smem_kernel<<<1, RREF_THREADS, smem, st>>>(bits, (int)R, Cw, pivots);
         SYM_LAUNCH_OK();
@@ -296,10 +298,10 @@ extern "C" int sym_rref(uint64_t *bits, int64_t R, int64_t C, int64_t Cw, int32_
     if (g_rref_variant == 1 && kk >= 1) {
         uint32_t *mask = ar.take<uint32_t>((size_t)R);
         int *pv = ar.take<int>(PANEL_MAX);
-        static bool panel_attr = false;
-        if (!panel_attr) {
+        static bool attr_done[64] = {};   // per device
+        if (dev >= 0 && dev < 64 && !attr_done[dev]) {
             SYM_CUDA_OK(cudaFuncSetAttribute(rref_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)panel_cap));
-            panel_attr = true;
+            attr_done[dev] = true;
         }
         const dim3 sweep_grid((unsigned)((Cw + SWEEP_WORDS - 1) / SWEEP_WORDS), (unsigned)((R + SWEEP_ROWS - 1) / SWEEP_ROWS));
         for (int64_t i0 = 0; i0 < R; i0 += kk) {
